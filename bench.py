@@ -2,6 +2,7 @@
 """bench.py -- Mrays/s and ms/frame of the per-tile tracing hot path on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--full]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1: one rank per GPU)
 
 A step is one frame of the workload (default: killeroo + ground plane, 3840x2160, 16 spp, the
@@ -23,6 +24,9 @@ Prints ONE JSON line (rank 0):
   extra.configs   kernel / end-to-end / parity of the other BASELINE configs (C1-C4; C5 with --full), short runs
 `--impl reference` times the reference's own threaded CPU renderer (oracle/_ref), whole frames through its own
 worker pool, on the host cores instead.
+
+`--dump-outputs DIR` writes the frame the last timed step left in the host framebuffer (see dump_outputs), so that
+two builds can be compared pixel for pixel on the same workload.
 """
 import argparse
 import hashlib
@@ -79,6 +83,23 @@ def golden_digest(wl):
 
 def md5(a):
     return hashlib.md5(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+DUMP_MAX_PIXELS = 1 << 21  # 32 MiB of float32 BGRA + 16 MiB of float64 indices, under 64 MB in all
+
+
+def dump_outputs(out_dir, image):
+    """Write a BGRA frame ([H, W] uint32) as DIR/pixel_index.npy (float64 [n], row-major pixel index y * W + x) and
+    DIR/bgra.npy (float32 [n, 4], the channel bytes B, G, R, A).  Frames of more than DUMP_MAX_PIXELS pixels are
+    sampled at a fixed, seeded set of pixels, so every run of the same workload writes the same pixels."""
+    flat = np.ascontiguousarray(image, np.uint32).reshape(-1)
+    if flat.size > DUMP_MAX_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(flat.size, DUMP_MAX_PIXELS, replace=False))
+    else:
+        idx = np.arange(flat.size)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "bgra.npy"), flat[idx].view(np.uint8).reshape(-1, 4).astype(np.float32))
 
 
 def measured_peaks():
@@ -158,11 +179,11 @@ class ClockSampler:
 def time_reference_cpu(wl, steps, warmup, budget_s):
     """The reference's own CPU renderer (oracle/_ref: unmodified sources + headless driver): WHOLE frames through
     Framebuffer::WorkerThread (framebuffer.cpp:59-92) on hardware_concurrency() threads, `warmup` untimed + `steps`
-    timed (BASELINE.md 3.5: >= 1 + >= 5, best and median reported).  If that many frames do not fit budget_s the
-    number of timed frames is cut (never the frame).  The 50 M-triangle soup is the one exception (BASELINE.md 3.6):
-    its CPU side is the oracle port on a band of image rows -- the reference's own grid build does not finish on it
-    (FLT_MIN-seeded candidate ranges, triangle.h:123: ~10^5 cells per triangle at 512^3); the port builds the
-    identical grid with tight ranges.  Falls back to the port as well if oracle/_ref could not be built."""
+    timed (BASELINE.md 3.5: >= 1 + >= 5, best and median reported).  If the warm-up frames do not fit a share of
+    budget_s their number is cut; the number of timed frames is always `steps`.  The 50 M-triangle soup is the one
+    exception (BASELINE.md 3.6): its CPU side is the oracle port on a band of image rows -- the reference's own grid
+    build does not finish on it (FLT_MIN-seeded candidate ranges, triangle.h:123: ~10^5 cells per triangle at
+    512^3); the port builds the identical grid with tight ranges.  Falls back to the port as well if oracle/_ref could not be built."""
     from oracle import pyoracle as po
     scenes = pkg("scenes")
     w, h, spp = wl["width"], wl["height"], wl["spp"]
@@ -175,19 +196,17 @@ def time_reference_cpu(wl, steps, warmup, budget_s):
         t0 = time.perf_counter()
         r = ref.renderer(mesh, fov, cam, wl["grid_res"])
         build_s = time.perf_counter() - t0
-        # first frame: a warm-up, and the estimate the frame counts are cut to the budget with
+        # first frame: a warm-up, and the estimate the warm-up count is cut to the budget with
         sec, img = r.render(w, h, spp, want_image=True)
-        done_warm, spent = 1, sec
+        done_warm = 1
         n_warm = min(warmup, max(1, int(0.15 * budget_s / max(sec, 1e-6)))) if warmup > 0 else 0
         while done_warm < n_warm:
-            s2, _ = r.render(w, h, spp, want_image=False)
-            spent += s2
+            r.render(w, h, spp, want_image=False)
             done_warm += 1
-        n_timed = min(steps, max(5, int((budget_s - spent) / max(sec, 1e-6))))
         times = [sec] if warmup == 0 else []     # without warm-up frames the first one counts
         if warmup == 0:
             done_warm = 0
-        while len(times) < n_timed:
+        while len(times) < steps:
             s2, img = r.render(w, h, spp, want_image=True)
             times.append(s2)
         total = sum(times)
@@ -498,6 +517,8 @@ def run_ours(args, wl, rank, world, local_rank, dist):
         group.barrier()
     barrier_ms = float(group.allreduce_max([(time.perf_counter() - t0) / 20 * 1e3])[0])
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, g.host_fb)
 
     # ---- untimed: work counters, CPU baseline, parity, the other configs
     counters = g.count_work()
@@ -569,8 +590,11 @@ def main():
     ap.add_argument("--no-side-configs", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--no-class-route", action="store_true", help="skip the Renderer / Framebuffer class-route timing")
     ap.add_argument("--full", action="store_true", help="also run C5 (50 M triangles) among the side configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR as .npy files")
     args = ap.parse_args()
     args.steps = max(args.steps, 1)
+    if args.dump_outputs and args.impl != "ours":
+        raise SystemExit("--dump-outputs writes the GPU path's frame: use it with --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -89,16 +89,27 @@ def test_reference_tile_layout():
     assert (cover == 1).all()
 
 
-def test_bmp_writer_matches_reference_bytes(ref, tmp_path):
-    """Headless SaveToBMP path: same 54-byte header + pixel bytes as the reference's WriteBitmap."""
+def test_bmp_writer_matches_reference_bytes(ref_answers, port, scene_data, tmp_path):
+    """Headless SaveToBMP path: same 54-byte header + pixel bytes as the reference's WriteBitmap, on a frame equal to
+    the reference's own render."""
     hostlib = pkg("hostapi").load_host_library()
     hostlib.rtm_write_bitmap.restype = C.c_int
     hostlib.rtm_write_bitmap.argtypes = [C.c_char_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32)]
-    scenes = pkg("scenes")
-    m, fov, cam = scenes.build(ref.api, "cornell")
-    r = ref.renderer(m, fov, cam)
-    _, img = r.render(64, 48, 1)
+    sd = scene_data("cornell")
+    img = port.scene(sd.vtx, sd.tri, 64).render(sd.cam16, sd.fov, 64, 48, 1)["bgra"]
+
+    def ref_renderer(r):
+        m, fov, cam = pkg("scenes").build(r.api, "cornell")
+        return r.renderer(m, fov, cam)
+
+    ref_answers.check("port_render/cornell/64x48x1/bgra", img, lambda r: ref_renderer(r).render(64, 48, 1)[1])
     a, b = str(tmp_path / "ref.bmp"), str(tmp_path / "host.bmp")
-    r.save_bmp(a)
     assert hostlib.rtm_write_bitmap(b.encode(), 64, 48, img.ctypes.data_as(C.POINTER(C.c_uint32))) == 1
-    assert open(a, "rb").read() == open(b, "rb").read()
+
+    def ref_bmp(r):
+        rr = ref_renderer(r)
+        rr.render(64, 48, 1)
+        rr.save_bmp(a)
+        return np.fromfile(a, np.uint8)
+
+    ref_answers.check("save_bmp/cornell/64x48x1", np.fromfile(b, np.uint8), ref_bmp)

@@ -1,5 +1,6 @@
 """The C++ host mirror (Renderer : Framebuffer, Scene, Grid -- host/*.h) driven on one GPU and compared with the
-unmodified reference's classes of the same names (oracle/_ref), or with the committed digests when it is absent.
+unmodified reference's classes of the same names (oracle/_ref), or with the committed digests of their answers
+(tests/golden) when it is absent.
 
 Everything here goes Mesh -> Scene -> Renderer -> Resize/StartRendering -> WaitRendering -> tiles, i.e. the route a
 viewer using the reference's API takes (INTEGRATION.md route A)."""
@@ -29,16 +30,15 @@ def _ref_renderer(ref, name, grid_res=64):
 
 
 @pytest.mark.parametrize("name,w,h,spp", [("cornell", 200, 120, 4), ("killeroo", 333, 217, 2), ("head", 128, 128, 16)])
-def test_renderer_frame_matches_reference(ref, name, w, h, spp):
+def test_renderer_frame_matches_reference(ref_answers, name, w, h, spp):
     hr, _, _ = _host_renderer(name)
     sec, img = hr.render(w, h, spp)
     assert sec > 0 and hr.last_kernel_ms() > 0
-    _, want = _ref_renderer(ref, name).render(w, h, spp)
-    assert np.array_equal(img, want)
+    ref_answers.check("renderer/%s/%dx%dx%d" % (name, w, h, spp), img, lambda r: _ref_renderer(r, name).render(w, h, spp)[1])
     # a second frame at another size and sample count through the same Renderer (Resize path)
-    _, img2 = hr.render(w // 2 + 1, h // 2 + 3, 1)
-    _, want2 = _ref_renderer(ref, name).render(w // 2 + 1, h // 2 + 3, 1)
-    assert np.array_equal(img2, want2)
+    w2, h2 = w // 2 + 1, h // 2 + 3
+    _, img2 = hr.render(w2, h2, 1)
+    ref_answers.check("renderer/%s/%dx%dx1" % (name, w2, h2), img2, lambda r: _ref_renderer(r, name).render(w2, h2, 1)[1])
 
 
 def test_renderer_digest_without_reference():
@@ -55,37 +55,51 @@ def test_renderer_digest_without_reference():
     assert int(np.float32(gi["cell_wdh"]).view(np.uint32)) == d["cell_wdh_bits"]
 
 
-def test_save_bmp_byte_identical(ref, tmp_path):
+def test_save_bmp_byte_identical(ref_answers, tmp_path):
     hr, _, _ = _host_renderer("cornell")
     hr.render(96, 64, 2)
-    rr = _ref_renderer(ref, "cornell")
-    rr.render(96, 64, 2)
     a, b = str(tmp_path / "host.bmp"), str(tmp_path / "ref.bmp")
     hr.save_bmp(a)
-    rr.save_bmp(b)
-    with open(a, "rb") as fa, open(b, "rb") as fb:
-        assert fa.read() == fb.read()
+
+    def ref_bmp(r):
+        rr = _ref_renderer(r, "cornell")
+        rr.render(96, 64, 2)
+        rr.save_bmp(b)
+        return np.fromfile(b, np.uint8)
+
+    ref_answers.check("save_bmp/cornell/96x64x2", np.fromfile(a, np.uint8), ref_bmp)
 
 
-def test_grid_intersect_and_ray_march_single_ray(ref):
-    """Grid::Intersect (grid.cpp:208-334) and Renderer::RayMarch (renderer.cpp:24-41) as one-ray queries."""
+def test_grid_intersect_and_ray_march_single_ray(ref_answers, port):
+    """Grid::Intersect (grid.cpp:208-334) and Renderer::RayMarch (renderer.cpp:24-41) as one-ray queries.
+    Per queried ray: hit triangle (MISS if none), t / u / v bits (0 on a miss), march hit flag, march t bits."""
     hr, _, _ = _host_renderer("cornell")
-    rr = _ref_renderer(ref, "cornell")
-    o3, d3 = rr.generate_rays(16, 12, 1, 0, 12)
+    o3, d3 = ref_answers.rays(port, "cornell", 16, 12, 1, 0, 12)
     o, d = o3.reshape(-1, 3), d3.reshape(-1, 3)
-    idx, t, u, v = rr.intersect_rays(o, d)
-    mh, mt = rr.ray_march(o, d)
-    hits = 0
-    for i in range(0, len(o), 7):
+    sel = range(0, len(o), 7)
+    got = np.zeros((len(sel), 6), np.uint32)
+    for row, i in enumerate(sel):
         ok, tuv, tri = hr.intersect(o[i], d[i])
-        assert ok == (idx[i] != 0xFFFFFFFF)
+        got[row, 0] = tri if ok else 0xFFFFFFFF
         if ok:
-            hits += 1
-            assert tri == idx[i]
-            assert np.array_equal(tuv.view(np.uint32), np.array([t[i], u[i], v[i]], np.float32).view(np.uint32))
+            got[row, 1:4] = np.asarray(tuv, np.float32).view(np.uint32)
         got_hit, got_t = hr.ray_march(o[i], d[i])
-        assert got_hit == bool(mh[i]) and np.float32(got_t).view(np.uint32) == mt[i].view(np.uint32)
-    assert hits > 5
+        got[row, 4], got[row, 5] = int(bool(got_hit)), np.float32(got_t).view(np.uint32)
+
+    def want(r):
+        rr = _ref_renderer(r, "cornell")
+        idx, t, u, v = rr.intersect_rays(o, d)
+        mh, mt = rr.ray_march(o, d)
+        w = np.zeros_like(got)
+        for row, i in enumerate(sel):
+            w[row, 0] = idx[i]
+            if idx[i] != 0xFFFFFFFF:
+                w[row, 1:4] = np.array([t[i], u[i], v[i]], np.float32).view(np.uint32)
+            w[row, 4], w[row, 5] = int(bool(mh[i])), mt[i:i + 1].view(np.uint32)[0]
+        return w
+
+    ref_answers.check("intersect_and_march/cornell/16x12x1/every7", got, want)
+    assert int((got[:, 0] != 0xFFFFFFFF).sum()) > 5
 
 
 def test_renderer_alternates_match_port(port):
@@ -104,15 +118,22 @@ def test_renderer_alternates_match_port(port):
         assert np.array_equal(img, want), (ortho, mode)
 
 
-def test_grid_info_matches_reference(ref):
+def test_grid_info_matches_reference(ref_answers):
+    """Grid dimensions, reference count, cell size bits, bounding box bits: [dim x3, refs, cell_wdh, min x3, max x3]."""
+    def record(dim, refs, cell_wdh, mn, mx):
+        f32 = lambda a: np.asarray(a, np.float32).reshape(-1).view(np.uint32).astype(np.uint64)
+        return np.concatenate([np.asarray(dim, np.uint64), [np.uint64(refs)], f32(cell_wdh), f32(mn), f32(mx)])
+
     for name, res in (("killeroo", 64), ("room", 32)):
         hr, _, _ = _host_renderer(name, res)
         gi = hr.grid_info()
-        g = _ref_renderer(ref, name, res).grid()
-        assert np.array_equal(gi["dim"], g["dim"]) and gi["num_refs"] == len(g["tri_index"])
-        assert np.float32(gi["cell_wdh"]).view(np.uint32) == np.float32(g["cell_wdh"]).view(np.uint32)
-        for k in ("aabb_min", "aabb_max"):
-            assert np.array_equal(gi[k].view(np.uint32), np.asarray(g[k], np.float32).view(np.uint32))
+        got = record(gi["dim"], gi["num_refs"], gi["cell_wdh"], gi["aabb_min"], gi["aabb_max"])
+
+        def want(r):
+            g = _ref_renderer(r, name, res).grid()
+            return record(g["dim"], len(g["tri_index"]), g["cell_wdh"], g["aabb_min"], g["aabb_max"])
+
+        ref_answers.check("grid_info/%s/g%d" % (name, res), got, want)
 
 
 def test_tiles_into_gives_every_tile_its_own_buffer(scene_data, port):

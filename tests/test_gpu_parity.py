@@ -382,39 +382,41 @@ def test_shading_alternates(cuda_trace, port, scene_data, name, spp, shade_mode)
         assert not np.array_equal(img, live)
 
 
-def test_brute_force_self_check(cuda_trace, ref, port, scene_data):
+def test_brute_force_self_check(cuda_trace, ref_answers, port, scene_data):
     """Renderer::IntersectBruteForce on the device: bit-exact against the reference's own brute force, and
     -- the author's cross-check -- equal to the grid result except where the grid's in-cell rule decides."""
     sd = scene_data("cornell")
-    scenes = pkg("scenes")
-    m, fov, cam = scenes.build(ref.api, "cornell")
-    r = ref.renderer(m, fov, cam)
     cuda_trace.upload_scene(sd.vtx, sd.tri, 64)
-    o3, d3 = r.generate_rays(96, 64, 2, 0, 64)
+    o3, d3 = ref_answers.rays(port, "cornell", 96, 64, 2, 0, 64)
     o, d = o3.reshape(-1, 3), d3.reshape(-1, 3)
     bt = cuda_trace.intersect_rays_brute_force(o, d)
-    rt = r.intersect_rays_brute_force(o, d)
-    assert np.array_equal(bt[0], rt[0])
-    for i in (1, 2, 3):
-        assert np.array_equal(bt[i].view(np.uint32), rt[i].view(np.uint32))
+
+    def want(r):
+        m, fov, cam = pkg("scenes").build(r.api, "cornell")
+        rt = r.renderer(m, fov, cam).intersect_rays_brute_force(o, d)
+        return np.stack([rt[0]] + [rt[i].view(np.uint32) for i in (1, 2, 3)])
+
+    ref_answers.check("brute_force/cornell/96x64x2", np.stack([bt[0]] + [bt[i].view(np.uint32) for i in (1, 2, 3)]), want)
     gt = cuda_trace.intersect_rays(o, d, 0)
     assert (gt[0] != bt[0]).mean() < 0.01  # grid vs brute force: only boundary / tie cases differ
     assert (bt[0] != 0xFFFFFFFF).sum() > 1000
 
 
-def test_ray_march_matches_reference(cuda_trace, ref, scene_data):
+def test_ray_march_matches_reference(cuda_trace, ref_answers, port, scene_data):
     """Renderer::RayMarch + DistanceBruteForce + DistancePointTri on the device, bit-exact (hit flag and the
     parameter t reached) against the reference's own functions, on camera rays of the Cornell scene."""
     sd = scene_data("cornell")
-    scenes = pkg("scenes")
-    m, fov, cam = scenes.build(ref.api, "cornell")
-    r = ref.renderer(m, fov, cam)
     cuda_trace.upload_scene(sd.vtx, sd.tri, 64)
-    o3, d3 = r.generate_rays(48, 32, 1, 0, 32)
+    o3, d3 = ref_answers.rays(port, "cornell", 48, 32, 1, 0, 32)
     o, d = o3.reshape(-1, 3), d3.reshape(-1, 3)
     gh, gt = cuda_trace.ray_march(o, d)
-    rh, rt = r.ray_march(o, d)
-    assert np.array_equal(gh, rh) and np.array_equal(gt.view(np.uint32), rt.view(np.uint32))
+
+    def want(r):
+        m, fov, cam = pkg("scenes").build(r.api, "cornell")
+        rh, rt = r.renderer(m, fov, cam).ray_march(o, d)
+        return np.stack([np.asarray(rh, np.uint32), rt.view(np.uint32)])
+
+    ref_answers.check("ray_march/cornell/48x32x1", np.stack([np.asarray(gh, np.uint32), gt.view(np.uint32)]), want)
     assert 100 < int(gh.sum()) < len(gh)
 
 
@@ -461,27 +463,31 @@ def test_errors(cuda_trace, scene_data):
         capi.CudaTrace(devices=[99])
 
 
-def test_cost_ordered_split_frames_match_image_order(ref, scene_data):
+def test_cost_ordered_split_frames_match_image_order(ref_answers, scene_data):
     """Scheduling must never change results.  Frames 2.. of one layout run through the cost order of the previous
     frame, with its expensive strips split into pieces (csrc/schedule.cu); the camera moves between frames so a
     skipped piece cannot hide behind a stale pixel.  1080p / 16 spp: 128-ray strips, 4 pieces, order on by default;
     both the plain read-back and the overlapped per-band one (whose counters count pieces) are used."""
     capi, scenes = pkg("capi"), pkg("scenes")
+    api = ref_answers.api
     sd = scene_data("killeroo")
     w, h, spp = 1920, 1080, 16
-    fov_xs, aspect = ref.api.camera_constants(sd.fov, w, h)
+    fov_xs, aspect = api.camera_constants(sd.fov, w, h)
     cams = []
     for eye_x in (-1.6, -1.5, -1.4):
-        cams.append(ref.api.look_at((eye_x, 1.2, -1.0), (0.0, 0.0, -0.1)))
+        cams.append(api.look_at((eye_x, 1.2, -1.0), (0.0, 0.0, -0.1)))
     fresh = capi.CudaTrace(1)
     fresh.upload_scene(sd.vtx, sd.tri, 64)
     want = []
     for cam in cams:  # every frame in image order: a new layout (different tiles) in between invalidates the order
         fresh.trace_tiles(fresh.make_frame(64, 64, 1, cam, fov_xs, aspect))
         want.append(fresh.trace_tiles(fresh.make_frame(w, h, spp, cam, fov_xs, aspect)).copy())
-    m, fov, _ = scenes.build(ref.api, "killeroo")
-    _, ref_img = ref.renderer(m, fov, cams[0]).render(w, h, spp)
-    assert np.array_equal(want[0], ref_img)
+
+    def ref_frame(r):
+        m, fov, _ = scenes.build(r.api, "killeroo")
+        return r.renderer(m, fov, cams[0]).render(w, h, spp)[1]
+
+    ref_answers.check("renderer/killeroo_eye-1.6/%dx%dx%d" % (w, h, spp), want[0], ref_frame)
     fresh.close()
 
     ct = capi.CudaTrace(1)

@@ -1,5 +1,5 @@
 """CPU tests: the host library's Mesh / Matrix44f mirror against the unmodified reference
-(oracle/_ref), bit for bit.  Skipped where the reference could not be built."""
+(oracle/_ref, or the digests of its answers in tests/golden/ref_answers.json where it is not built), bit for bit."""
 import os
 
 import numpy as np
@@ -17,63 +17,80 @@ def bits(a):
     return np.ascontiguousarray(a, np.float32).view(np.uint32)
 
 
-def test_matrix_builders(host, ref):
-    r = ref.api
-    for deg in (0.0, 30.0, 45.0, 90.0, -17.5, 123.456, 360.0):
-        assert np.array_equal(bits(host.rotation_x(deg)), bits(r.rotation_x(deg)))
-        assert np.array_equal(bits(host.rotation_y(deg)), bits(r.rotation_y(deg)))
-        assert np.array_equal(bits(host.rotation_z(deg)), bits(r.rotation_z(deg)))
-    assert np.array_equal(bits(host.identity()), bits(r.identity()))
-    assert np.array_equal(bits(host.scaling(0.25)), bits(r.scaling(0.25)))
-    assert np.array_equal(bits(host.translation(-0.065, -0.1, 0.05)), bits(r.translation(-0.065, -0.1, 0.05)))
-    for eye, at in [((-1.00001, 1.0, 1.0), (0.0, -0.2, 0.0)), ((0, 0, -2), (0, 0, 0)), ((-0.47, 0.15, -0.3), (1.0, -0.7, 0.9)),
-                    ((-1.6, 1.2, -1.0), (0.0, 0.0, -0.1)), ((0.5, 0.5, 0.0), (0, 0, 0))]:
-        assert np.array_equal(bits(host.look_at(eye, at)), bits(r.look_at(eye, at)))
+def test_matrix_builders(host, ref_answers):
+    def run(api):
+        out = []
+        for deg in (0.0, 30.0, 45.0, 90.0, -17.5, 123.456, 360.0):
+            out += [api.rotation_x(deg), api.rotation_y(deg), api.rotation_z(deg)]
+        out += [api.identity(), api.scaling(0.25), api.translation(-0.065, -0.1, 0.05)]
+        for eye, at in [((-1.00001, 1.0, 1.0), (0.0, -0.2, 0.0)), ((0, 0, -2), (0, 0, 0)), ((-0.47, 0.15, -0.3), (1.0, -0.7, 0.9)),
+                        ((-1.6, 1.2, -1.0), (0.0, 0.0, -0.1)), ((0.5, 0.5, 0.0), (0, 0, 0))]:
+            out.append(api.look_at(eye, at))
+        return np.stack([bits(np.asarray(m).reshape(-1)) for m in out])
+
+    ref_answers.check("matrix_builders", run(host), lambda r: run(r.api))
 
 
-def test_matrix_multiply_and_invert_random(host, ref):
+def test_matrix_multiply_and_invert_random(host, ref_answers):
+    """Per case: the product's bits, the inverse's success flag and bits."""
     rs = np.random.RandomState(3)
+    cases = []
     for i in range(300):
         a = rs.normal(size=16).astype(np.float32) * np.float32(10.0 ** rs.randint(-3, 3))
         b = rs.normal(size=16).astype(np.float32)
-        assert np.array_equal(bits(host.multiply(a, b)), bits(ref.api.multiply(a, b)))
-        ok_h, inv_h = host.invert(a)
-        ok_r, inv_r = ref.api.invert(a)
-        assert ok_h == ok_r
-        assert np.array_equal(bits(inv_h), bits(inv_r))
+        cases.append((a, b))
+
+    def run(api):
+        out = np.zeros((len(cases), 33), np.uint32)
+        for i, (a, b) in enumerate(cases):
+            ok, inv = api.invert(a)
+            out[i, :16] = bits(api.multiply(a, b))
+            out[i, 16] = ok
+            out[i, 17:] = bits(inv)
+        return out
+
+    ref_answers.check("matrix_multiply_invert/300", run(host), lambda r: run(r.api))
     sing = np.zeros(16, np.float32)
-    assert host.invert(sing)[0] is False and ref.api.invert(sing)[0] is False
+    assert host.invert(sing)[0] is False
+    if ref_answers.ref is not None:
+        assert ref_answers.ref.api.invert(sing)[0] is False
 
 
-def test_camera_constants(host, ref, port):
-    for fov in (30.0, 45.0, 51.0, 60.0, 75.0, 90.0, 1.0, 179.0):
-        for w, h in ((512, 512), (1920, 1080), (3840, 2160), (67, 45)):
-            a = host.camera_constants(fov, w, h)
-            b = ref.api.camera_constants(fov, w, h)
-            c = port.camera_constants(fov, w, h)
-            assert bits(a[0]) == bits(b[0]) == bits(c[0]) and bits(a[1]) == bits(b[1]) == bits(c[1])
+def test_camera_constants(host, ref_answers, port):
+    def run(api):
+        out = []
+        for fov in (30.0, 45.0, 51.0, 60.0, 75.0, 90.0, 1.0, 179.0):
+            for w, h in ((512, 512), (1920, 1080), (3840, 2160), (67, 45)):
+                out.append(bits(np.asarray(api.camera_constants(fov, w, h), np.float32)))
+        return np.stack(out)
+
+    got = run(host)
+    assert np.array_equal(got, run(port))
+    ref_answers.check("camera_constants", got, lambda r: run(r.api))
 
 
-def test_cornell_box_and_quads(host, ref):
+def test_cornell_box_and_quads(host, ref_answers):
     hv, ht = host.mesh().cornell_box().arrays()
-    rv, rt = ref.api.mesh().cornell_box().arrays()
-    assert np.array_equal(hv.view(np.uint32), rv.view(np.uint32)) and np.array_equal(ht, rt)
     assert len(ht) == 32 and len(hv) == 64
+    ref_answers.check("cornell_box/vtx", hv.view(np.uint32), lambda r: r.api.mesh().cornell_box().arrays()[0].view(np.uint32))
+    ref_answers.check("cornell_box/tri", ht, lambda r: r.api.mesh().cornell_box().arrays()[1])
 
 
 @pytest.mark.parametrize("name", list(range(10)) + ["tiger_soup_small"])
-def test_scene_presets_bitwise(host, ref, name):
+def test_scene_presets_bitwise(host, ref_answers, name):
+    """Field of view and camera bits, triangles, vertex bits, bounding box bits of every preset."""
     scenes = pkg("scenes")
-    hm, hf, hc = scenes.build(host, name)
-    rm, rf, rc = scenes.build(ref.api, name)
-    assert hf == rf and np.array_equal(bits(hc), bits(rc))
-    hv, ht = hm.arrays()
-    rv, rt = rm.arrays()
-    assert np.array_equal(ht, rt)
-    assert np.array_equal(hv.view(np.uint32), rv.view(np.uint32))
-    ha, hb = hm.compute_aabb()
-    ra, rb = rm.compute_aabb()
-    assert np.array_equal(bits(ha), bits(ra)) and np.array_equal(bits(hb), bits(rb))
+
+    def run(api):
+        m, fov, cam = scenes.build(api, name)
+        v, t = m.arrays()
+        a, b = m.compute_aabb()
+        return [bits(np.concatenate([[fov], np.asarray(cam).reshape(-1), np.asarray(a).reshape(-1),
+                                     np.asarray(b).reshape(-1)])), np.ascontiguousarray(t), v.view(np.uint32)]
+
+    got = run(host)
+    for part, g in zip(("fov_cam_aabb", "tri", "vtx"), got):
+        ref_answers.check("scene/%s/%s" % (name, part), g, lambda r, part=part: dict(zip(("fov_cam_aabb", "tri", "vtx"), run(r.api)))[part])
 
 
 REF_MESH_DIR = "/root/reference/meshes"
@@ -97,7 +114,7 @@ def test_ascii_reader_matches_reference_and_assets(host, ref):
             assert np.array_equal(at, rt) and np.array_equal(av.view(np.uint32), rv.view(np.uint32)), name
 
 
-def test_float_parsing_matches_reference_on_hard_decimals(host, ref, tmp_path):
+def test_float_parsing_matches_reference_on_hard_decimals(host, ref_answers, tmp_path):
     """The host reader parses plain decimals on a fast exact path and leaves the rest to strtof (host/mesh.cpp);
     the reference uses fscanf("%f").  Positions written in every notation that occurs in practice plus the hard
     cases: float rounding midpoints spelled out exactly, one digit above / below them, 17+ significant digits,
@@ -118,12 +135,16 @@ def test_float_parsing_matches_reference_on_hard_decimals(host, ref, tmp_path):
     lines = [" ".join(vals[i:i + 3]) for i in range(0, len(vals), 3)]
     path = tmp_path / "hard.dat"
     path.write_text("\n".join(lines) + "\n")
-    hm, rm = host.mesh(), ref.api.mesh()
-    assert hm.read_file(str(path)) and rm.read_file(str(path))
-    hv, _ = hm.arrays()
-    rv, _ = rm.arrays()
-    assert len(hv) == len(vals) // 3
-    assert np.array_equal(hv[:, :3].view(np.uint32), rv[:, :3].view(np.uint32))
+
+    def run(api):
+        m = api.mesh()
+        assert m.read_file(str(path))
+        v, _ = m.arrays()
+        return np.ascontiguousarray(v[:, :3]).view(np.uint32)
+
+    got = run(host)
+    assert len(got) == len(vals) // 3
+    ref_answers.check("float_parsing/hard_decimals", got, lambda r: run(r.api))
 
 
 def test_reader_errors(host, tmp_path):
