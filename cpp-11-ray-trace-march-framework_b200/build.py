@@ -21,7 +21,7 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-fmad=false", "-prec-div=true", "-prec-sqrt=true", "-ftz=false",
               "-Xcompiler", "-fPIC,-O2,-ffp-contract=off", "-Xptxas", "-v"]
-CU_SOURCES = ["api.cu", "trace_kernels.cu", "pool_trace.cu", "pack.cu", "grid_build.cu", "schedule.cu", "qmc.cu"]
+CU_SOURCES = ["api.cu", "trace_kernels.cu", "ray_query.cu", "pool_trace.cu", "pack.cu", "grid_build.cu", "schedule.cu", "qmc.cu"]
 LIB_MEASURE = os.path.join(PKG, "libcuda_trace_measure.so")
 
 

@@ -14,6 +14,8 @@ LIB_PATH = os.path.join(PKG, "libcuda_trace.so")
 MISS = 0xFFFFFFFF
 VARIANT_MT = 0
 VARIANT_BARY = 1
+QUERY_CLOSEST = 0
+QUERY_OCCLUSION = 1
 FLAG_GAMMA = 1
 FLAG_KEEP_HITS = 2
 FLAG_ORTHO = 4              # camera.h:25-36; the frame's fov_xs then carries the width of the viewing volume
@@ -38,6 +40,13 @@ class GridDesc(C.Structure):
     _fields_ = [("dim", C.c_uint32 * 3), ("aabb_min", C.c_float * 3), ("aabb_max", C.c_float * 3),
                 ("cell_wdh", C.c_float), ("inv_cell_wdh", C.c_float), ("num_cells", C.c_uint64),
                 ("num_refs", C.c_uint64)]
+
+
+class RayBatch(C.Structure):
+    """cuda_trace_ray_batch: every pointer is device memory"""
+    _fields_ = [("n", C.c_uint32), ("kind", C.c_uint32), ("variant", C.c_uint32), ("t_max_all", C.c_float),
+                ("origins", C.c_void_p), ("dirs", C.c_void_p), ("t_max", C.c_void_p), ("tri_idx", C.c_void_p),
+                ("t", C.c_void_p), ("u", C.c_void_p), ("v", C.c_void_p), ("occluded", C.c_void_p)]
 
 
 class CountersC(C.Structure):
@@ -71,6 +80,7 @@ SYMBOLS = {
     "cuda_trace_intersect_rays": (C.c_int, [C.c_void_p, C.c_uint32, _F32P, _F32P, C.c_uint32, _U32P, _F32P,
                                             _F32P, _F32P]),
     "cuda_trace_mailbox_stats": (C.c_int, [C.c_void_p, _U64P, _U64P]),
+    "cuda_trace_query_rays": (C.c_int, [C.c_void_p, C.POINTER(RayBatch), C.c_void_p]),
     "cuda_trace_intersect_rays_brute_force": (C.c_int, [C.c_void_p, C.c_uint32, _F32P, _F32P, _U32P, _F32P, _F32P, _F32P]),
     "cuda_trace_band_shares": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32,
                                          _U32P, _U32P, _U32P, _U32P, _U32P]),
@@ -401,6 +411,58 @@ class CudaTrace:
         self._ck(self.lib.cuda_trace_intersect_rays(self.h, n, _p(o, _F32P), _p(d, _F32P), variant,
                                                     _p(tri, _U32P), _p(t, _F32P), _p(u, _F32P), _p(v, _F32P)))
         return tri, t, u, v
+
+    def query_rays(self, origins, dirs, t_max=None, occlusion=False, variant=VARIANT_MT, stream=None):
+        """cuda_trace_query_rays on torch CUDA tensors: origins / dirs float32 (n, 3) on the context's first device,
+        t_max None (unbounded), a float, or a float32 (n,) tensor.  Enqueued on ``stream`` (default: torch's current
+        stream) without waiting; the outputs are allocated on that stream.  -> (tri int32 with -1 on a miss, t, u, v)
+        for the closest hit, or a bool (n,) tensor for ``occlusion``."""
+        import torch
+        dev = torch.device("cuda", self.devices[0])
+
+        def check(x, name, shape):
+            if not isinstance(x, torch.Tensor):
+                raise TypeError("%s must be a torch tensor" % name)
+            if x.device != dev:
+                raise ValueError("%s must be on %s (got %s)" % (name, dev, x.device))
+            if x.dtype != torch.float32:
+                raise TypeError("%s must be float32 (got %s)" % (name, x.dtype))
+            if tuple(x.shape) != shape:
+                raise ValueError("%s must have shape %s (got %s)" % (name, shape, tuple(x.shape)))
+            return x.contiguous()
+
+        if not isinstance(origins, torch.Tensor) or origins.dim() != 2:
+            raise ValueError("origins must be a (n, 3) tensor")
+        n = origins.shape[0]
+        if n >= 2 ** 32:
+            raise ValueError("at most 2^32 - 1 rays per query")
+        stream = torch.cuda.current_stream(dev) if stream is None else stream
+        with torch.cuda.stream(stream):
+            o = check(origins, "origins", (n, 3))
+            d = check(dirs, "dirs", (n, 3))
+            b = RayBatch()
+            b.n, b.variant = n, int(variant)
+            b.kind = QUERY_OCCLUSION if occlusion else QUERY_CLOSEST
+            b.origins, b.dirs = o.data_ptr(), d.data_ptr()
+            tm = None
+            if isinstance(t_max, torch.Tensor):
+                tm = check(t_max, "t_max", (n,))
+                b.t_max, b.t_max_all = tm.data_ptr(), float("inf")
+            else:
+                b.t_max, b.t_max_all = None, float("inf") if t_max is None else float(t_max)
+            if occlusion:
+                occ = torch.empty(n, dtype=torch.bool, device=dev)  # written as 0 / 1 bytes
+                b.occluded = occ.data_ptr()
+                out = occ
+            else:
+                tri = torch.empty(n, dtype=torch.int32, device=dev)
+                t, u, v = (torch.empty(n, dtype=torch.float32, device=dev) for _ in range(3))
+                b.tri_idx, b.t, b.u, b.v = tri.data_ptr(), t.data_ptr(), u.data_ptr(), v.data_ptr()
+                out = (tri, t, u, v)
+            # torch's default stream is the legacy NULL stream, which the C call would read as "the context's
+            # stream": name it as cudaStreamLegacy (0x1) instead
+            self._ck(self.lib.cuda_trace_query_rays(self.h, C.byref(b), C.c_void_p(stream.cuda_stream or 1)))
+        return out
 
     def intersect_rays_brute_force(self, origins, dirs):
         o = np.ascontiguousarray(origins, np.float32).reshape(-1, 3)

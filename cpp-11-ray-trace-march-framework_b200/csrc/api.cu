@@ -194,6 +194,9 @@ struct cuda_trace_ctx
     bool marks_armed = false;
     uint32_t *pinned_cancel_src = nullptr;
 
+    // cuda_trace_query_rays: per stream the context has been given, an event behind its last query (device 0).
+    // Replacing the scene or destroying the context waits for them before the scene arrays are freed.
+    std::vector<std::pair<cudaStream_t, cudaEvent_t>> query_events;
 };
 
 namespace
@@ -227,6 +230,16 @@ void free_scene(DeviceState& d)
     d.d_pcell_start = nullptr; d.d_pcell_occ = nullptr; d.d_pcell_dist = nullptr;
     d.d_vtx = nullptr; d.d_tri = nullptr; d.d_cell_start = nullptr; d.d_cell_occ = nullptr;
     d.d_tri_index = nullptr; d.d_cell_tris = nullptr; d.d_cell_tris_b = nullptr; d.d_tri_normals = nullptr;
+}
+
+// Queries still running on their callers' streams read the scene arrays: wait for them before those are freed
+void wait_for_queries(cuda_trace_ctx *ctx)
+{
+    if (ctx->dev.empty())
+        return;
+    cudaSetDevice(ctx->dev[0].ordinal);
+    for (auto& se : ctx->query_events)
+        cudaEventSynchronize(se.second);
 }
 
 GridDev grid_dev(const cuda_trace_ctx *ctx, const DeviceState& d)
@@ -589,6 +602,9 @@ void cuda_trace_destroy(cuda_trace_ctx *ctx)
         if (d.copy_stream && !ctx->shard_signals) cudaStreamSynchronize(d.copy_stream);
         if (d.order_stream) cudaStreamSynchronize(d.order_stream);
     }
+    wait_for_queries(ctx);
+    for (auto& se : ctx->query_events)
+        cudaEventDestroy(se.second);
     if (!ctx->dev.empty())
     {
         cudaSetDevice(ctx->dev[0].ordinal);
@@ -662,6 +678,7 @@ int cuda_trace_upload_scene(cuda_trace_ctx *ctx, const float *vertices, uint32_t
         return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene: grid_res must be > 0 (grid.cpp:16)");
     if ((rc = cuda_trace_sync(ctx)))
         return rc;
+    wait_for_queries(ctx);
     ctx->have_scene = false;
     ctx->num_vtx = num_vertices;
     ctx->num_tri = num_triangles;
@@ -727,6 +744,7 @@ int cuda_trace_upload_scene_with_grid(cuda_trace_ctx *ctx, const float *vertices
             return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene_with_grid: triangle index out of bounds");
     if ((rc = cuda_trace_sync(ctx)))
         return rc;
+    wait_for_queries(ctx);
     ctx->have_scene = false;
     ctx->num_vtx = num_vertices;
     ctx->num_tri = num_triangles;
@@ -1089,42 +1107,52 @@ void fill_camera(const cuda_trace_ctx *ctx, const cuda_trace_frame *f, const Fra
     std::memcpy(&p.pk_minus_one, minus_one, sizeof(p.pk_minus_one));
 }
 
-// Where the padded occupancy map is read from (warp_trace.cuh): one byte per cell in shared memory when that leaves
-// room (<= 160 KB), else bits in shared memory, else bits through L1.  Tiny frames skip the per-CTA staging.
+// Where the padded occupancy map is read from (warp_trace.cuh), for frames and ray queries alike: when staging is
+// worth it (smem_ok), one byte per cell in shared memory when that leaves room (<= 160 KB next to `other_smem` bytes
+// the kernel also needs), else bits in shared memory; otherwise the distance map through L1 where the scene has one,
+// else bits through L1.  RTM_OCC_MODE overrides the choice where the forced home exists and fits.
+void choose_occupancy_home(const cuda_trace_ctx *ctx, const DeviceState& d, bool smem_ok, size_t other_smem,
+                           uint32_t& occ_mode, uint32_t& occ_smem_words)
+{
+    const uint64_t pcells = (uint64_t) (ctx->desc.dim[0] + 2) * (ctx->desc.dim[1] + 2) * (ctx->desc.dim[2] + 2);
+    const uint64_t bit_words = (pcells + 31) / 32, byte_words = (pcells + 3) / 4;
+    occ_mode = kOccGlobalBits;
+    occ_smem_words = 0;
+    if (smem_ok)
+    {
+        if (byte_words * 4 + other_smem <= 160 * 1024)
+        {
+            occ_mode = kOccSmemBytes;
+            occ_smem_words = (uint32_t) byte_words;
+        }
+        else if (bit_words * 4 + other_smem <= 160 * 1024)
+        {
+            occ_mode = kOccSmemBits;
+            occ_smem_words = (uint32_t) bit_words;
+        }
+    }
+    if (occ_mode == kOccGlobalBits && d.d_pcell_dist && ctx->tune.occ_mode < 0)
+        occ_mode = kOccGlobalDist; // too large for shared memory: distance map through L1
+    const int m = ctx->tune.occ_mode;
+    if (m == kOccGlobalBits) { occ_mode = kOccGlobalBits; occ_smem_words = 0; }
+    if (m == kOccGlobalDist && d.d_pcell_dist) { occ_mode = kOccGlobalDist; occ_smem_words = 0; }
+    if (m == kOccSmemBits && bit_words * 4 + other_smem <= 200 * 1024) { occ_mode = kOccSmemBits; occ_smem_words = (uint32_t) bit_words; }
+    if (m == kOccSmemBytes && byte_words * 4 + other_smem <= 200 * 1024) { occ_mode = kOccSmemBytes; occ_smem_words = (uint32_t) byte_words; }
+}
+
+// Occupancy map: choose_occupancy_home, staged only for frames of >= 4 M rays (tiny frames skip the per-CTA staging).
 // CTA size: one 1024-thread CTA per SM measured best on every config (32 warps share one staged occupancy map and
 // pull neighbouring strips, which keeps the triangle records of that screen region in L1); small frames use
 // smaller CTAs so that every SM gets work.
 int choose_cta(const cuda_trace_ctx *ctx, const DeviceState& d, const cuda_trace_frame *f, uint64_t strips_here, TraceParams& p)
 {
     int threads = 1024;
-    const uint64_t pcells = (uint64_t) (ctx->desc.dim[0] + 2) * (ctx->desc.dim[1] + 2) * (ctx->desc.dim[2] + 2);
-    const uint64_t bit_words = (pcells + 31) / 32, byte_words = (pcells + 3) / 4;
     const uint64_t rays = (uint64_t) f->width * f->height * f->spp;
     const size_t smp_bytes = sizeof(float2) * f->spp;
     while (threads > 64 && strips_here < (uint64_t) d.sm_count * (threads / 32))
         threads /= 2;
-    p.occ_mode = kOccGlobalBits;
-    p.occ_smem_words = 0;
-    if (ctx->occ_in_smem && rays >= (4u << 20) && threads == 1024)
-    {
-        if (byte_words * 4 + smp_bytes <= 160 * 1024)
-        {
-            p.occ_mode = kOccSmemBytes;
-            p.occ_smem_words = (uint32_t) byte_words;
-        }
-        else if (bit_words * 4 + smp_bytes <= 160 * 1024)
-        {
-            p.occ_mode = kOccSmemBits;
-            p.occ_smem_words = (uint32_t) bit_words;
-        }
-    }
-    if (p.occ_mode == kOccGlobalBits && d.d_pcell_dist && ctx->tune.occ_mode < 0)
-        p.occ_mode = kOccGlobalDist; // too large for shared memory: distance map through L1
-    const int m = ctx->tune.occ_mode;
-    if (m == kOccGlobalBits) { p.occ_mode = kOccGlobalBits; p.occ_smem_words = 0; }
-    if (m == kOccGlobalDist && d.d_pcell_dist) { p.occ_mode = kOccGlobalDist; p.occ_smem_words = 0; }
-    if (m == kOccSmemBits && bit_words * 4 + smp_bytes <= 200 * 1024) { p.occ_mode = kOccSmemBits; p.occ_smem_words = (uint32_t) bit_words; }
-    if (m == kOccSmemBytes && byte_words * 4 + smp_bytes <= 200 * 1024) { p.occ_mode = kOccSmemBytes; p.occ_smem_words = (uint32_t) byte_words; }
+    choose_occupancy_home(ctx, d, ctx->occ_in_smem && rays >= (4u << 20) && threads == 1024, smp_bytes, p.occ_mode,
+                          p.occ_smem_words);
     if (ctx->tune.threads)
         threads = ctx->tune.threads;
     // |det| <= |e1| |e2| |d| <= 3 extent^2: below 1e14 the reciprocal's fast path is always valid
@@ -1880,6 +1908,39 @@ int cuda_trace_download_hits(cuda_trace_ctx *ctx, uint32_t *tri_idx, float *t, f
     return 0;
 }
 
+// Enqueue a checked query batch (all pointers device memory of d) on stream s
+static void launch_query(cuda_trace_ctx *ctx, const DeviceState& d, const cuda_trace_ray_batch& b, cudaStream_t s)
+{
+    const bool occlusion = b.kind == CUDA_TRACE_QUERY_OCCLUSION;
+    RayQueryParams p;
+    p.grid = grid_dev(ctx, d);
+    p.grid.pair_recs_rel = nullptr; // rewritten by frames per camera: never read by queries
+    p.n = b.n;
+    p.origins = b.origins;
+    p.dirs = b.dirs;
+    p.t_max = b.t_max;
+    p.t_max_all = b.t_max_all;
+    p.tri = occlusion ? nullptr : b.tri_idx;
+    p.t = occlusion ? nullptr : b.t;
+    p.u = occlusion ? nullptr : b.u;
+    p.v = occlusion ? nullptr : b.v;
+    p.occluded = occlusion ? b.occluded : nullptr;
+    // no sample table: the shared-memory budget is the map alone
+    choose_occupancy_home(ctx, d, ctx->occ_in_smem, 0, p.occ_mode, p.occ_smem_words);
+    const auto ordinary = [](float x) { return std::fabs(x) >= 0x1p-20f && std::fabs(x) <= 0x1p20f; };
+    p.fast_math = (ctx->fast_math && ordinary(ctx->desc.cell_wdh)) ? 1u : 0u;
+    const float one[2] = { 1.0f, 1.0f }, minus_one[2] = { -1.0f, -1.0f };
+    std::memcpy(&p.pk_one, one, sizeof(p.pk_one));
+    std::memcpy(&p.pk_minus_one, minus_one, sizeof(p.pk_minus_one));
+    // t_max == +inf for all rays is Grid::Intersect itself: the unbounded instantiation (K1's work per ray)
+    const bool bounded = b.t_max != nullptr || !(b.t_max_all == INFINITY);
+    // persistent CTAs, one per SM (the map is staged once per CTA), fewer for small batches
+    const int threads = ray_query_threads();
+    const uint64_t ctas = (b.n + threads - 1) / threads;
+    const int blocks = (int) std::min<uint64_t>(ctas, (uint64_t) d.sm_count);
+    launch_ray_query(p, b.variant, occlusion, bounded, blocks, s);
+}
+
 static int intersect_rays_impl(cuda_trace_ctx *ctx, uint32_t n, const float *origins, const float *dirs, uint32_t variant,
                                bool brute_force, uint32_t *tri_idx, float *t, float *u, float *v)
 {
@@ -1896,40 +1957,63 @@ static int intersect_rays_impl(cuda_trace_ctx *ctx, uint32_t n, const float *ori
     CK(cudaSetDevice(d.ordinal));
     float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr, *d_u = nullptr, *d_v = nullptr;
     uint32_t *d_i = nullptr;
-    CK(cudaMalloc(&d_o, (size_t) n * 12)); CK(cudaMalloc(&d_d, (size_t) n * 12));
-    CK(cudaMalloc(&d_t, (size_t) n * 4)); CK(cudaMalloc(&d_u, (size_t) n * 4));
-    CK(cudaMalloc(&d_v, (size_t) n * 4)); CK(cudaMalloc(&d_i, (size_t) n * 4));
+    unsigned long long *d_stats = nullptr;
+    // every return below, failures included, frees the temporaries -- after the stream has drained, because a
+    // failed call may leave copies or the kernel enqueued
+    struct Temporaries
+    {
+        DeviceState& d;
+        std::array<void *, 7> p;
+        ~Temporaries()
+        {
+            cudaStreamSynchronize(d.stream);
+            for (void *q : p)
+                cudaFree(q);
+        }
+    } temps{ d, {} };
+    CK(cudaMalloc(&d_o, (size_t) n * 12)); temps.p[0] = d_o;
+    CK(cudaMalloc(&d_d, (size_t) n * 12)); temps.p[1] = d_d;
+    CK(cudaMalloc(&d_t, (size_t) n * 4)); temps.p[2] = d_t;
+    CK(cudaMalloc(&d_u, (size_t) n * 4)); temps.p[3] = d_u;
+    CK(cudaMalloc(&d_v, (size_t) n * 4)); temps.p[4] = d_v;
+    CK(cudaMalloc(&d_i, (size_t) n * 4)); temps.p[5] = d_i;
     CK(cudaMemcpyAsync(d_o, origins, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
     CK(cudaMemcpyAsync(d_d, dirs, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
     RayBatchParams p;
     p.grid = grid_dev(ctx, d);
     p.n = n; p.origins = d_o; p.dirs = d_d; p.tri = d_i; p.t = d_t; p.u = d_u; p.v = d_v;
     p.mailbox_stats = nullptr;
-    unsigned long long *d_stats = nullptr;
     if (mailbox)
     {
         CK(cudaMalloc(&d_stats, 2 * sizeof(unsigned long long)));
+        temps.p[6] = d_stats;
         CK(cudaMemsetAsync(d_stats, 0, 2 * sizeof(unsigned long long), d.stream));
         p.mailbox_stats = d_stats;
     }
     if (brute_force)
         launch_brute_force(d.d_vtx, d.d_tri, ctx->num_tri, p, d.stream);
+    else if (mailbox)
+        launch_intersect_rays(p, variant, d.stream);
     else
-        launch_intersect_rays(p, variant, mailbox, d.stream);
+    {
+        // the warp-cooperative query kernel: the same bits, faster on every workload (profiles/r03_ray_query.txt)
+        cuda_trace_ray_batch q = {};
+        q.n = n; q.kind = CUDA_TRACE_QUERY_CLOSEST; q.variant = variant; q.t_max_all = INFINITY;
+        q.origins = d_o; q.dirs = d_d; q.tri_idx = d_i; q.t = d_t; q.u = d_u; q.v = d_v;
+        launch_query(ctx, d, q, d.stream);
+    }
     ctx->launches++;
     CK(cudaGetLastError());
     if (mailbox)
     {
         CK(cudaMemcpyAsync(ctx->mailbox_stats, d_stats, sizeof(ctx->mailbox_stats), cudaMemcpyDeviceToHost, d.stream));
         CK(cudaStreamSynchronize(d.stream));
-        cudaFree(d_stats);
     }
     CK(cudaMemcpyAsync(tri_idx, d_i, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
     CK(cudaMemcpyAsync(t, d_t, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
     CK(cudaMemcpyAsync(u, d_u, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
     CK(cudaMemcpyAsync(v, d_v, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
     CK(cudaStreamSynchronize(d.stream));
-    cudaFree(d_o); cudaFree(d_d); cudaFree(d_t); cudaFree(d_u); cudaFree(d_v); cudaFree(d_i);
     return 0;
 }
 
@@ -1953,6 +2037,78 @@ int cuda_trace_intersect_rays_brute_force(cuda_trace_ctx *ctx, uint32_t n, const
                                           uint32_t *tri_idx, float *t, float *u, float *v)
 {
     return intersect_rays_impl(ctx, n, origins, dirs, 0, true, tri_idx, t, u, v);
+}
+
+int cuda_trace_query_rays(cuda_trace_ctx *ctx, const cuda_trace_ray_batch *b, void *stream)
+{
+    if (!ctx)
+        return CUDA_TRACE_ERR_ARG;
+    std::lock_guard<std::recursive_mutex> guard(ctx->api_mtx);
+    if (!b)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "query_rays: batch is NULL");
+    if (b->kind != CUDA_TRACE_QUERY_CLOSEST && b->kind != CUDA_TRACE_QUERY_OCCLUSION)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "query_rays: kind must be CUDA_TRACE_QUERY_CLOSEST or _OCCLUSION");
+    if (b->variant & CUDA_TRACE_VARIANT_MAILBOX)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "query_rays: mailboxing is a mode of cuda_trace_intersect_rays only");
+    if (b->variant != CUDA_TRACE_VARIANT_MT && b->variant != CUDA_TRACE_VARIANT_BARY)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "query_rays: variant must be CUDA_TRACE_VARIANT_MT or _BARY");
+    const bool occlusion = b->kind == CUDA_TRACE_QUERY_OCCLUSION;
+    if (b->n && (!b->origins || !b->dirs))
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "query_rays: origins and dirs are required");
+    if (b->n && (occlusion ? !b->occluded : !b->tri_idx))
+        return fail(ctx, CUDA_TRACE_ERR_ARG, occlusion ? "query_rays: an occlusion query needs `occluded`"
+                                                       : "query_rays: a closest-hit query needs `tri_idx`");
+    if (!ctx->have_scene)
+        return fail(ctx, CUDA_TRACE_ERR_NO_SCENE, "query_rays: upload a scene first");
+    if (b->n == 0)
+        return 0;
+    DeviceState& d = ctx->dev[0];
+    CK(cudaSetDevice(d.ordinal));
+    // every buffer must be device (or managed) memory of device 0: nothing is staged through the host
+    const void *ptrs[8] = { b->origins, b->dirs, b->t_max };
+    const char *names[8] = { "origins", "dirs", "t_max" };
+    int n_ptrs = 3;
+    if (occlusion)
+    {
+        ptrs[n_ptrs] = b->occluded; names[n_ptrs++] = "occluded";
+    }
+    else
+    {
+        ptrs[n_ptrs] = b->tri_idx; names[n_ptrs++] = "tri_idx";
+        ptrs[n_ptrs] = b->t; names[n_ptrs++] = "t";
+        ptrs[n_ptrs] = b->u; names[n_ptrs++] = "u";
+        ptrs[n_ptrs] = b->v; names[n_ptrs++] = "v";
+    }
+    for (int k = 0; k < n_ptrs; k++)
+    {
+        if (!ptrs[k])
+            continue; // optional and absent
+        cudaPointerAttributes a;
+        const cudaError_t e = cudaPointerGetAttributes(&a, ptrs[k]);
+        if (e != cudaSuccess)
+            cudaGetLastError(); // not sticky: clear it so that the next call does not report it
+        if (e != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) ||
+            a.device != d.ordinal)
+            return fail(ctx, CUDA_TRACE_ERR_ARG, std::string("query_rays: ") + names[k] +
+                                                     " is not device memory of the context's device " +
+                                                     std::to_string(d.ordinal));
+    }
+    cudaStream_t s = stream ? (cudaStream_t) stream : d.stream;
+    launch_query(ctx, d, *b, s);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    // remember the stream so that freeing the scene waits for this query
+    cudaEvent_t ev = nullptr;
+    for (auto& se : ctx->query_events)
+        if (se.first == s)
+            ev = se.second;
+    if (!ev)
+    {
+        CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        ctx->query_events.emplace_back(s, ev);
+    }
+    CK(cudaEventRecord(ev, s));
+    return 0;
 }
 
 int cuda_trace_ray_march(cuda_trace_ctx *ctx, uint32_t n, const float *origins, const float *dirs, uint32_t *hit, float *t)

@@ -255,7 +255,7 @@ __global__ void __launch_bounds__(kTraceMaxThreads) trace_pool_kernel(const __gr
             generate_ray<false>(p.cam, px, py, off.x, off.y, o_ray, d);
             const uint32_t k = (py * p.width + px) * p.spp + s; // (< 2^32: checked by the launcher)
             bool active;
-            float n0, n1, n2, dl0, dl1, dl2;
+            float enter_t, n0, n1, n2, dl0, dl1, dl2;
             int c0, c1, c2, pc;
 #include "dda_setup.inc"
             if (valid && !active)

@@ -590,19 +590,15 @@ int trace_tiles_max_blocks_per_sm(uint32_t variant, bool keep_hits, bool count, 
     RTM_DISPATCH(occupancy_one, occ_mode, threads, smem_bytes);
 }
 
-void launch_intersect_rays(const RayBatchParams& p, uint32_t variant, bool mailbox, cudaStream_t stream)
+void launch_intersect_rays(const RayBatchParams& p, uint32_t variant, cudaStream_t stream)
 {
     const uint32_t blocks = (p.n + 127) / 128;
     if (blocks == 0)
         return;
-    if (variant && mailbox)
+    if (variant)
         intersect_rays_kernel<1, true><<<blocks, 128, 0, stream>>>(p);
-    else if (variant)
-        intersect_rays_kernel<1, false><<<blocks, 128, 0, stream>>>(p);
-    else if (mailbox)
-        intersect_rays_kernel<0, true><<<blocks, 128, 0, stream>>>(p);
     else
-        intersect_rays_kernel<0, false><<<blocks, 128, 0, stream>>>(p);
+        intersect_rays_kernel<0, true><<<blocks, 128, 0, stream>>>(p);
 }
 
 void launch_brute_force(const float *vtx, const uint32_t *tri, uint32_t num_tri, const RayBatchParams& p, cudaStream_t stream)

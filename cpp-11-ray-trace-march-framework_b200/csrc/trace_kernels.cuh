@@ -115,6 +115,23 @@ struct RayBatchParams
     unsigned long long *mailbox_stats; // mailbox mode: [0] tests asked for, [1] answered from the mailbox (or null)
 };
 
+// cuda_trace_query_rays (ray_query.cu): every pointer is device memory; tri / occluded by kind, t / u / v optional
+struct RayQueryParams
+{
+    GridDev grid;
+    uint64_t n;
+    const float *origins, *dirs; // n x 3
+    const float *t_max;          // n, or null: t_max_all for every ray
+    float t_max_all;
+    uint32_t *tri;               // closest hit
+    float *t, *u, *v;
+    uint8_t *occluded;           // occlusion
+    uint32_t occ_mode;           // as TraceParams
+    uint32_t occ_smem_words;
+    uint32_t fast_math;          // the range-check-free DDA set-up may be used (rays with |dir| <= 1, voted per warp)
+    unsigned long long pk_one, pk_minus_one;
+};
+
 void launch_trace_tiles(const TraceParams& p, uint32_t variant, bool keep_hits, bool count, int grid_blocks,
                         int threads, cudaStream_t stream);
 int trace_tiles_max_blocks_per_sm(uint32_t variant, bool keep_hits, bool count, int occ_mode, int threads,
@@ -124,7 +141,13 @@ size_t trace_tiles_smem_bytes(uint32_t spp, uint32_t occ_smem_words);
 // (all four required); follow it with launch_trace_tiles(variant = kVariantFromHits) on the same stream
 void launch_trace_pool(const TraceParams& p, int grid_blocks, int threads, cudaStream_t stream);
 size_t trace_pool_smem_bytes(uint32_t spp, int threads);
-void launch_intersect_rays(const RayBatchParams& p, uint32_t variant, bool mailbox, cudaStream_t stream);
+// the scalar one-thread-per-ray walk, kept for the mailboxing mode of cuda_trace_intersect_rays (the plain mode runs
+// launch_ray_query)
+void launch_intersect_rays(const RayBatchParams& p, uint32_t variant, cudaStream_t stream);
+// bounded: the t_max rules apply (t_max given per ray or finite); occlusion queries always run bounded
+void launch_ray_query(const RayQueryParams& p, uint32_t variant, bool occlusion, bool bounded, int grid_blocks,
+                      cudaStream_t stream);
+int ray_query_threads(); // CTA size of launch_ray_query
 void launch_sample_table(float2 *smp, uint32_t spp, cudaStream_t stream);
 void launch_ray_march(const float *vtx, const uint32_t *tri, uint32_t num_tri, uint32_t n, const float *origins,
                       const float *dirs, uint32_t *hit, float *t, cudaStream_t stream);

@@ -202,6 +202,45 @@ int cuda_trace_download_hits(cuda_trace_ctx *ctx, uint32_t *tri_idx, float *t, f
 int cuda_trace_intersect_rays(cuda_trace_ctx *ctx, uint32_t n, const float *origins, const float *dirs,
                               uint32_t variant, uint32_t *tri_idx, float *t, float *u, float *v);
 
+/* ---- ray queries on rays that already live on the GPU -------------------------------------------
+ * No counterpart in the reference: Grid::Intersect (grid.cpp:159-281) for a batch of caller rays in device memory,
+ * bounded by t_max, plus a yes/no occlusion answer (shadow rays, ambient occlusion, picking, rays built on the GPU).
+ *
+ * Closest hit, bounded: the reference walk with two changes --
+ *   1. a triangle is accepted in a cell only if  hit && t < best && t < next_crossing_t[step_axis] && t < t_max;
+ *   2. the walk ends as a miss at the first cell the ray enters through a crossing greater than t_max (the first
+ *      cell's entry is the box entry, 0 for an origin inside the box).
+ * Only occupied cells are affected by rule 2, so every occupancy-map mode gives the same bits.  Consequences:
+ *   - t_max = +INFINITY gives exactly Grid::Intersect (and cuda_trace_intersect_rays); the crossing test is strict,
+ *     so an infinite crossing (delta overflowing on an unnormalised direction) does not end the walk;
+ *   - t_max <= 0 or NaN gives a miss;
+ *   - the result equals "the unbounded hit, kept if t < t_max" except for one floating-point corner of the grid
+ *     build: a triangle the grid registers only in cells entered after t_max can still be hit at t < t_max, and
+ *     the bounded walk, which stops before those cells, reports a miss.
+ * Occlusion: occluded[i] = 1 exactly when the bounded closest-hit query with the same t_max hits.  Acceptance does
+ * not depend on earlier hits before the first one, so the first accepted triangle decides (any-hit exit).
+ *
+ * Variants: CUDA_TRACE_VARIANT_MT or CUDA_TRACE_VARIANT_BARY; CUDA_TRACE_VARIANT_MAILBOX is refused (ERR_ARG). */
+#define CUDA_TRACE_QUERY_CLOSEST   0u
+#define CUDA_TRACE_QUERY_OCCLUSION 1u
+typedef struct cuda_trace_ray_batch
+{
+    uint32_t n, kind, variant;       /* rays, CUDA_TRACE_QUERY_*, CUDA_TRACE_VARIANT_MT / _BARY                  */
+    float    t_max_all;              /* used when t_max == NULL; INFINITY = unbounded                            */
+    const float *origins, *dirs;     /* DEVICE memory, n x 3 float, contiguous                                   */
+    const float *t_max;              /* DEVICE, n, or NULL                                                       */
+    uint32_t *tri_idx;               /* CLOSEST: DEVICE, n, required; CUDA_TRACE_MISS on a miss                  */
+    float *t, *u, *v;                /* CLOSEST: DEVICE, n, each may be NULL (0 on a miss)                       */
+    uint8_t *occluded;               /* OCCLUSION: DEVICE, n, required (0 / 1)                                   */
+} cuda_trace_ray_batch;
+/* Enqueues the query on `stream` (a cudaStream_t of the context's device 0; NULL = cuda_trace_stream(ctx)) and
+ * returns: no host synchronisation, no allocation.  Every pointer must be device or managed memory of device 0
+ * (checked with cudaPointerGetAttributes); otherwise, and for a bad kind / variant, the MAILBOX bit, a missing
+ * required output or n > 0 with NULL inputs, CUDA_TRACE_ERR_ARG is returned and nothing is enqueued.  No scene:
+ * CUDA_TRACE_ERR_NO_SCENE.  Queries read only immutable scene arrays, so they may overlap a frame; replacing the
+ * scene or destroying the context first waits for the queries already enqueued. */
+int cuda_trace_query_rays(cuda_trace_ctx *ctx, const cuda_trace_ray_batch *b, void *stream);
+
 /* After a CUDA_TRACE_VARIANT_MAILBOX call: ray/triangle tests the walk asked for, and how many of them the
  * mailbox answered */
 int cuda_trace_mailbox_stats(cuda_trace_ctx *ctx, uint64_t *tests, uint64_t *reused);

@@ -8,6 +8,10 @@
  *                          csrc/rt_device.cuh): 4 entries, round-robin over the tests actually computed -- returns the
  *                          hit and counts tests asked for / answered from the mailbox (tests/test_mailbox_model_cpu.py
  *                          checks that results equal the plain walk and that the counts equal what the GPU reported)
+ *   rts_bounded_walk       the walk bounded by t_max of the product's ray queries (cuda_trace_query_rays, include/
+ *   rts_query_rays         cuda_trace.h): rto_grid_intersect with its rules 1 and 2; a batch entry for the tests
+ *                          (tests/test_ray_query_cpu.py, tests/test_gpu_ray_query.py).  The oracle's own walk stays
+ *                          the reference's and nothing else, so this one lives here
  *   rts_study_ray          mailbox study  -- how often a ray re-tests a triangle it has tested within its last
  *                                            2 / 8 / 64 tests (the author's "mailboxing" TODO, grid.cpp:172)
  *                          pre-test study -- a conservative sphere reject in front of Moeller-Trumbore: the ray
@@ -237,4 +241,102 @@ int rts_mailbox_walk(const rto_scene *sc, const float *origin, const float *dir,
         next_t[sa] += delta_t[sa];
     }
     return 0;
+}
+
+/* rto_grid_intersect (grid.cpp:159-281) bounded by t_max:
+ *   rule 1  a triangle is accepted only if also t < t_max;
+ *   rule 2  the walk ends as a miss at the first OCCUPIED cell entered through a crossing greater than t_max (the
+ *           first cell's entry is enter_t; every later cell's is the next_t[sa] of the step that entered it).
+ * Returns 1 on a hit, 0 on a miss, 2 on a miss decided by rule 2. */
+int rts_bounded_walk(const rto_scene *sc, const float *origin, const float *dir, int variant, float t_max, float *t,
+                     float *u, float *v, uint32_t *tri_idx)
+{
+    const rto_grid *g = &sc->grid;
+    float enter_t, leave_t, gi[3];
+    if (rto_point_in_aabb(origin, g->aabb_min, g->aabb_max))
+    {
+        enter_t = 0.0f;
+        gi[0] = origin[0]; gi[1] = origin[1]; gi[2] = origin[2];
+    }
+    else if (rto_ray_aabb(origin, dir, g->aabb_min, g->aabb_max, &enter_t, &leave_t))
+    {
+        gi[0] = origin[0] + dir[0] * enter_t;
+        gi[1] = origin[1] + dir[1] * enter_t;
+        gi[2] = origin[2] + dir[2] * enter_t;
+    }
+    else
+        return 0;
+    float next_t[3], delta_t[3] = { 0.0f, 0.0f, 0.0f };
+    int step[3] = { 1, 1, 1 }, out[3], pos[3];
+    for (int a = 0; a < 3; a++)
+    {
+        out[a] = (int) g->dim[a];
+        pos[a] = to_voxel(g, gi, a);
+        if (dir[a] == 0.0f)
+            next_t[a] = FLT_MAX;
+        else if (dir[a] > 0.0f)
+        {
+            next_t[a] = enter_t + (to_pos(g, pos[a] + 1, a) - gi[a]) / dir[a];
+            delta_t[a] = g->cell_wdh / dir[a];
+        }
+        else
+        {
+            next_t[a] = enter_t + (to_pos(g, pos[a], a) - gi[a]) / dir[a];
+            delta_t[a] = -g->cell_wdh / dir[a];
+            step[a] = -1;
+            out[a] = -1;
+        }
+    }
+    float entry = enter_t;
+    *t = FLT_MAX;
+    for (;;)
+    {
+        const int sa = (next_t[0] < next_t[1]) ? ((next_t[0] < next_t[2]) ? 0 : 2) : ((next_t[1] < next_t[2]) ? 1 : 2);
+        const uint64_t cell = (uint64_t) pos[0] + (uint64_t) pos[2] * g->dim[0] + (uint64_t) pos[1] * g->dim[0] * g->dim[2];
+        if (g->cell_offset[cell] != g->cell_offset[cell + 1] && entry > t_max)
+            return 2;
+        for (uint64_t k = g->cell_offset[cell]; k < g->cell_offset[cell + 1]; k++)
+        {
+            const uint32_t ci = g->tri_index[k];
+            const uint32_t *tr = sc->tri + (size_t) ci * 6;
+            const float *v0 = sc->vtx + (size_t) tr[0] * 6, *v1 = sc->vtx + (size_t) tr[1] * 6, *v2 = sc->vtx + (size_t) tr[2] * 6;
+            float ct, cu, cv;
+            const int hit = variant == RTO_VARIANT_BARY
+                                ? rto_ray_tri_bary(origin, dir, v0, v1, v2, (const float *) (tr + 3), &ct, &cu, &cv, NULL)
+                                : rto_ray_tri(origin, dir, v0, v1, v2, &ct, &cu, &cv, NULL);
+            if (hit && ct < *t && ct < next_t[sa] && ct < t_max)
+            {
+                *t = ct; *u = cu; *v = cv; *tri_idx = ci;
+            }
+        }
+        if (*t != FLT_MAX)
+            return 1;
+        entry = next_t[sa];
+        pos[sa] += step[sa];
+        if (pos[sa] == out[sa])
+            break;
+        next_t[sa] += delta_t[sa];
+    }
+    return 0;
+}
+
+/* A batch of rts_bounded_walk: t_max per ray, or t_max_all for every ray when t_max is NULL.  Outputs as
+ * cuda_trace_query_rays writes them (tri = RTO_MISS and t = u = v = 0 on a miss); stopped[i] = 1 where rule 2 decided
+ * the miss (may be NULL). */
+void rts_query_rays(const rto_scene *sc, uint32_t n, const float *origins, const float *dirs, const float *t_max,
+                    float t_max_all, int variant, uint32_t *tri_idx, float *t, float *u, float *v, uint8_t *stopped)
+{
+    for (uint32_t i = 0; i < n; i++)
+    {
+        float ct = 0.0f, cu = 0.0f, cv = 0.0f;
+        uint32_t idx = RTO_MISS;
+        const int r = rts_bounded_walk(sc, origins + 3 * (size_t) i, dirs + 3 * (size_t) i, variant,
+                                       t_max ? t_max[i] : t_max_all, &ct, &cu, &cv, &idx);
+        tri_idx[i] = r == 1 ? idx : RTO_MISS;
+        t[i] = r == 1 ? ct : 0.0f;
+        u[i] = r == 1 ? cu : 0.0f;
+        v[i] = r == 1 ? cv : 0.0f;
+        if (stopped)
+            stopped[i] = r == 2;
+    }
 }
