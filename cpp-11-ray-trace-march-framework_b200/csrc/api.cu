@@ -61,6 +61,12 @@ struct DeviceState
     float4 *d_pair_recs_rel = nullptr;  // ... relative to rel_origin (primary rays; built on demand, pack.cu)
     float rel_origin[3] = { 0.0f, 0.0f, 0.0f };
     bool rel_valid = false;
+    // screen boxes of the pair records (K1's screen cull, pack.cu) for the camera sbox_cam, and the per-scene gate
+    // taken from them: cull only when enough pairs project small (sbox_cull)
+    float4 *d_pair_sbox = nullptr;
+    unsigned int *d_sbox_small = nullptr;
+    CameraDev sbox_cam;
+    bool sbox_valid = false, sbox_cull = false;
 
     // frame
     float2 *d_smp = nullptr;
@@ -148,6 +154,7 @@ struct cuda_trace_ctx
     bool occ_in_smem = true;
     bool rel_records = true;    // RTM_REL_RECORDS=0: always the plain records, 2: origin-relative at any frame size (experiments)
     bool rel_records_forced = false;
+    int screen_cull = -1;       // RTM_SCREEN_CULL: -1 automatic (the per-scene gate), 0 off, 1 on wherever rel records are used
     bool fast_math = true;      // RTM_FAST_MATH=0: always the range-checked intrinsics (experiments)
     int cost_order_forced = -1; // schedule.cu: -1 automatic, 0 / 1 forced by RTM_COST_ORDER (experiments)
     std::atomic<uint64_t> launches{0};
@@ -226,6 +233,9 @@ void free_scene(DeviceState& d)
     cudaFree(d.d_ppair_start); cudaFree(d.d_pair_recs); cudaFree(d.d_pair_recs_rel);
     d.d_ppair_start = nullptr; d.d_pair_recs = nullptr; d.d_pair_recs_rel = nullptr;
     d.rel_valid = false;
+    cudaFree(d.d_pair_sbox); cudaFree(d.d_sbox_small);
+    d.d_pair_sbox = nullptr; d.d_sbox_small = nullptr;
+    d.sbox_valid = false;
     cudaFree(d.d_pcell_start); cudaFree(d.d_pcell_occ); cudaFree(d.d_pcell_dist);
     d.d_pcell_start = nullptr; d.d_pcell_occ = nullptr; d.d_pcell_dist = nullptr;
     d.d_vtx = nullptr; d.d_tri = nullptr; d.d_cell_start = nullptr; d.d_cell_occ = nullptr;
@@ -546,6 +556,8 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
         ctx->rel_records = std::atoi(e) != 0;
         ctx->rel_records_forced = std::atoi(e) == 2;
     }
+    if (const char *e = std::getenv("RTM_SCREEN_CULL"))
+        ctx->screen_cull = std::atoi(e) < 0 ? -1 : (std::atoi(e) != 0 ? 1 : 0);
     if (const char *e = std::getenv("RTM_COST_ORDER"))
         ctx->cost_order_forced = std::atoi(e) != 0 ? 1 : 0;
     if (const char *e = std::getenv("RTM_FAST_MATH"))
@@ -1262,6 +1274,7 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
 
     TraceParams p;
     p.grid = grid_dev(ctx, d);
+    p.pair_sbox = nullptr;
     fill_camera(ctx, f, kind, p);
     p.smp = d.d_smp;
     p.tile_rects = d.d_tile_rects;
@@ -1366,6 +1379,38 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
             d.rel_valid = true;
         }
         p.grid.pair_recs_rel = d.d_pair_recs_rel;
+        if (ctx->screen_cull != 0)
+        {
+            // screen boxes for this frame's camera, rebuilt (inside the timed region) when any camera constant the
+            // boxes depend on changed.  The cull pays where a fair share of the pairs projects small -- killeroo4k: 30 %
+            // of its boxes are <= 32 pixels, 69 % of its pair iterations are skipped; the room of C4: none are, 6 % would
+            // be skipped, and every kept iteration costs a box load and a vote -- so the boxes are counted once per
+            // camera (a read-back, only then) and the cull is on when at least a fifth are small
+            if (!d.d_pair_sbox)
+            {
+                CK(cudaMalloc(&d.d_pair_sbox, std::max<uint64_t>(ctx->num_pairs, 1) * sizeof(float4)));
+                CK(cudaMalloc(&d.d_sbox_small, sizeof(unsigned int)));
+            }
+            const CameraDev& c = p.cam;
+            const bool same = d.sbox_valid && std::memcmp(d.sbox_cam.m, c.m, sizeof(c.m)) == 0 &&
+                              std::memcmp(d.sbox_cam.origin, c.origin, sizeof(c.origin)) == 0 &&
+                              std::memcmp(&d.sbox_cam.fov_xs, &c.fov_xs, sizeof(float)) == 0 &&
+                              std::memcmp(&d.sbox_cam.aspect, &c.aspect, sizeof(float)) == 0 &&
+                              std::memcmp(&d.sbox_cam.width_f, &c.width_f, sizeof(float)) == 0;
+            if (!same)
+            {
+                launch_screen_boxes(d.d_pair_recs, ctx->num_pairs, c, d.d_pair_sbox, d.d_sbox_small, d.stream);
+                ctx->launches++;
+                unsigned int small = 0;
+                CK(cudaMemcpyAsync(&small, d.d_sbox_small, sizeof(small), cudaMemcpyDeviceToHost, d.stream));
+                CK(cudaStreamSynchronize(d.stream));
+                d.sbox_cam = c;
+                d.sbox_cull = (uint64_t) small * 5 >= ctx->num_pairs;
+                d.sbox_valid = true;
+            }
+            if (ctx->screen_cull == 1 || d.sbox_cull)
+                p.pair_sbox = d.d_pair_sbox;
+        }
     }
     if (pl.total && use_pool)
     {

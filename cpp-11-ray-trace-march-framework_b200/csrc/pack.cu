@@ -4,6 +4,8 @@
 // Compiled with -fmad=false: e1/e2 and the variant-B constants must carry the reference's bits.
 #include "trace_kernels.cuh"
 
+#include <math_constants.h>
+
 namespace rtm
 {
 
@@ -289,7 +291,153 @@ __global__ void origin_relative_pairs_kernel(const float4 *__restrict__ pair_rec
     o[6] = make_float4(q[0][2], q[1][2], e2q[0], e2q[1]);
 }
 
+// ---- screen boxes (K1's screen cull, warp_trace.cuh test_pair_list; DESIGN.md section 3, "Screen cull"): for one camera,
+// the box in generate_ray's image plane (x = ndc_x * fov_xs, y = ndc_y * fov_xs / aspect) outside which no ray can be
+// accepted by either triangle of a pair.  float64 throughout, without contraction (-fmad=false), operation for
+// operation as tools/screen_cull.py restates it; the final narrowing rounds outwards.
+constexpr double kCullEps = 5.9604644775390625e-8; // 2^-24
+constexpr double kCullTau = 0.015625;              // a vertex counts as in front if its depth > 2^-6 |camera-space vector|
+constexpr double kCullRound = 16.0, kCullDir = 16.0, kCullSafety = 16.0, kCullKappaMax = 1.0e4;
+
+struct CullCamera
+{
+    double inv[9], k;
+    bool ok;
+};
+
+__device__ CullCamera cull_camera(const CameraDev& cam)
+{
+    CullCamera c;
+    const double m00 = cam.m[0][0], m01 = cam.m[0][1], m02 = cam.m[0][2], m10 = cam.m[1][0], m11 = cam.m[1][1],
+                 m12 = cam.m[1][2], m20 = cam.m[2][0], m21 = cam.m[2][1], m22 = cam.m[2][2];
+    const double c00 = m11 * m22 - m12 * m21, c01 = m12 * m20 - m10 * m22, c02 = m10 * m21 - m11 * m20;
+    const double det = m00 * c00 + m01 * c01 + m02 * c02;
+    c.inv[0] = c00 / det; c.inv[1] = (m02 * m21 - m01 * m22) / det; c.inv[2] = (m01 * m12 - m02 * m11) / det;
+    c.inv[3] = c01 / det; c.inv[4] = (m00 * m22 - m02 * m20) / det; c.inv[5] = (m02 * m10 - m00 * m12) / det;
+    c.inv[6] = c02 / det; c.inv[7] = (m01 * m20 - m00 * m21) / det; c.inv[8] = (m00 * m11 - m01 * m10) / det;
+    const double m[9] = { m00, m01, m02, m10, m11, m12, m20, m21, m22 };
+    double fro = 0.0, fro_inv = 0.0;
+    for (int i = 0; i < 9; i++)
+        fro = fro + m[i] * m[i];
+    for (int i = 0; i < 9; i++)
+        fro_inv = fro_inv + c.inv[i] * c.inv[i];
+    fro = sqrt(fro);
+    fro_inv = sqrt(fro_inv);
+    const double fx = cam.fov_xs, fy = fx / (double) cam.aspect;
+    const double l_img = sqrt(1.0 + 4.0 * (fx * fx) + 4.0 * (fy * fy));
+    c.k = kCullEps * fro * l_img / fabs(det);
+    c.ok = isfinite(c.k) && det != 0.0 && isfinite(fro_inv) && fro * fro_inv <= kCullKappaMax;
+    return c;
+}
+
+__device__ __forceinline__ double norm3(double x, double y, double z) { return sqrt(x * x + y * y + z * z); }
+
+// box {xmin, xmax, ymin, ymax} of one triangle (v0, e1, e2 as the records hold them): the projected triangle with each
+// edge line pushed outwards by kCullSafety x the bound on that edge's error; +-inf = never cull; empty for the dummy
+__device__ void triangle_screen_box(float v0x, float v0y, float v0z, float e1x, float e1y, float e1z, float e2x, float e2y,
+                                    float e2z, uint32_t idx, const CameraDev& cam, const CullCamera& cc, double box[4])
+{
+    if (idx == 0xFFFFFFFFu)
+    {
+        box[0] = box[2] = CUDART_INF;
+        box[1] = box[3] = -CUDART_INF;
+        return;
+    }
+    const double o[3] = { cam.origin[0], cam.origin[1], cam.origin[2] };
+    const double p[3][3] = { { v0x, v0y, v0z },
+                             { (double) v0x + (double) e1x, (double) v0y + (double) e1y, (double) v0z + (double) e1z },
+                             { (double) v0x + (double) e2x, (double) v0y + (double) e2y, (double) v0z + (double) e2z } };
+    double V[3][3], cx[3], cy[3], w[3];
+    bool good = cc.ok;
+    for (int q = 0; q < 3; q++)
+    {
+        const double vx = p[q][0] - o[0], vy = p[q][1] - o[1], vz = p[q][2] - o[2];
+        const double x = vx * cc.inv[0] + vy * cc.inv[3] + vz * cc.inv[6];
+        const double y = vx * cc.inv[1] + vy * cc.inv[4] + vz * cc.inv[7];
+        const double z = vx * cc.inv[2] + vy * cc.inv[5] + vz * cc.inv[8];
+        V[q][0] = vx; V[q][1] = vy; V[q][2] = vz;
+        cx[q] = x / -z;
+        cy[q] = y / -z;
+        w[q] = -z;
+        good = good && w[q] > kCullTau * norm3(x, y, z);
+    }
+    const double R = fmax(fmax(norm3(V[0][0], V[0][1], V[0][2]), norm3(V[1][0], V[1][1], V[1][2])), norm3(V[2][0], V[2][1], V[2][2]));
+    const double l1 = norm3(e1x, e1y, e1z), l2 = norm3(e2x, e2y, e2z);
+    // rounding error of the test's three edge functions: v's numerator (edge 0-1), the u + v <= 1 test (edge 1-2),
+    // u's numerator (edge 2-0)
+    const double base[3] = { kCullRound * (R * l1), kCullRound * (R * (l1 + l2) + l1 * l2), kCullRound * (R * l2) };
+    const double a2s = (cx[1] - cx[0]) * (cy[2] - cy[0]) - (cy[1] - cy[0]) * (cx[2] - cx[0]);
+    const double sgn = a2s < 0.0 ? -1.0 : 1.0;
+    double nx[3], ny[3], off[3], perim_slack = 0.0;
+    for (int q = 0; q < 3; q++)
+    {
+        const int i = q, j = q == 2 ? 0 : q + 1;
+        const double dx = cx[j] - cx[i], dy = cy[j] - cy[i];
+        const double lij = sqrt(dx * dx + dy * dy);
+        const double crx = V[i][1] * V[j][2] - V[i][2] * V[j][1];
+        const double cry = V[i][2] * V[j][0] - V[i][0] * V[j][2];
+        const double crz = V[i][0] * V[j][1] - V[i][1] * V[j][0];
+        const double dij = kCullSafety * (cc.k * (base[q] + kCullDir * norm3(crx, cry, crz)) / (w[i] * w[j] * lij));
+        nx[q] = sgn * dy / lij; // outward unit normal
+        ny[q] = -sgn * dx / lij;
+        off[q] = dij;
+        perim_slack = perim_slack + lij * dij;
+    }
+    // vertex q lies on edges q - 1 and q: its pushed-out position solves n . s = slack for both lines
+    double px[3], py[3];
+    for (int q = 0; q < 3; q++)
+    {
+        const int a = (q + 2) % 3, b = q;
+        const double det2 = nx[a] * ny[b] - ny[a] * nx[b];
+        px[q] = cx[q] + (off[a] * ny[b] - off[b] * ny[a]) / det2;
+        py[q] = cy[q] + (nx[a] * off[b] - nx[b] * off[a]) / det2;
+        good = good && isfinite(px[q]) && isfinite(py[q]);
+    }
+    box[0] = fmin(fmin(px[0], px[1]), px[2]);
+    box[1] = fmax(fmax(px[0], px[1]), px[2]);
+    box[2] = fmin(fmin(py[0], py[1]), py[2]);
+    box[3] = fmax(fmax(py[0], py[1]), py[2]);
+    good = good && perim_slack < fabs(a2s);
+    for (int q = 0; q < 4; q++)
+        good = good && isfinite(box[q]);
+    if (!good)
+    {
+        box[0] = box[2] = -CUDART_INF;
+        box[1] = box[3] = CUDART_INF;
+    }
+}
+
+// one thread per pair record
+__global__ void screen_boxes_kernel(const float4 *__restrict__ pair_recs, uint64_t num_pairs, const __grid_constant__ CameraDev cam,
+                                    float small_side, float4 *__restrict__ sbox, unsigned int *__restrict__ small_boxes)
+{
+    const uint64_t k = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= num_pairs)
+        return;
+    const CullCamera cc = cull_camera(cam);
+    const float4 *r = pair_recs + 5 * k;
+    const float4 f0 = r[0], f1 = r[1], f2 = r[2], f3 = r[3], f4 = r[4];
+    double a[4], b[4];
+    triangle_screen_box(f0.x, f0.z, f1.x, f1.z, f2.x, f2.z, f3.x, f3.z, f4.x, __float_as_uint(f4.z), cam, cc, a);
+    triangle_screen_box(f0.y, f0.w, f1.y, f1.w, f2.y, f2.w, f3.y, f3.w, f4.y, __float_as_uint(f4.w), cam, cc, b);
+    const float4 out = make_float4(__double2float_rd(fmin(a[0], b[0])), __double2float_ru(fmax(a[1], b[1])),
+                                   __double2float_rd(fmin(a[2], b[2])), __double2float_ru(fmax(a[3], b[3])));
+    sbox[k] = out;
+    if (fmaxf(out.y - out.x, out.w - out.z) <= small_side)
+        atomicAdd(small_boxes, 1u);
+}
+
 } // namespace
+
+void launch_screen_boxes(const float4 *pair_recs, uint64_t num_pairs, const CameraDev& cam, float4 *sbox,
+                         unsigned int *small_boxes, cudaStream_t stream)
+{
+    cudaMemsetAsync(small_boxes, 0, sizeof(unsigned int), stream);
+    // kScreenCullSmallPixels pixels: the image spans 2 fov_xs over width_f pixels
+    const float small_side = kScreenCullSmallPixels * (2.0f * cam.fov_xs / cam.width_f);
+    if (num_pairs)
+        screen_boxes_kernel<<<blocks_for(num_pairs, 128), 128, 0, stream>>>(pair_recs, num_pairs, cam, small_side, sbox, small_boxes);
+}
 
 void launch_origin_relative_pairs(const float4 *pair_recs, uint64_t num_pairs, const float origin[3], float4 *rel,
                                   cudaStream_t stream)

@@ -23,7 +23,7 @@ constexpr unsigned kFull = 0xFFFFFFFFu;
 constexpr size_t kOptInDynamicSmem = 24 * 1024;
 
 // One sample per lane; ALL lanes of the warp call this together (valid == false: no ray)
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD>
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool CULL>
 __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void *s_occ, bool valid,
                                                uint32_t px, uint32_t py, uint32_t s, const float2 *smp, Counters *cnt)
 {
@@ -49,13 +49,18 @@ __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void 
     else
     {
         float3 o, d;
+        float2 img;
         const float2 off = smp[valid ? s : 0];
-        generate_ray<ALT>(p.cam, px, py, off.x, off.y, o, d);
+        generate_ray<ALT>(p.cam, px, py, off.x, off.y, o, d, CULL ? &img : nullptr);
         if (COUNT && valid) cnt->rays++;
         PackedUnits pku;
         pku.one = p.pk_one;
         pku.minus_one = p.pk_minus_one;
-        is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD>(p.grid, s_occ, o, d, valid, hit, cnt, pku, p.cam.fast_math != 0);
+        if constexpr (CULL)
+            is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD, false, false, true>(
+                p.grid, s_occ, o, d, valid, hit, cnt, pku, p.cam.fast_math != 0, FLT_MAX, p.pair_sbox, img);
+        else
+            is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD>(p.grid, s_occ, o, d, valid, hit, cnt, pku, p.cam.fast_math != 0);
         if (COUNT && is_hit) cnt->hits++;
         if (KEEP_HITS && valid)
         {
@@ -107,7 +112,7 @@ __device__ __forceinline__ void release_add(const TraceParams& p, uint32_t band,
     }
 }
 
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS>
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS, bool CULL = false>
 __global__ void __launch_bounds__(kTraceMaxThreads) trace_tiles_kernel(const __grid_constant__ TraceParams p)
 {
     // shared memory: [sample table (renderer.cpp:49-60), spp x float2]
@@ -236,7 +241,7 @@ __global__ void __launch_bounds__(kTraceMaxThreads) trace_tiles_kernel(const __g
                 if (!__any_sync(kFull, active))
                     continue;
                 const uint32_t px = bx0 + ox, py = by0 + oy;
-                const float3 rgb = trace_sample<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD>(p, s_occ, active, px, py, s, s_smp, &cnt);
+                const float3 rgb = trace_sample<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, CULL>(p, s_occ, active, px, py, s, s_smp, &cnt);
                 // col += sample, smp = 0..N-1 in order (renderer.cpp:87-122).  The samples of a pixel sit in
                 // consecutive lanes; they go through shared memory -- one 16-byte store per lane, one broadcast
                 // load per term -- and every lane of the pixel adds them up in sample order (red and green as one
@@ -276,7 +281,7 @@ __global__ void __launch_bounds__(kTraceMaxThreads) trace_tiles_kernel(const __g
                 for (uint32_t sb = 0; sb < p.spp; sb += 32)
                 {
                     const uint32_t s = sb + lane;
-                    const float3 rgb = trace_sample<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD>(p, s_occ, inside && s < p.spp, px, py, s, s_smp, &cnt);
+                    const float3 rgb = trace_sample<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, CULL>(p, s_occ, inside && s < p.spp, px, py, s, s_smp, &cnt);
                     const uint32_t n = min(32u, p.spp - sb);
                     for (uint32_t k = 0; k < n; k++)
                     {
@@ -474,10 +479,8 @@ __global__ void sample_table_kernel(float2 *smp, uint32_t spp)
     smp[s] = make_float2((float) (x - 0.5), (float) (val - 0.5));
 }
 
-// The plain kernel exists with / without the rcp range guard (scenes larger than 1e14 units) and
-// with / without the row-band completion counters; the instrumented variants always carry both.
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS>
-void launch_instance(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
+template <auto KERNEL>
+void launch_kernel(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
 {
     if (smem > kOptInDynamicSmem)
     {
@@ -487,13 +490,24 @@ void launch_instance(const TraceParams& p, int grid_blocks, int threads, size_t 
         cudaGetDevice(&dev);
         if (dev < 0 || dev >= 64 || opted_in[dev] < smem)
         {
-            cudaFuncSetAttribute(trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+            cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
             if (dev >= 0 && dev < 64)
                 opted_in[dev] = smem;
         }
     }
-    trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS><<<grid_blocks, threads, smem, stream>>>(p);
+    KERNEL<<<grid_blocks, threads, smem, stream>>>(p);
+}
+
+// The plain kernel exists with / without the rcp range guard (scenes larger than 1e14 units) and
+// with / without the row-band completion counters; the instrumented variants always carry both.
+// kVariantMTRel also exists with the screen cull (p.pair_sbox set); nothing else culls.
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS>
+void launch_instance(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
+{
+    if constexpr (VARIANT == kVariantMTRel)
+        if (p.pair_sbox)
+            return launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS, true>>(p, grid_blocks, threads, smem, stream);
+    launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS>>(p, grid_blocks, threads, smem, stream);
 }
 
 template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE>

@@ -103,6 +103,8 @@ struct TraceParams
     // (1.0f, 1.0f) and (-1.0f, -1.0f) as register pairs: the multiplier of the packed sums and differences in
     // warp_trace.cuh.  Passed as data so that ptxas cannot fold them into a contracted FFMA2.
     unsigned long long pk_one, pk_minus_one;
+    const float4 *pair_sbox;           // kVariantMTRel: screen box of every pair record for this camera (pack.cu) or
+                                       // null = no screen cull
 };
 
 struct RayBatchParams
@@ -169,6 +171,11 @@ void launch_pack_pairs(const uint32_t *pcell_start, const uint32_t *ppair_start,
                        float4 *pair_recs, cudaStream_t stream);
 void launch_origin_relative_pairs(const float4 *pair_recs, uint64_t num_pairs, const float origin[3], float4 *rel,
                                   cudaStream_t stream);
+// screen box of every pair record for camera `cam` (pack.cu); *small_boxes (zeroed here) counts the pairs whose box is at
+// most kScreenCullSmallPixels pixels on its longer side
+void launch_screen_boxes(const float4 *pair_recs, uint64_t num_pairs, const CameraDev& cam, float4 *sbox,
+                         unsigned int *small_boxes, cudaStream_t stream);
+constexpr float kScreenCullSmallPixels = 32.0f;
 void launch_pack_cell_tris(const float *vtx, const uint32_t *tri, const uint32_t *tri_index, uint64_t num_refs,
                            float4 *cell_tris, float4 *cell_tris_b, cudaStream_t stream);
 void launch_pack_normals(const float *vtx, const uint32_t *tri, uint32_t num_tri, float4 *tri_normals,

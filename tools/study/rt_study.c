@@ -4,6 +4,8 @@
  * (rto_ray_tri, rto_ray_aabb, ... from oracle/librt_oracle.so) and adds:
  *
  *   rts_ray_walk_profile   the triangle-list length of every cell a ray visits, in order (tools/warp_walk_model.py)
+ *   rts_ray_walk_cells     the indices of the occupied cells a ray visits, in order (the screen-cull model of
+ *                          tools/warp_walk_model.py)
  *   rts_mailbox_walk       the walk WITH the mailbox of the product's optional mode (CUDA_TRACE_VARIANT_MAILBOX,
  *                          csrc/rt_device.cuh): 4 entries, round-robin over the tests actually computed -- returns the
  *                          hit and counts tests asked for / answered from the mailbox (tests/test_mailbox_model_cpu.py
@@ -45,8 +47,8 @@ static int to_voxel(const rto_grid *g, const float *p, int axis)
 static float to_pos(const rto_grid *g, int vox, int axis) { return g->aabb_min[axis] + vox * g->cell_wdh; }
 
 /* the walk of grid.cpp:159-281 (Moeller-Trumbore) with both recorders; either output may be NULL */
-static int walk(const rto_scene *sc, const float *origin, const float *dir, uint16_t *lens, uint32_t cap, uint32_t *n_cells,
-                rts_counters *cnt)
+static int walk(const rto_scene *sc, const float *origin, const float *dir, uint16_t *lens, uint32_t *ids, uint32_t cap,
+                uint32_t *n_cells, rts_counters *cnt)
 {
     const rto_grid *g = &sc->grid;
     float enter_t, leave_t, gi[3];
@@ -91,7 +93,10 @@ static int walk(const rto_scene *sc, const float *origin, const float *dir, uint
         const uint64_t len = g->cell_offset[cell + 1] - g->cell_offset[cell];
         if (lens && *n_cells < cap)
             lens[*n_cells] = (uint16_t) (len > 65535 ? 65535 : len);
-        (*n_cells)++;
+        if (ids && len && *n_cells < cap)
+            ids[*n_cells] = (uint32_t) cell;
+        if (!ids || len)
+            (*n_cells)++;
         for (uint64_t k = g->cell_offset[cell]; k < g->cell_offset[cell + 1]; k++)
         {
             const uint32_t ci = g->tri_index[k];
@@ -147,14 +152,23 @@ uint32_t rts_ray_walk_profile(const rto_scene *sc, const float *origin, const fl
                               int *hit)
 {
     uint32_t n = 0;
-    *hit = walk(sc, origin, dir, list_lengths, cap, &n, NULL);
+    *hit = walk(sc, origin, dir, list_lengths, NULL, cap, &n, NULL);
+    return n;
+}
+
+/* -> number of OCCUPIED cells visited, their (unpadded) cell indices in order in cell_ids (at most cap are written; the
+ * last one is the hit's cell when *hit) -- tools/warp_walk_model.py --screen-cull */
+uint32_t rts_ray_walk_cells(const rto_scene *sc, const float *origin, const float *dir, uint32_t cap, uint32_t *cell_ids, int *hit)
+{
+    uint32_t n = 0;
+    *hit = walk(sc, origin, dir, NULL, cell_ids, cap, &n, NULL);
     return n;
 }
 
 int rts_study_ray(const rto_scene *sc, const float *origin, const float *dir, rts_counters *cnt)
 {
     uint32_t n = 0;
-    return walk(sc, origin, dir, NULL, 0, &n, cnt);
+    return walk(sc, origin, dir, NULL, NULL, 0, &n, cnt);
 }
 
 /* The product's mailbox mode restated on the CPU: same walk, same 4-entry round-robin mailbox keyed by triangle index,

@@ -6,7 +6,12 @@ lane = pixel-in-round * spp + sample): phase A costs the LONGEST empty-cell run 
 list, and compares with (a) the useful work, i.e. perfect packing, and (b) re-pairing the strip's rays between phases
 (the rays of one strip pooled, sorted by what they need next, and dealt to the strip's warps).
 
-python tools/warp_walk_model.py [workload] [n_strips]        (test infrastructure: imports oracle/)"""
+With --screen-cull it replays phase B of the same warps against the screen boxes of the pair records
+(tools/screen_cull.py) instead: the fraction of pair iterations in which every lane
+that owns a pair is outside its box -- the iterations K1 could skip before loading the record -- with one box per pair
+and, for comparison, one per triangle.
+
+python tools/warp_walk_model.py [workload] [n_strips] [--screen-cull]        (test infrastructure: imports oracle/)"""
 import ctypes as C
 import importlib
 import os
@@ -24,8 +29,10 @@ scenes, hostapi, mr = pkg("scenes"), pkg("hostapi"), pkg("multirank")
 
 C_DDA, C_TEST, C_ITER = 13, 61, 24  # SASS instructions: one DDA step, one triangle test, fixed cost of one A+B iteration
 
-wl = sys.argv[1] if len(sys.argv) > 1 else "killeroo4k"
-n_strips = int(sys.argv[2]) if len(sys.argv) > 2 else 1500
+CULL = "--screen-cull" in sys.argv
+args = [a for a in sys.argv[1:] if a != "--screen-cull"]
+wl = args[0] if args else "killeroo4k"
+n_strips = int(args[1]) if len(args) > 1 else 1500
 scene, w, h, spp, res = scenes.CONFIGS[wl]
 host = hostapi.host_api()
 m, fov, cam = scenes.build(host, scene)
@@ -40,6 +47,8 @@ subprocess.check_call(["bash", os.path.join(STUDY, "build.sh")])
 study = C.CDLL(os.path.join(STUDY, "librt_study.so"))
 study.rts_ray_walk_profile.restype = C.c_uint32
 study.rts_ray_walk_profile.argtypes = [C.c_void_p, F, F, C.c_uint32, U16, C.POINTER(C.c_int)]
+study.rts_ray_walk_cells.restype = C.c_uint32
+study.rts_ray_walk_cells.argtypes = [C.c_void_p, F, F, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_int)]
 smp = port.sample_table(spp)
 fov_xs, aspect = port.camera_constants(fov, w, h)
 cam32 = np.ascontiguousarray(cam, np.float32)
@@ -116,6 +125,69 @@ def model_pooled(rays, n_warps):
         cost += C_ITER * ((len(a_steps) + 31) // 32) + 40  # + a shared-memory exchange per phase pair
     return cost
 
+
+def cull_model():
+    """Phase B of K1's warp rounds with the screen cull: counts pair iterations, those every owning lane skips (pair
+    box; per-triangle boxes), and the lane-level pair tests."""
+    import screen_cull as sc
+    pstart, a, b = sc.pair_records(ps)
+    inv, k, ok = sc.camera_terms(cam32, fov_xs, aspect)
+    org = cam32.reshape(-1)[12:15]
+    ta, tb = sc.triangle_boxes(*a, org, inv, k, ok), sc.triangle_boxes(*b, org, inv, k, ok)
+    pb = sc.pair_boxes(ta, tb).astype(np.float64)
+    ta32, tb32 = sc.pair_boxes(ta, ta).astype(np.float64), sc.pair_boxes(tb, tb).astype(np.float64)
+    print("pairs %d, never culled (whole plane) %.2f %%" % (len(pb), 100.0 * np.mean(np.isinf(pb[:, 0]) & (pb[:, 0] < 0))))
+    ids = np.zeros(4096, np.uint32)
+    cnt = dict(iters=0, skip_pair=0, skip_tri=0, lane_tests=0, lane_out=0)
+    out = lambda box, j, x, y: (x < box[j, 0]) | (x > box[j, 1]) | (y < box[j, 2]) | (y > box[j, 3])
+    n_x, n_y = w // sw, h // sh
+    for _ in range(n_strips):
+        bx, by = rs.randint(n_x) * sw, rs.randint(n_y) * sh
+        lanes = []
+        for slot in range(sw * sh):
+            ox = (slot & 1) | ((slot >> 1) & 2) | ((slot >> 2) & 4)
+            oy = ((slot >> 1) & 1) | ((slot >> 2) & 2)
+            for s in range(spp):
+                o, d = np.zeros(3, np.float32), np.zeros(3, np.float32)
+                lib.rto_generate_ray(cam32.ctypes.data_as(F), bx + ox, by + oy, w, h, float(smp[s, 0]), float(smp[s, 1]),
+                                     float(fov_xs), float(aspect), o.ctypes.data_as(F), d.ctypes.data_as(F))
+                hit = C.c_int(0)
+                n = study.rts_ray_walk_cells(C.byref(ps.s), o.ctypes.data_as(F), d.ctypes.data_as(F), len(ids),
+                                             ids.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(hit))
+                x, y = sc.image_point(bx + ox, by + oy, w, h, smp[s, 0], smp[s, 1], fov_xs, aspect)
+                lanes.append((ids[:min(n, len(ids))].astype(np.int64).copy(), float(x), float(y)))
+        for wbase in range(0, len(lanes), 32):
+            warp = lanes[wbase:wbase + 32]
+            xs = np.array([l[1] for l in warp])
+            ys = np.array([l[2] for l in warp])
+            for r in range(max(len(l[0]) for l in warp)):
+                has = np.array([r < len(l[0]) for l in warp])
+                cell = np.array([l[0][r] if r < len(l[0]) else 0 for l in warp])
+                beg = pstart[cell]
+                ln = np.where(has, pstart[cell + 1] - beg, 0)
+                for i in range(int(ln.max())):
+                    mine = i < ln
+                    j = beg + np.minimum(i, np.maximum(ln - 1, 0))
+                    op = out(pb, j, xs, ys)
+                    ot = out(ta32, j, xs, ys) & out(tb32, j, xs, ys)
+                    cnt["iters"] += 1
+                    cnt["skip_pair"] += bool(np.all(~mine | op))
+                    cnt["skip_tri"] += bool(np.all(~mine | ot))
+                    cnt["lane_tests"] += int(mine.sum())
+                    cnt["lane_out"] += int((mine & op).sum())
+    fp, ft = cnt["skip_pair"] / cnt["iters"], cnt["skip_tri"] / cnt["iters"]
+    print("%s: %d strips, %d warp pair-iterations" % (wl, n_strips, cnt["iters"]))
+    print("skipped by the pair box %.1f %%, by per-triangle boxes %.1f %%; lane pair tests outside the pair box %.1f %%"
+          % (100 * fp, 100 * ft, 100 * cnt["lane_out"] / cnt["lane_tests"]))
+    # a skipped iteration saves ~37 issue slots, a kept one costs ~8 more (estimated from the r02 SASS)
+    for name, f in (("pair box", fp), ("triangle boxes", ft)):
+        print("  %s: net instructions saved per pair iteration %.1f (37 f - 8 (1 - f))" % (name, 37 * f - 8 * (1 - f)))
+
+
+if CULL:
+    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+    cull_model()
+    sys.exit(0)
 
 tot = dict(k1=0.0, useful=0.0, pooled=0.0)
 n_x, n_y = w // sw, h // sh
