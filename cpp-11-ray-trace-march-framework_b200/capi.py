@@ -68,6 +68,8 @@ SYMBOLS = {
                                                     C.POINTER(GridDesc), _U64P, _U32P]),
     "cuda_trace_download_grid": (C.c_int, [C.c_void_p, C.POINTER(GridDesc), _U64P, _U32P]),
     "cuda_trace_download_distance_map": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]),
+    "cuda_trace_download_screen_boxes": (C.c_int, [C.c_void_p, _F32P, C.c_uint64, C.POINTER(C.c_uint64),
+                                                   C.POINTER(C.c_uint32), C.POINTER(C.c_int)]),
     "cuda_trace_tiles": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.POINTER(TileRect), C.c_uint32, _U32P]),
     "cuda_trace_tiles_into": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.POINTER(TileRect), C.c_uint32, C.POINTER(_U32P),
                                         C.c_void_p, C.c_void_p]),
@@ -307,6 +309,17 @@ class CudaTrace:
         d = GridDesc()
         self._ck(self.lib.cuda_trace_download_grid(self.h, C.byref(d), None, None))
         return out.reshape(d.dim[1] + 2, d.dim[2] + 2, d.dim[0] + 2)
+
+    def download_screen_boxes(self):
+        """-> (boxes float32 [num_pairs, 4] {xmin, xmax, ymin, ymax}, small, cull_on): the screen boxes of device 0
+        for the camera of the last frame that built them; num_pairs = 0 when none are built"""
+        n, small, on = C.c_uint64(0), C.c_uint32(0), C.c_int(0)
+        self._ck(self.lib.cuda_trace_download_screen_boxes(self.h, None, 0, C.byref(n), C.byref(small), C.byref(on)))
+        out = np.zeros((n.value, 4), np.float32)
+        if n.value:
+            self._ck(self.lib.cuda_trace_download_screen_boxes(self.h, _p(out, _F32P), out.size, C.byref(n),
+                                                               C.byref(small), C.byref(on)))
+        return out, int(small.value), bool(on.value)
 
     # -- frames
     @staticmethod

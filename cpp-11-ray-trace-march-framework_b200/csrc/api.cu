@@ -66,6 +66,7 @@ struct DeviceState
     float4 *d_pair_sbox = nullptr;
     unsigned int *d_sbox_small = nullptr;
     CameraDev sbox_cam;
+    uint32_t sbox_small = 0; // boxes of at most kScreenCullSmallPixels pixels for sbox_cam (the gate's count)
     bool sbox_valid = false, sbox_cull = false;
 
     // frame
@@ -835,6 +836,32 @@ int cuda_trace_download_distance_map(cuda_trace_ctx *ctx, uint8_t *out, uint64_t
     return 0;
 }
 
+int cuda_trace_download_screen_boxes(cuda_trace_ctx *ctx, float *boxes, uint64_t capacity, uint64_t *num_pairs,
+                                     uint32_t *small, int *cull_on)
+{
+    if (!ctx || !num_pairs || !small || !cull_on || (capacity && !boxes))
+        return CUDA_TRACE_ERR_ARG;
+    std::lock_guard<std::recursive_mutex> guard(ctx->api_mtx);
+    *num_pairs = 0;
+    *small = 0;
+    *cull_on = 0;
+    if (!ctx->have_scene || ctx->dev.empty() || !ctx->dev[0].sbox_valid)
+        return 0;
+    // read only: the boxes, their camera and the gate stay as the last frame left them
+    DeviceState& d = ctx->dev[0];
+    *num_pairs = ctx->num_pairs;
+    *small = d.sbox_small;
+    *cull_on = d.sbox_cull ? 1 : 0;
+    const uint64_t n = std::min<uint64_t>(*num_pairs, capacity / 4);
+    if (n)
+    {
+        CK(cudaSetDevice(d.ordinal));
+        CK(cudaMemcpyAsync(boxes, d.d_pair_sbox, n * sizeof(float4), cudaMemcpyDeviceToHost, d.stream));
+        CK(cudaStreamSynchronize(d.stream));
+    }
+    return 0;
+}
+
 // ----------------------------------------------------------------------------------- tracing
 int cuda_trace_prepare_framebuffer(cuda_trace_ctx *ctx, uint32_t width, uint32_t height)
 {
@@ -1405,6 +1432,7 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
                 CK(cudaMemcpyAsync(&small, d.d_sbox_small, sizeof(small), cudaMemcpyDeviceToHost, d.stream));
                 CK(cudaStreamSynchronize(d.stream));
                 d.sbox_cam = c;
+                d.sbox_small = small;
                 d.sbox_cull = (uint64_t) small * 5 >= ctx->num_pairs;
                 d.sbox_valid = true;
             }

@@ -158,6 +158,15 @@ int cuda_trace_download_grid(cuda_trace_ctx *ctx, cuda_trace_grid_desc *desc, ui
  * the map's size, 0 when this scene has none. */
 int cuda_trace_download_distance_map(cuda_trace_ctx *ctx, uint8_t *out, uint64_t *num_bytes);
 
+/* Diagnostics: the screen boxes of device 0 for the camera of the last frame that built them (K1's screen cull,
+ * DESIGN.md section 3): 4 floats {xmin, xmax, ymin, ymax} per pair record, in pair-record order; at most
+ * capacity / 4 boxes are written.  boxes == NULL: query only.  *num_pairs = pair records (0 when no boxes are
+ * built: no scene, or no frame since the upload used the origin-relative records); *small = boxes counted small
+ * for that camera; *cull_on = whether the automatic gate turned the cull on (RTM_SCREEN_CULL=1 culls regardless).
+ * Read only: it changes neither the boxes nor when they are rebuilt. */
+int cuda_trace_download_screen_boxes(cuda_trace_ctx *ctx, float *boxes, uint64_t capacity, uint64_t *num_pairs,
+                                     uint32_t *small, int *cull_on);
+
 /* ---- tracing --------------------------------------------------------------------------------
  * cuda_trace_tiles replaces Framebuffer::CreateWorkerThreads + WorkerThread + RenderTile for the
  * given tiles (framebuffer.cpp:16-27,59-92; renderer.cpp:43-136): it renders every pixel of every

@@ -50,9 +50,11 @@ def camera_terms(cam16, fov_xs, aspect):
     return inv, float(k), ok
 
 
-def triangle_boxes(v0, e1, e2, idx, origin, inv, k, ok):
+def triangle_boxes(v0, e1, e2, idx, origin, inv, k, ok, edges_out=None):
     """v0, e1, e2: (n, 3) float32 as the records hold them; idx: (n,) uint32.  -> (n, 4) float64 {xmin, xmax, ymin, ymax}:
-    +-inf for "never cull", an empty box (+inf, -inf, ...) for the dummy triangle."""
+    +-inf for "never cull", an empty box (+inf, -inf, ...) for the dummy triangle.  edges_out (a dict) receives the
+    projected vertices "cx", "cy" and, per edge q = 0-1, 1-2, 2-0, its outward unit normal "nx", "ny" and push-out
+    "off", each (3, n) -- what tests aim rays at."""
     v0, e1, e2 = (np.asarray(a, np.float32).astype(np.float64) for a in (v0, e1, e2))
     o = np.asarray(origin, np.float32).astype(np.float64)
     n = len(v0)
@@ -101,6 +103,9 @@ def triangle_boxes(v0, e1, e2, idx, origin, inv, k, ok):
             good &= w[q] > TAU * clen[q]
         good &= perim_slack < np.abs(a2s)
         good &= np.isfinite(box).all(1)
+    if edges_out is not None:
+        edges_out.update(cx=np.array([p[0] for p in c]), cy=np.array([p[1] for p in c]), nx=np.array(nx),
+                         ny=np.array(ny), off=np.array(off))
     box[~good] = (-INF, INF, -INF, INF)
     box[np.asarray(idx) == DUMMY] = (INF, -INF, INF, -INF)
     return box
