@@ -156,6 +156,7 @@ struct cuda_trace_ctx
     bool rel_records = true;    // RTM_REL_RECORDS=0: always the plain records, 2: origin-relative at any frame size (experiments)
     bool rel_records_forced = false;
     int screen_cull = -1;       // RTM_SCREEN_CULL: -1 automatic (the per-scene gate), 0 off, 1 on wherever rel records are used
+    bool cull_scan = true;      // RTM_CULL_SCAN=0: the culling K1 checks one pair box at a time instead of a warp's 32 at once
     bool fast_math = true;      // RTM_FAST_MATH=0: always the range-checked intrinsics (experiments)
     int cost_order_forced = -1; // schedule.cu: -1 automatic, 0 / 1 forced by RTM_COST_ORDER (experiments)
     std::atomic<uint64_t> launches{0};
@@ -559,6 +560,8 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
     }
     if (const char *e = std::getenv("RTM_SCREEN_CULL"))
         ctx->screen_cull = std::atoi(e) < 0 ? -1 : (std::atoi(e) != 0 ? 1 : 0);
+    if (const char *e = std::getenv("RTM_CULL_SCAN"))
+        ctx->cull_scan = std::atoi(e) != 0;
     if (const char *e = std::getenv("RTM_COST_ORDER"))
         ctx->cost_order_forced = std::atoi(e) != 0 ? 1 : 0;
     if (const char *e = std::getenv("RTM_FAST_MATH"))
@@ -1302,6 +1305,7 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     TraceParams p;
     p.grid = grid_dev(ctx, d);
     p.pair_sbox = nullptr;
+    p.cull_scan = ctx->cull_scan ? 1u : 0u;
     fill_camera(ctx, f, kind, p);
     p.smp = d.d_smp;
     p.tile_rects = d.d_tile_rects;

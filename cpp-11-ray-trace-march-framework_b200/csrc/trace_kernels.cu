@@ -23,7 +23,7 @@ constexpr unsigned kFull = 0xFFFFFFFFu;
 constexpr size_t kOptInDynamicSmem = 24 * 1024;
 
 // One sample per lane; ALL lanes of the warp call this together (valid == false: no ray)
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool CULL>
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, int CULL>
 __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void *s_occ, bool valid,
                                                uint32_t px, uint32_t py, uint32_t s, const float2 *smp, Counters *cnt)
 {
@@ -56,8 +56,8 @@ __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void 
         PackedUnits pku;
         pku.one = p.pk_one;
         pku.minus_one = p.pk_minus_one;
-        if constexpr (CULL)
-            is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD, false, false, true>(
+        if constexpr (CULL != kCullOff)
+            is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD, false, false, CULL>(
                 p.grid, s_occ, o, d, valid, hit, cnt, pku, p.cam.fast_math != 0, FLT_MAX, p.pair_sbox, img);
         else
             is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD>(p.grid, s_occ, o, d, valid, hit, cnt, pku, p.cam.fast_math != 0);
@@ -112,7 +112,7 @@ __device__ __forceinline__ void release_add(const TraceParams& p, uint32_t band,
     }
 }
 
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS, bool CULL = false>
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS, int CULL = kCullOff>
 __global__ void __launch_bounds__(kTraceMaxThreads) trace_tiles_kernel(const __grid_constant__ TraceParams p)
 {
     // shared memory: [sample table (renderer.cpp:49-60), spp x float2]
@@ -500,13 +500,18 @@ void launch_kernel(const TraceParams& p, int grid_blocks, int threads, size_t sm
 
 // The plain kernel exists with / without the rcp range guard (scenes larger than 1e14 units) and
 // with / without the row-band completion counters; the instrumented variants always carry both.
-// kVariantMTRel also exists with the screen cull (p.pair_sbox set); nothing else culls.
+// kVariantMTRel also exists with the screen cull (p.pair_sbox set), as the serial box check or the warp scan
+// (p.cull_scan); nothing else culls.
 template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS>
 void launch_instance(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
 {
     if constexpr (VARIANT == kVariantMTRel)
         if (p.pair_sbox)
-            return launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS, true>>(p, grid_blocks, threads, smem, stream);
+        {
+            if (p.cull_scan)
+                return launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS, kCullScan>>(p, grid_blocks, threads, smem, stream);
+            return launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS, kCullSerial>>(p, grid_blocks, threads, smem, stream);
+        }
     launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS>>(p, grid_blocks, threads, smem, stream);
 }
 

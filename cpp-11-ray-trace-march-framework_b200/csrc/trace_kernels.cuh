@@ -105,6 +105,7 @@ struct TraceParams
     unsigned long long pk_one, pk_minus_one;
     const float4 *pair_sbox;           // kVariantMTRel: screen box of every pair record for this camera (pack.cu) or
                                        // null = no screen cull
+    uint32_t cull_scan;                // with pair_sbox: 1 the warp scan of the boxes, 0 a box check per pair (warp_trace.cuh)
 };
 
 struct RayBatchParams

@@ -8,8 +8,8 @@ edge line pushed outwards by SAFETY x a bound on the image-plane error of that e
 outwards to float32.  Written operation by operation, without contraction, so that a device pre-pass can restate it
 bit for bit.
 
-Used by tools/warp_walk_model.py --screen-cull (how many pair iterations a warp could skip) and by
-tests/test_screen_cull_cpu.py (no culled ray is accepted by the oracle port)."""
+Used by tools/warp_walk_model.py --screen-cull / --warp-scan (how many pair iterations a warp could skip) and by
+tests/test_screen_cull_cpu.py (no culled ray is accepted by the oracle port) and tests/test_cull_scan_cpu.py."""
 import numpy as np
 
 EPS = 2.0 ** -24
@@ -174,6 +174,19 @@ def scene_pair_boxes(ps, cam16, fov_xs, aspect):
     inv, k, ok = camera_terms(cam16, fov_xs, aspect)
     origin = np.asarray(cam16, np.float32).reshape(-1)[12:15]
     return pstart, pair_boxes(triangle_boxes(*a, origin, inv, k, ok), triangle_boxes(*b, origin, inv, k, ok))
+
+
+def footprint_skips(boxes, x, y):
+    """The warp scan of K1's screen cull (csrc/warp_trace.cuh test_pair_list, kCullScan) for the lanes standing on one
+    cell: boxes (n, 4) float32 of the cell's pairs, x / y the float32 image points of those lanes.  -> (n,) bool, True
+    where a pair's box is disjoint from the footprint, the bounding box of the points -- then every lane lies outside
+    it.  A NaN point makes the footprint NaN, and nothing is skipped."""
+    b = np.asarray(boxes, np.float32)
+    x, y = np.asarray(x, np.float32), np.asarray(y, np.float32)
+    if np.isnan(x).any() or np.isnan(y).any():
+        return np.zeros(len(b), bool)
+    x_lo, x_hi, y_lo, y_hi = x.min(), x.max(), y.min(), y.max()
+    return (x_hi < b[:, 0]) | (x_lo > b[:, 1]) | (y_hi < b[:, 2]) | (y_lo > b[:, 3])
 
 
 def image_point(px, py, w, h, off_x, off_y, fov_xs, aspect):

@@ -11,7 +11,14 @@ With --screen-cull it replays phase B of the same warps against the screen boxes
 that owns a pair is outside its box -- the iterations K1 could skip before loading the record -- with one box per pair
 and, for comparison, one per triangle.
 
-python tools/warp_walk_model.py [workload] [n_strips] [--screen-cull]        (test infrastructure: imports oracle/)"""
+With --warp-scan it also replays the warp scan of the cull (csrc/warp_trace.cuh test_pair_list, kCullScan): in a round
+whose lanes with a list all stand on one cell, 32 boxes are checked at once against the footprint of the lanes' image
+points (screen_cull.footprint_skips) and only the pairs left are walked; other rounds keep the serial walk.  It reports
+how often the fast path applies, the 32-pair chunks, the pairs the footprint keeps against those the per-lane check
+keeps, and the pair iterations before and after; and, as the alternative for phase A, the share of a lane's occupied-
+cell visits whose point lies outside the cell's box (the union of its pair boxes).
+
+python tools/warp_walk_model.py [workload] [n_strips] [--screen-cull | --warp-scan]   (test infrastructure: imports oracle/)"""
 import ctypes as C
 import importlib
 import os
@@ -29,8 +36,9 @@ scenes, hostapi, mr = pkg("scenes"), pkg("hostapi"), pkg("multirank")
 
 C_DDA, C_TEST, C_ITER = 13, 61, 24  # SASS instructions: one DDA step, one triangle test, fixed cost of one A+B iteration
 
-CULL = "--screen-cull" in sys.argv
-args = [a for a in sys.argv[1:] if a != "--screen-cull"]
+SCAN = "--warp-scan" in sys.argv
+CULL = "--screen-cull" in sys.argv or SCAN
+args = [a for a in sys.argv[1:] if a not in ("--screen-cull", "--warp-scan")]
 wl = args[0] if args else "killeroo4k"
 n_strips = int(args[1]) if len(args) > 1 else 1500
 scene, w, h, spp, res = scenes.CONFIGS[wl]
@@ -139,6 +147,16 @@ def cull_model():
     print("pairs %d, never culled (whole plane) %.2f %%" % (len(pb), 100.0 * np.mean(np.isinf(pb[:, 0]) & (pb[:, 0] < 0))))
     ids = np.zeros(4096, np.uint32)
     cnt = dict(iters=0, skip_pair=0, skip_tri=0, lane_tests=0, lane_out=0)
+    # --warp-scan: rounds, one-cell rounds, their chunks, pair iterations, and the pairs kept by footprint / per lane
+    scan = dict(rounds=0, one_cell=0, chunks=0, iters_one=0, kept_fp=0, kept_lane=0, iters_after=0, checks_after=0,
+                visits=0, visits_out=0)
+    if SCAN:
+        ncell = len(pstart) - 1
+        cell_of = np.repeat(np.arange(ncell), np.diff(pstart))
+        cb = np.empty((ncell, 4))
+        cb[:, 0::2], cb[:, 1::2] = np.inf, -np.inf
+        for q, fn in enumerate((np.minimum, np.maximum, np.minimum, np.maximum)):
+            fn.at(cb[:, q], cell_of, pb[:, q])
     out = lambda box, j, x, y: (x < box[j, 0]) | (x > box[j, 1]) | (y < box[j, 2]) | (y > box[j, 3])
     n_x, n_y = w // sw, h // sh
     for _ in range(n_strips):
@@ -156,6 +174,11 @@ def cull_model():
                                              ids.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(hit))
                 x, y = sc.image_point(bx + ox, by + oy, w, h, smp[s, 0], smp[s, 1], fov_xs, aspect)
                 lanes.append((ids[:min(n, len(ids))].astype(np.int64).copy(), float(x), float(y)))
+                if SCAN:
+                    cells = lanes[-1][0]
+                    scan["visits"] += len(cells)
+                    scan["visits_out"] += int(((x < cb[cells, 0]) | (x > cb[cells, 1]) | (y < cb[cells, 2]) |
+                                               (y > cb[cells, 3])).sum())
         for wbase in range(0, len(lanes), 32):
             warp = lanes[wbase:wbase + 32]
             xs = np.array([l[1] for l in warp])
@@ -165,6 +188,24 @@ def cull_model():
                 cell = np.array([l[0][r] if r < len(l[0]) else 0 for l in warp])
                 beg = pstart[cell]
                 ln = np.where(has, pstart[cell + 1] - beg, 0)
+                if SCAN and ln.max() > 0:
+                    scan["rounds"] += 1
+                    on = ln > 0
+                    if len(set(beg[on])) == 1:
+                        b0, n0 = int(beg[on][0]), int(ln.max())
+                        sk = sc.footprint_skips(pb[b0:b0 + n0].astype(np.float32), xs[on], ys[on])
+                        lane_in = ~out(pb, np.arange(b0, b0 + n0)[:, None], xs[on][None, :], ys[on][None, :])
+                        assert not (sk & lane_in.any(1)).any()  # the footprint skips only pairs every lane skips
+                        scan["one_cell"] += 1
+                        scan["chunks"] += (n0 + 31) // 32
+                        scan["iters_one"] += n0
+                        scan["kept_fp"] += int((~sk).sum())
+                        scan["kept_lane"] += int(lane_in.any(1).sum())
+                        scan["iters_after"] += int((~sk).sum())
+                        scan["checks_after"] += (n0 + 31) // 32
+                    else:
+                        scan["iters_after"] += int(ln.max())
+                        scan["checks_after"] += int(ln.max())
                 for i in range(int(ln.max())):
                     mine = i < ln
                     j = beg + np.minimum(i, np.maximum(ln - 1, 0))
@@ -182,6 +223,19 @@ def cull_model():
     # a skipped iteration saves ~37 issue slots, a kept one costs ~8 more (estimated from the r02 SASS)
     for name, f in (("pair box", fp), ("triangle boxes", ft)):
         print("  %s: net instructions saved per pair iteration %.1f (37 f - 8 (1 - f))" % (name, 37 * f - 8 * (1 - f)))
+    if SCAN:
+        c = scan
+        print("warp scan: phase-B rounds %d, on one cell %d (%.1f %%); in those: %d pairs in %d chunks of 32, kept by the "
+              "footprint %d (%.1f %%), by the per-lane check %d (%.1f %%)"
+              % (c["rounds"], c["one_cell"], 100 * c["one_cell"] / c["rounds"], c["iters_one"], c["chunks"], c["kept_fp"],
+                 100 * c["kept_fp"] / c["iters_one"], c["kept_lane"], 100 * c["kept_lane"] / c["iters_one"]))
+        print("  warp pair iterations %d -> %d (%.1f %% fewer); box checks (serial: one per iteration) %d -> %d"
+              % (cnt["iters"], c["iters_after"], 100 * (1 - c["iters_after"] / cnt["iters"]), cnt["iters"],
+                 c["checks_after"]))
+        print("  %d skipped iterations of %d remain (the serial walk of multi-cell rounds, and pairs the footprint keeps)"
+              % (c["iters_after"] - (cnt["iters"] - cnt["skip_pair"]), c["iters_after"]))
+        print("cell boxes (a phase-A alternative): lane occupied-cell visits outside the cell's box %d of %d (%.1f %%)"
+              % (c["visits_out"], c["visits"], 100 * c["visits_out"] / c["visits"]))
 
 
 if CULL:
