@@ -16,6 +16,7 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <tuple>
 #include <vector>
 
 #include "grid_build.cuh"
@@ -81,7 +82,7 @@ struct DeviceState
     uint32_t *d_cancel_seen = nullptr;     // device view of h_cancel_seen
     uint32_t launched_seq = 0;             // sequence number of the frame in flight on this device
     uint64_t layout_serial = 0;            // FramePlan the device copies d_tile_rects / d_tile_prefix hold
-    std::vector<long long> occupancy_key;  // launch configuration `blocks_per_sm` was queried for
+    std::tuple<TraceTilesKernel, int, size_t> occupancy_key{}; // K1 instance, CTA size, dynamic smem `blocks_per_sm` is for
     int blocks_per_sm = 0;
     Counters *d_counters = nullptr;
     // cost-ordered scheduling (schedule.cu): cycles per strip of the last frame -> order of the next
@@ -108,11 +109,9 @@ struct Tuning
     int occ_mode = -1;     // RTM_OCC_MODE = 0 | 1 | 2 | 3 home of the occupancy map (-1: by grid size)
     int pool = -1;         // RTM_POOL = 0 | 1 pooled-ray traversal K7 for the frames it supports (-1: grids with a distance map)
     int pool_steps = 24;   // RTM_POOL_STEPS = DDA steps per ray in one walk round of K7
-    int pool_dual = 1;     // RTM_POOL_DUAL = 0 | 1 two rays per lane in K7's walk rounds
     int threads = 0;       // RTM_THREADS = CTA size (0: by frame size)
     int band_flush = 0;    // RTM_BAND_FLUSH = 1..8 strips a warp holds before publishing (0: by frame size)
     int shard_chunk = 0;   // RTM_SHARD_CHUNK = strips per deal when sharding (0: 32)
-    bool force_bands = false; // RTM_FORCE_BANDS: publish band completion without a host buffer
 };
 
 // What a frame's tile list turns into.  Kept between calls: a viewer renders the same layout every frame.
@@ -156,7 +155,6 @@ struct cuda_trace_ctx
     bool rel_records = true;    // RTM_REL_RECORDS=0: always the plain records, 2: origin-relative at any frame size (experiments)
     bool rel_records_forced = false;
     int screen_cull = -1;       // RTM_SCREEN_CULL: -1 automatic (the per-scene gate), 0 off, 1 on wherever rel records are used
-    bool cull_scan = true;      // RTM_CULL_SCAN=0: the culling K1 checks one pair box at a time instead of a warp's 32 at once
     bool fast_math = true;      // RTM_FAST_MATH=0: always the range-checked intrinsics (experiments)
     int cost_order_forced = -1; // schedule.cu: -1 automatic, 0 / 1 forced by RTM_COST_ORDER (experiments)
     std::atomic<uint64_t> launches{0};
@@ -168,7 +166,8 @@ struct cuda_trace_ctx
 
     // Overlapped read-back: the framebuffer allocation carries kMaxBands completion counters
     // behind the pixels (so IPC peers reach them through the same mapping).  K1 bumps a band's
-    // counter once per finished strip; band_expected is the running total rank 0 waits for.
+    // counter once per GPU that has finished its share of the band; band_expected is the running total
+    // rank 0 waits for.
     uint32_t band_rows = 1, n_bands = 1;
     uint32_t band_expected[kMaxBands] = {};
     std::vector<uint64_t> band_inc_sig;
@@ -180,7 +179,6 @@ struct cuda_trace_ctx
     std::vector<std::vector<uint32_t>> tile_groups;
     uint32_t *staging = nullptr;  // page-locked W x H image small frames pass through on their way into tile buffers
     size_t staging_pixels = 0;
-    bool two_level = false;       // this frame's band counters are read outside the GPU that bumps them (see plan_band_counts)
     bool overlap_d2h = true;      // RTM_OVERLAP_D2H=0 disables
     bool shard_signals = false;   // cuda_trace_set_shard_signals: other ranks bump the counters too
     int (*wait_value32)(cudaStream_t, unsigned long long, unsigned int, unsigned int) = nullptr;
@@ -560,8 +558,6 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
     }
     if (const char *e = std::getenv("RTM_SCREEN_CULL"))
         ctx->screen_cull = std::atoi(e) < 0 ? -1 : (std::atoi(e) != 0 ? 1 : 0);
-    if (const char *e = std::getenv("RTM_CULL_SCAN"))
-        ctx->cull_scan = std::atoi(e) != 0;
     if (const char *e = std::getenv("RTM_COST_ORDER"))
         ctx->cost_order_forced = std::atoi(e) != 0 ? 1 : 0;
     if (const char *e = std::getenv("RTM_FAST_MATH"))
@@ -578,8 +574,6 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
         ctx->tune.occ_mode = (std::atoi(e) >= 0 && std::atoi(e) <= 3) ? std::atoi(e) : -1;
     if (const char *e = std::getenv("RTM_POOL"))
         ctx->tune.pool = std::atoi(e) != 0 ? 1 : 0;
-    if (const char *e = std::getenv("RTM_POOL_DUAL"))
-        ctx->tune.pool_dual = std::atoi(e) != 0 ? 1 : 0;
     if (const char *e = std::getenv("RTM_POOL_STEPS"))
         ctx->tune.pool_steps = std::min(4096, std::max(1, std::atoi(e)));
     if (const char *e = std::getenv("RTM_THREADS"))
@@ -592,7 +586,6 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
         ctx->tune.band_flush = std::min(64, std::max(1, std::atoi(e)));
     if (const char *e = std::getenv("RTM_SHARD_CHUNK"))
         ctx->shard_chunk = (uint32_t) std::max(1, std::atoi(e));
-    ctx->tune.force_bands = std::getenv("RTM_FORCE_BANDS") != nullptr;
     *out = ctx;
     return 0;
 }
@@ -1051,18 +1044,14 @@ void plan_band_counts(cuda_trace_ctx *ctx)
     const FramePlan& pl = ctx->plan;
     band_layout(pl.width, pl.height, pl.strip_h, ctx->band_rows, ctx->n_bands);
     const uint32_t participants = ctx->shard_world * (uint32_t) ctx->dev.size();
-    // Two levels (ctx->two_level): every GPU counts its pieces per band in its own memory (release at GPU scope:
-    // cheap) and the warp that completes the GPU's share bumps the band counter once, at system scope -- whenever
-    // the reader is another GPU or a copy engine.  One level only for counters nobody outside this GPU reads.
-    const uint64_t two_level = ctx->two_level ? 1u : 0u;
-    const std::vector<uint64_t> sig = { pl.serial, participants, ctx->shard_chunk, two_level };
+    // Two levels: every GPU counts its pieces per band in its own memory (release at GPU scope: cheap) and the warp
+    // that completes the GPU's share bumps the band counter once, at system scope -- the reader is a copy engine or
+    // another GPU.  So a frame adds to a band's counter the number of GPUs with a share in it.
+    const std::vector<uint64_t> sig = { pl.serial, participants, ctx->shard_chunk };
     if (sig == ctx->band_inc_sig)
         return;
     band_shares(pl.rects, pl.prefix, pl.strip_w, pl.strip_h, ctx->band_rows, pl.split_parts, ctx->shard_chunk, participants,
                 ctx->band_share, ctx->band_inc);
-    if (!two_level)
-        for (int b = 0; b < kMaxBands; b++)
-            ctx->band_inc[b] = ctx->band_share[0][b];
     ctx->band_inc_sig = sig;
 }
 
@@ -1305,7 +1294,6 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     TraceParams p;
     p.grid = grid_dev(ctx, d);
     p.pair_sbox = nullptr;
-    p.cull_scan = ctx->cull_scan ? 1u : 0u;
     fill_camera(ctx, f, kind, p);
     p.smp = d.d_smp;
     p.tile_rects = d.d_tile_rects;
@@ -1326,16 +1314,11 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     p.framebuffer = ctx->d_fb;
     p.band_done = use_bands ? band_counters(ctx) : nullptr;
     p.band_rows = ctx->band_rows;
-    p.band_local = ctx->two_level ? d.d_strip_counter + 32 : nullptr; // own cache line
+    p.band_local = use_bands ? d.d_strip_counter + 32 : nullptr; // own cache line
     std::memset(p.band_share, 0, sizeof(p.band_share));
     if (use_bands)
         std::memcpy(p.band_share, ctx->band_share[p.shard_rank].data(), sizeof(p.band_share));
-    // Who reads the band counters and the pixels behind them?  Another GPU's memory or a copy engine: neither is
-    // inside this GPU's .gpu scope, so the publishing release is at system scope.  (.gpu only for RTM_FORCE_BANDS
-    // runs without a reader.)
-    p.band_scope_sys = ctx->two_level ? 1u : 0u;
     p.pool_walk_steps = 0;
-    p.pool_dual = 0;
     p.hit_tri = kind.keep_hits ? ctx->d_hit_tri : nullptr;
     p.hit_t = kind.keep_hits ? ctx->d_hit_t : nullptr;
     p.hit_u = kind.keep_hits ? ctx->d_hit_u : nullptr;
@@ -1373,27 +1356,6 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     const uint32_t kvariant = kind.alternates ? (uint32_t) kVariantMTAlt + f->variant
                               : (f->variant == kVariantMT && !kind.count_inst && ctx->rel_records && rel_fits)
                                   ? (uint32_t) kVariantMTRel : f->variant;
-    const size_t smem_bytes = trace_tiles_smem_bytes(f->spp, p.occ_smem_words);
-    const std::vector<long long> okey = { (long long) kvariant, kind.keep_hits, kind.count_inst, (long long) p.occ_mode, threads,
-                                          (long long) smem_bytes };
-    if (okey != d.occupancy_key)
-    {
-        d.blocks_per_sm = std::max(1, trace_tiles_max_blocks_per_sm(kvariant, kind.keep_hits, kind.count_inst, (int) p.occ_mode,
-                                                                    threads, smem_bytes));
-        d.occupancy_key = okey;
-    }
-    const uint64_t want = (strips_here + (threads / 32) - 1) / (threads / 32);
-    const int blocks = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) d.sm_count * d.blocks_per_sm, want));
-    {
-        // How many finished strips a warp collects before it publishes them to the band counters: the fence
-        // costs ~1 us, but a held-back strip delays its band's read-back -- at most 1/16 of a warp's share
-        // of the frame (8 strips for a whole 4K frame on one GPU, every strip for an eighth of it)
-        const uint64_t warps = (uint64_t) blocks * (threads / 32);
-        uint64_t hold = std::min<uint64_t>(8, std::max<uint64_t>(1, strips_here / std::max<uint64_t>(1, warps * 16)));
-        if (ctx->tune.band_flush)
-            hold = (uint64_t) ctx->tune.band_flush;
-        p.band_flush_units = (uint32_t) hold * pl.split_parts;
-    }
     if (i == 0)
         ctx->t_launching_ms = ms_since(ctx->t_enter);
     CK(cudaEventRecord(d.ev_begin, d.stream));
@@ -1444,12 +1406,33 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
                 p.pair_sbox = d.d_pair_sbox;
         }
     }
+    // K1's instance for this frame, now that the records and the cull are decided, and the grid its occupancy allows
+    const TraceTilesKernel kernel = trace_tiles_instance(kvariant, kind.keep_hits, kind.count_inst, (int) p.occ_mode,
+                                                         p.rcp_guard != 0, p.band_done != nullptr, p.pair_sbox != nullptr);
+    const size_t smem_bytes = trace_tiles_smem_bytes(f->spp, p.occ_smem_words);
+    const std::tuple<TraceTilesKernel, int, size_t> okey(kernel, threads, smem_bytes);
+    if (okey != d.occupancy_key)
+    {
+        d.blocks_per_sm = std::max(1, trace_tiles_max_blocks_per_sm(kernel, threads, smem_bytes));
+        d.occupancy_key = okey;
+    }
+    const uint64_t want = (strips_here + (threads / 32) - 1) / (threads / 32);
+    const int blocks = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) d.sm_count * d.blocks_per_sm, want));
+    {
+        // How many finished strips a warp collects before it publishes them to the band counters: the fence
+        // costs ~1 us, but a held-back strip delays its band's read-back -- at most 1/16 of a warp's share
+        // of the frame (8 strips for a whole 4K frame on one GPU, every strip for an eighth of it)
+        const uint64_t warps = (uint64_t) blocks * (threads / 32);
+        uint64_t hold = std::min<uint64_t>(8, std::max<uint64_t>(1, strips_here / std::max<uint64_t>(1, warps * 16)));
+        if (ctx->tune.band_flush)
+            hold = (uint64_t) ctx->tune.band_flush;
+        p.band_flush_units = (uint32_t) hold * pl.split_parts;
+    }
     if (pl.total && use_pool)
     {
         // hit records: the caller's (KEEP_HITS, device 0) or this device's own
         TraceParams pp = p;
         pp.pool_walk_steps = (uint32_t) ctx->tune.pool_steps;
-        pp.pool_dual = (uint32_t) ctx->tune.pool_dual;
         if (!kind.keep_hits)
         {
             const uint64_t need = (uint64_t) f->width * f->height * f->spp;
@@ -1472,19 +1455,20 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
         // K1 behind it: shading, in-order sample sum, resolve, band publication -- from the hit records
         pp.occ_mode = kOccGlobalBits;
         pp.occ_smem_words = 0;
+        const TraceTilesKernel resolve = trace_tiles_instance(kVariantFromHits, false, false, kOccGlobalBits, pp.rcp_guard != 0,
+                                                              pp.band_done != nullptr, false);
         if (d.resolve_threads != threads)
         {
-            d.resolve_blocks_per_sm = std::max(1, trace_tiles_max_blocks_per_sm(kVariantFromHits, false, false, kOccGlobalBits, threads,
-                                                                              trace_tiles_smem_bytes(f->spp, 0)));
+            d.resolve_blocks_per_sm = std::max(1, trace_tiles_max_blocks_per_sm(resolve, threads, trace_tiles_smem_bytes(f->spp, 0)));
             d.resolve_threads = threads;
         }
         const int resolve_blocks = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) d.sm_count * d.resolve_blocks_per_sm, want));
-        launch_trace_tiles(pp, kVariantFromHits, false, false, resolve_blocks, threads, d.stream);
+        launch_trace_tiles(resolve, pp, resolve_blocks, threads, d.stream);
         ctx->launches += 2;
     }
     else if (pl.total)
     {
-        launch_trace_tiles(p, kvariant, kind.keep_hits, kind.count_inst, blocks, threads, d.stream);
+        launch_trace_tiles(kernel, p, blocks, threads, d.stream);
         ctx->launches++;
     }
     if (i == 0)
@@ -1671,9 +1655,8 @@ static int tiles_async_impl(cuda_trace_ctx *ctx, const cuda_trace_frame *f, cons
     const bool bands_usable = ctx->overlap_d2h && ctx->wait_value32 && !ctx->fb_imported && pl.total > 0 &&
                               (ctx->shard_world == 1 || ctx->shard_signals);
     const bool can_overlap = (host_bgra && bands_usable && pl.covers_frame) || (dst.tile && bands_usable);
-    const bool use_bands = ctx->shard_signals || can_overlap || ctx->tune.force_bands;
+    const bool use_bands = ctx->shard_signals || can_overlap;
     ctx->tile_groups.clear();
-    ctx->two_level = ctx->shard_world * n_dev > 1 || ctx->fb_imported || ctx->shard_signals || can_overlap;
     if (use_bands)
         plan_band_counts(ctx);
 

@@ -284,7 +284,7 @@ __global__ void __launch_bounds__(kTraceMaxThreads) trace_pool_kernel(const __gr
             // pool has them, so that one ray's look-up is in flight while the other one steps.  A ray that has
             // arrived idles until the round's budget is used up or every ray has arrived
             pick_slots(pw, lane, walkers);
-            const uint32_t n_round = min(n_walk, p.pool_dual ? 64u : 32u);
+            const uint32_t n_round = min(n_walk, 64u);
             Walker wa, wb;
             walker_load(pw, pw.list[lane < n_round ? lane : 0u], lane < n_round, lane, stride_y, stride_z, dist, wa);
             walker_load(pw, pw.list[lane + 32u < n_round ? lane + 32u : 0u], lane + 32u < n_round, lane, stride_y, stride_z, dist, wb);

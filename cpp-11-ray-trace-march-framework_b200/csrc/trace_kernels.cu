@@ -12,6 +12,9 @@
 #include "trace_kernels.cuh"
 #include "warp_trace.cuh"
 
+#include <map>
+#include <mutex>
+
 namespace rtm
 {
 
@@ -23,7 +26,7 @@ constexpr unsigned kFull = 0xFFFFFFFFu;
 constexpr size_t kOptInDynamicSmem = 24 * 1024;
 
 // One sample per lane; ALL lanes of the warp call this together (valid == false: no ray)
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, int CULL>
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool CULL>
 __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void *s_occ, bool valid,
                                                uint32_t px, uint32_t py, uint32_t s, const float2 *smp, Counters *cnt)
 {
@@ -56,7 +59,7 @@ __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void 
         PackedUnits pku;
         pku.one = p.pk_one;
         pku.minus_one = p.pk_minus_one;
-        if constexpr (CULL != kCullOff)
+        if constexpr (CULL)
             is_hit = warp_grid_intersect<TRI_VARIANT, COUNT, OCC_MODE, RCP_GUARD, false, false, CULL>(
                 p.grid, s_occ, o, d, valid, hit, cnt, pku, p.cam.fast_math != 0, FLT_MAX, p.pair_sbox, img);
         else
@@ -81,38 +84,23 @@ __device__ __forceinline__ float3 trace_sample(const TraceParams& p, const void 
 // its own memory: pieces of strips finished, a release at GPU scope -- cheap, once per few strips (no acquire
 // here: that would invalidate the SM's L1 and cost 6 % of the frame).  Level 2: the warp whose increment
 // completes this GPU's share of the band turns it into an acquire with a fence and bumps the band's counter
-// behind the (possibly remote) framebuffer, once per band and GPU, with a release at the scope that counter
-// needs.  Every pixel store of the band on this GPU happens-before that release (warp barrier -> level-1
-// release -> level-1 read + acquire fence by the completing warp -> its release; causality order is
-// cumulative), so whoever waits on the band counter sees the pixels.  A system-scope release per strip batch
-// instead costs +35 % kernel time on the GPUs that store over NVLink.
+// behind the (possibly remote) framebuffer, once per band and GPU, with a release at system scope: the counter's
+// reader is a copy engine or another GPU, neither inside this GPU's .gpu scope.  Every pixel store of the band on
+// this GPU happens-before that release (warp barrier -> level-1 release -> level-1 read + acquire fence by the
+// completing warp -> its release; causality order is cumulative), so whoever waits on the band counter sees the
+// pixels.  A system-scope release per strip batch instead costs +35 % kernel time on the GPUs that store over NVLink.
 __device__ __forceinline__ void release_add(const TraceParams& p, uint32_t band, uint32_t count)
 {
-    if (!p.band_local) // a single GPU rendering into its own framebuffer: one level, the band counter counts pieces
-    {
-        // (system scope when a copy engine waits on the counter and reads the pixels: it is not in this GPU's .gpu scope)
-        if (p.band_scope_sys)
-            asm volatile("red.release.sys.global.add.u32 [%0], %1;" :: "l"(p.band_done + band), "r"(count) : "memory");
-        else
-            asm volatile("red.release.gpu.global.add.u32 [%0], %1;" :: "l"(p.band_done + band), "r"(count) : "memory");
-        return;
-    }
     uint32_t before;
     asm volatile("atom.release.gpu.global.add.u32 %0, [%1], %2;" : "=r"(before) : "l"(p.band_local + band), "r"(count) : "memory");
     if (before + count == p.band_share[band])
     {
-        if (p.band_scope_sys)
-            asm volatile("fence.acq_rel.sys;" ::: "memory");
-        else
-            asm volatile("fence.acq_rel.gpu;" ::: "memory");
-        if (p.band_scope_sys)
-            asm volatile("red.release.sys.global.add.u32 [%0], %1;" :: "l"(p.band_done + band), "r"(1u) : "memory");
-        else
-            asm volatile("red.release.gpu.global.add.u32 [%0], %1;" :: "l"(p.band_done + band), "r"(1u) : "memory");
+        asm volatile("fence.acq_rel.sys;" ::: "memory");
+        asm volatile("red.release.sys.global.add.u32 [%0], %1;" :: "l"(p.band_done + band), "r"(1u) : "memory");
     }
 }
 
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS, int CULL = kCullOff>
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS, bool CULL>
 __global__ void __launch_bounds__(kTraceMaxThreads) trace_tiles_kernel(const __grid_constant__ TraceParams p)
 {
     // shared memory: [sample table (renderer.cpp:49-60), spp x float2]
@@ -479,134 +467,110 @@ __global__ void sample_table_kernel(float2 *smp, uint32_t spp)
     smp[s] = make_float2((float) (x - 0.5), (float) (val - 0.5));
 }
 
-template <auto KERNEL>
-void launch_kernel(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
+// The instance set of trace_tiles_kernel.  The plain kernel (no hit records, no counters, not an alternate) exists with
+// and without the rcp range guard (scenes larger than 1e14 units) and with and without the row-band completion
+// counters; every other kernel carries both
+template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool CULL>
+TraceTilesKernel instance_by_flags(bool rcp_guard, bool bands)
 {
-    if (smem > kOptInDynamicSmem)
+    if constexpr (!KEEP_HITS && !COUNT && VARIANT < kVariantMTAlt)
     {
-        // opt in to large dynamic shared memory once per device and size, not on every launch
-        static size_t opted_in[64] = {};
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (dev < 0 || dev >= 64 || opted_in[dev] < smem)
-        {
-            cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-            if (dev >= 0 && dev < 64)
-                opted_in[dev] = smem;
-        }
+        if (!rcp_guard && !bands) return trace_tiles_kernel<VARIANT, false, false, OCC_MODE, false, false, CULL>;
+        if (!rcp_guard)           return trace_tiles_kernel<VARIANT, false, false, OCC_MODE, false, true, CULL>;
+        if (!bands)               return trace_tiles_kernel<VARIANT, false, false, OCC_MODE, true, false, CULL>;
     }
-    KERNEL<<<grid_blocks, threads, smem, stream>>>(p);
+    return trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, true, true, CULL>;
 }
 
-// The plain kernel exists with / without the rcp range guard (scenes larger than 1e14 units) and
-// with / without the row-band completion counters; the instrumented variants always carry both.
-// kVariantMTRel also exists with the screen cull (p.pair_sbox set), as the serial box check or the warp scan
-// (p.cull_scan); nothing else culls.
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE, bool RCP_GUARD, bool BANDS>
-void launch_instance(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
+template <int VARIANT, bool KEEP_HITS, bool COUNT, bool CULL>
+TraceTilesKernel instance_by_occ(int occ_mode, bool rcp_guard, bool bands)
+{
+    switch (occ_mode)
+    {
+        case kOccSmemBits: return instance_by_flags<VARIANT, KEEP_HITS, COUNT, kOccSmemBits, CULL>(rcp_guard, bands);
+        case kOccSmemBytes: return instance_by_flags<VARIANT, KEEP_HITS, COUNT, kOccSmemBytes, CULL>(rcp_guard, bands);
+        case kOccGlobalDist: return instance_by_flags<VARIANT, KEEP_HITS, COUNT, kOccGlobalDist, CULL>(rcp_guard, bands);
+        default: return instance_by_flags<VARIANT, KEEP_HITS, COUNT, kOccGlobalBits, CULL>(rcp_guard, bands);
+    }
+}
+
+// the screen cull exists for kVariantMTRel only: the boxes belong to the origin-relative records
+template <int VARIANT, bool KEEP_HITS, bool COUNT>
+TraceTilesKernel instance_by_cull(int occ_mode, bool rcp_guard, bool bands, bool cull)
 {
     if constexpr (VARIANT == kVariantMTRel)
-        if (p.pair_sbox)
-        {
-            if (p.cull_scan)
-                return launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS, kCullScan>>(p, grid_blocks, threads, smem, stream);
-            return launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS, kCullSerial>>(p, grid_blocks, threads, smem, stream);
-        }
-    launch_kernel<trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, RCP_GUARD, BANDS>>(p, grid_blocks, threads, smem, stream);
+        if (cull)
+            return instance_by_occ<VARIANT, KEEP_HITS, COUNT, true>(occ_mode, rcp_guard, bands);
+    return instance_by_occ<VARIANT, KEEP_HITS, COUNT, false>(occ_mode, rcp_guard, bands);
 }
 
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE>
-void launch_mode(const TraceParams& p, int grid_blocks, int threads, size_t smem, cudaStream_t stream)
+// the work counters exist for variants 0 and 1 only, the hit records for every variant that traverses
+template <int VARIANT>
+TraceTilesKernel instance_by_records(bool keep_hits, bool count, int occ_mode, bool rcp_guard, bool bands, bool cull)
 {
-    constexpr bool kPlain = !KEEP_HITS && !COUNT && VARIANT < kVariantMTAlt; // the alternates: one instantiation each
-    if (kPlain)
-    {
-        const bool guard = p.rcp_guard != 0, bands = p.band_done != nullptr;
-        if (!guard && !bands) return launch_instance<VARIANT, KEEP_HITS, COUNT, OCC_MODE, !kPlain, !kPlain>(p, grid_blocks, threads, smem, stream);
-        if (!guard && bands)  return launch_instance<VARIANT, KEEP_HITS, COUNT, OCC_MODE, !kPlain, true>(p, grid_blocks, threads, smem, stream);
-        if (guard && !bands)  return launch_instance<VARIANT, KEEP_HITS, COUNT, OCC_MODE, true, !kPlain>(p, grid_blocks, threads, smem, stream);
-    }
-    launch_instance<VARIANT, KEEP_HITS, COUNT, OCC_MODE, true, true>(p, grid_blocks, threads, smem, stream);
+    constexpr bool kCounts = VARIANT == kVariantMT || VARIANT == kVariantBary, kHits = VARIANT != kVariantFromHits;
+    if constexpr (kCounts)
+        if (count)
+            return keep_hits ? instance_by_cull<VARIANT, true, true>(occ_mode, rcp_guard, bands, cull)
+                             : instance_by_cull<VARIANT, false, true>(occ_mode, rcp_guard, bands, cull);
+    if constexpr (kHits)
+        if (keep_hits)
+            return instance_by_cull<VARIANT, true, false>(occ_mode, rcp_guard, bands, cull);
+    return instance_by_cull<VARIANT, false, false>(occ_mode, rcp_guard, bands, cull);
 }
 
-template <int VARIANT, bool KEEP_HITS, bool COUNT>
-void launch_one(const TraceParams& p, int grid_blocks, int threads, cudaStream_t stream)
+// opt in to large dynamic shared memory once per device, kernel and size, not on every launch
+void opt_in_smem(TraceTilesKernel k, size_t smem)
 {
-    const size_t smem = trace_tiles_smem_bytes(p.spp, p.occ_smem_words);
-    if (p.occ_mode == kOccSmemBytes)
-        launch_mode<VARIANT, KEEP_HITS, COUNT, kOccSmemBytes>(p, grid_blocks, threads, smem, stream);
-    else if (p.occ_mode == kOccSmemBits)
-        launch_mode<VARIANT, KEEP_HITS, COUNT, kOccSmemBits>(p, grid_blocks, threads, smem, stream);
-    else if (p.occ_mode == kOccGlobalDist)
-        launch_mode<VARIANT, KEEP_HITS, COUNT, kOccGlobalDist>(p, grid_blocks, threads, smem, stream);
-    else
-        launch_mode<VARIANT, KEEP_HITS, COUNT, kOccGlobalBits>(p, grid_blocks, threads, smem, stream);
-}
-
-template <int VARIANT, bool KEEP_HITS, bool COUNT, int OCC_MODE>
-int occupancy_mode(int threads, size_t smem)
-{
-    int n = 0;
-    if (smem > kOptInDynamicSmem)
-        cudaFuncSetAttribute(trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, true, true>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, trace_tiles_kernel<VARIANT, KEEP_HITS, COUNT, OCC_MODE, true, true>, threads, smem);
-    return n;
-}
-
-template <int VARIANT, bool KEEP_HITS, bool COUNT>
-int occupancy_one(int occ_mode, int threads, size_t smem)
-{
-    if (occ_mode == kOccSmemBytes)
-        return occupancy_mode<VARIANT, KEEP_HITS, COUNT, kOccSmemBytes>(threads, smem);
-    if (occ_mode == kOccSmemBits)
-        return occupancy_mode<VARIANT, KEEP_HITS, COUNT, kOccSmemBits>(threads, smem);
-    if (occ_mode == kOccGlobalDist)
-        return occupancy_mode<VARIANT, KEEP_HITS, COUNT, kOccGlobalDist>(threads, smem);
-    return occupancy_mode<VARIANT, KEEP_HITS, COUNT, kOccGlobalBits>(threads, smem);
+    if (smem <= kOptInDynamicSmem)
+        return;
+    static std::mutex mtx;
+    static std::map<std::pair<TraceTilesKernel, int>, size_t> opted_in;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    std::lock_guard<std::mutex> lock(mtx);
+    size_t& done = opted_in[{ k, dev }];
+    if (done < smem && cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem) == cudaSuccess)
+        done = smem;
 }
 
 } // namespace
 
-// variants 2 (origin-relative records) and 3 / 4 (alternates) exist without the counting instrumentation only
-#define RTM_DISPATCH(FN, ...)                                                                    \
-    do {                                                                                         \
-        const int key = (int) (variant == kVariantMTRel && count ? 0u : variant) * 4 | (keep_hits ? 2 : 0) | (count ? 1 : 0); \
-        switch (key)                                                                             \
-        {                                                                                        \
-            case 8: return FN<2, false, false>(__VA_ARGS__);                                     \
-            case 10: return FN<2, true, false>(__VA_ARGS__);                                     \
-            case 12: case 13: return FN<3, false, false>(__VA_ARGS__);                           \
-            case 14: case 15: return FN<3, true, false>(__VA_ARGS__);                            \
-            case 16: case 17: return FN<4, false, false>(__VA_ARGS__);                           \
-            case 18: case 19: return FN<4, true, false>(__VA_ARGS__);                            \
-            case 20: case 21: case 22: case 23: return FN<5, false, false>(__VA_ARGS__);         \
-            case 0: return FN<0, false, false>(__VA_ARGS__);                                     \
-            case 1: return FN<0, false, true>(__VA_ARGS__);                                      \
-            case 2: return FN<0, true, false>(__VA_ARGS__);                                      \
-            case 3: return FN<0, true, true>(__VA_ARGS__);                                       \
-            case 4: return FN<1, false, false>(__VA_ARGS__);                                     \
-            case 5: return FN<1, false, true>(__VA_ARGS__);                                      \
-            case 6: return FN<1, true, false>(__VA_ARGS__);                                      \
-            default: return FN<1, true, true>(__VA_ARGS__);                                      \
-        }                                                                                        \
-    } while (0)
+TraceTilesKernel trace_tiles_instance(uint32_t variant, bool keep_hits, bool count, int occ_mode, bool rcp_guard, bool bands,
+                                      bool cull)
+{
+    switch (variant)
+    {
+        case kVariantMT: return instance_by_records<kVariantMT>(keep_hits, count, occ_mode, rcp_guard, bands, cull);
+        case kVariantBary: return instance_by_records<kVariantBary>(keep_hits, count, occ_mode, rcp_guard, bands, cull);
+        case kVariantMTRel: // the counting kernels walk the plain records
+            return count ? instance_by_records<kVariantMT>(keep_hits, count, occ_mode, rcp_guard, bands, cull)
+                         : instance_by_records<kVariantMTRel>(keep_hits, count, occ_mode, rcp_guard, bands, cull);
+        case kVariantMTAlt: return instance_by_records<kVariantMTAlt>(keep_hits, count, occ_mode, rcp_guard, bands, cull);
+        case kVariantBaryAlt: return instance_by_records<kVariantBaryAlt>(keep_hits, count, occ_mode, rcp_guard, bands, cull);
+        case kVariantFromHits: return instance_by_records<kVariantFromHits>(keep_hits, count, occ_mode, rcp_guard, bands, cull);
+        default: return nullptr;
+    }
+}
 
 size_t trace_tiles_smem_bytes(uint32_t spp, uint32_t occ_smem_words)
 {
     return sizeof(float2) * spp + sizeof(uint32_t) * occ_smem_words;
 }
 
-void launch_trace_tiles(const TraceParams& p, uint32_t variant, bool keep_hits, bool count, int grid_blocks,
-                        int threads, cudaStream_t stream)
+void launch_trace_tiles(TraceTilesKernel k, const TraceParams& p, int grid_blocks, int threads, cudaStream_t stream)
 {
-    RTM_DISPATCH(launch_one, p, grid_blocks, threads, stream);
+    const size_t smem = trace_tiles_smem_bytes(p.spp, p.occ_smem_words);
+    opt_in_smem(k, smem);
+    k<<<grid_blocks, threads, smem, stream>>>(p);
 }
 
-int trace_tiles_max_blocks_per_sm(uint32_t variant, bool keep_hits, bool count, int occ_mode, int threads,
-                                  size_t smem_bytes)
+int trace_tiles_max_blocks_per_sm(TraceTilesKernel k, int threads, size_t smem_bytes)
 {
-    RTM_DISPATCH(occupancy_one, occ_mode, threads, smem_bytes);
+    int n = 0;
+    opt_in_smem(k, smem_bytes);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, threads, smem_bytes);
+    return n;
 }
 
 void launch_intersect_rays(const RayBatchParams& p, uint32_t variant, cudaStream_t stream)

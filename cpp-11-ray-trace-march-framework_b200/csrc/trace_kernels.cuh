@@ -80,6 +80,7 @@ struct TraceParams
     const uint32_t *fetch_order;       // cost-ordered visit list of this shard (schedule.cu) or null = strips in image order
     const uint32_t *visit_total;       // device word: entries in fetch_order
     uint32_t split_parts;              // pieces an expensive strip is visited in (strip_split_parts); band counters count pieces
+    uint32_t pool_walk_steps;          // K7: DDA steps per ray in one walk round
     uint32_t *visit_cycles;            // out: cycles spent per visit (feeds the next frame's order, schedule.cu) or null
     uint32_t *strip_counter;           // dynamic strip scheduler (zeroed before launch)
     const uint32_t *cancel;            // == frame_seq => stop tracing (the word names the frame to cancel, api.cu)
@@ -89,14 +90,10 @@ struct TraceParams
     uint32_t *band_done;               // per row band: GPUs whose share of the band is finished (monotone across frames;
                                        // lives behind the framebuffer, so peers / other ranks reach it through the
                                        // same mapping) or null
-    uint32_t *band_local;              // per row band: pieces of strips THIS GPU has finished in this frame (local memory);
-                                       // null = single GPU, band_done counts pieces directly
+    uint32_t *band_local;              // per row band: pieces of strips THIS GPU has finished in this frame (local memory)
     uint32_t band_share[kMaxBands];    // ... and how many that makes when its share of the band is complete
     uint32_t band_rows;                // rows per band
     uint32_t band_flush_units;         // a warp publishes its finished pieces once it holds this many
-    uint32_t band_scope_sys;           // 1: counters / pixels may live on another GPU (system-scope release), 0: local
-    uint32_t pool_walk_steps;          // K7: DDA steps per ray in one walk round
-    uint32_t pool_dual;                // K7: walk rounds take two rays per lane when the pool has them
     uint32_t *hit_tri;                 // optional per-sample records (KEEP_HITS)
     float *hit_t, *hit_u, *hit_v;
     Counters *counters;                // optional (COUNT)
@@ -105,7 +102,6 @@ struct TraceParams
     unsigned long long pk_one, pk_minus_one;
     const float4 *pair_sbox;           // kVariantMTRel: screen box of every pair record for this camera (pack.cu) or
                                        // null = no screen cull
-    uint32_t cull_scan;                // with pair_sbox: 1 the warp scan of the boxes, 0 a box check per pair (warp_trace.cuh)
 };
 
 struct RayBatchParams
@@ -135,13 +131,19 @@ struct RayQueryParams
     unsigned long long pk_one, pk_minus_one;
 };
 
-void launch_trace_tiles(const TraceParams& p, uint32_t variant, bool keep_hits, bool count, int grid_blocks,
-                        int threads, cudaStream_t stream);
-int trace_tiles_max_blocks_per_sm(uint32_t variant, bool keep_hits, bool count, int occ_mode, int threads,
-                                  size_t smem_bytes);
+// K1 (trace_kernels.cu): the kernel instance for a frame's intersection variant, per-sample hit records (KEEP_HITS),
+// work counters (COUNT), occupancy map home, rcp range guard (TraceParams::rcp_guard), band publication
+// (TraceParams::band_done set) and screen cull (TraceParams::pair_sbox set).  Only the plain kernel exists without the
+// guard or without band publication (the others test rcp_guard and band_done at run time); the work counters exist for
+// variants 0 and 1 (2 counts as 0), the cull for variant 2.  Null for an unknown variant.
+using TraceTilesKernel = void (*)(TraceParams);
+TraceTilesKernel trace_tiles_instance(uint32_t variant, bool keep_hits, bool count, int occ_mode, bool rcp_guard, bool bands,
+                                      bool cull);
+void launch_trace_tiles(TraceTilesKernel k, const TraceParams& p, int grid_blocks, int threads, cudaStream_t stream);
+int trace_tiles_max_blocks_per_sm(TraceTilesKernel k, int threads, size_t smem_bytes);
 size_t trace_tiles_smem_bytes(uint32_t spp, uint32_t occ_smem_words);
 // K7: traverses the strips of this launch's shard with pooled rays and leaves (tri, t, u, v) per sample in p.hit_*
-// (all four required); follow it with launch_trace_tiles(variant = kVariantFromHits) on the same stream
+// (all four required); follow it with K1 in variant kVariantFromHits on the same stream
 void launch_trace_pool(const TraceParams& p, int grid_blocks, int threads, cudaStream_t stream);
 size_t trace_pool_smem_bytes(uint32_t spp, int threads);
 // the scalar one-thread-per-ray walk, kept for the mailboxing mode of cuda_trace_intersect_rays (the plain mode runs

@@ -1,4 +1,4 @@
-"""The warp scan of K1's screen cull (csrc/warp_trace.cuh test_pair_list, kCullScan) restated on the CPU
+"""The warp scan of K1's screen cull (csrc/warp_trace.cuh test_pair_list) restated on the CPU
 (tools/screen_cull.py footprint_skips): a pair whose box is disjoint from the footprint of a warp's image points -- their
 bounding box -- has every lane outside it, and walking only the pairs the footprint keeps, in ascending list position,
 gives every lane the (tri, t, u, v) of the serial walk that checks each pair's box against every lane.  Checked on the

@@ -87,7 +87,7 @@ def test_default_instantiation_reproduces_full_size_reference_frames(key):
     d = DIGESTS[key]
     capi, hostapi = pkg("capi"), pkg("hostapi")
     for var in ("RTM_REL_RECORDS", "RTM_OCC_MODE", "RTM_THREADS", "RTM_COST_ORDER", "RTM_STRIP_PIXELS", "RTM_FAST_MATH",
-                "RTM_OVERLAP_D2H", "RTM_FORCE_BANDS"):
+                "RTM_OVERLAP_D2H"):
         assert var not in os.environ
     vtx, tri, fov, cam = host_scene(d["scene"])
     w, h, spp = d["width"], d["height"], d["spp"]

@@ -177,7 +177,7 @@ def scene_pair_boxes(ps, cam16, fov_xs, aspect):
 
 
 def footprint_skips(boxes, x, y):
-    """The warp scan of K1's screen cull (csrc/warp_trace.cuh test_pair_list, kCullScan) for the lanes standing on one
+    """The warp scan of K1's screen cull (csrc/warp_trace.cuh test_pair_list) for the lanes standing on one
     cell: boxes (n, 4) float32 of the cell's pairs, x / y the float32 image points of those lanes.  -> (n,) bool, True
     where a pair's box is disjoint from the footprint, the bounding box of the points -- then every lane lies outside
     it.  A NaN point makes the footprint NaN, and nothing is skipped."""

@@ -11,7 +11,7 @@ With --screen-cull it replays phase B of the same warps against the screen boxes
 that owns a pair is outside its box -- the iterations K1 could skip before loading the record -- with one box per pair
 and, for comparison, one per triangle.
 
-With --warp-scan it also replays the warp scan of the cull (csrc/warp_trace.cuh test_pair_list, kCullScan): in a round
+With --warp-scan it also replays the warp scan of the cull (csrc/warp_trace.cuh test_pair_list): in a round
 whose lanes with a list all stand on one cell, 32 boxes are checked at once against the footprint of the lanes' image
 points (screen_cull.footprint_skips) and only the pairs left are walked; other rounds keep the serial walk.  It reports
 how often the fast path applies, the 32-pair chunks, the pairs the footprint keeps against those the per-lane check
