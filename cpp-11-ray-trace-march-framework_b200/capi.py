@@ -63,6 +63,8 @@ SYMBOLS = {
     "cuda_trace_set_shard": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
     "cuda_trace_set_shard_signals": (C.c_int, [C.c_void_p, C.c_int]),
     "cuda_trace_upload_scene": (C.c_int, [C.c_void_p, _F32P, C.c_uint32, _U32P, C.c_uint32, C.c_uint32]),
+    "cuda_trace_upload_scene_device": (C.c_int, [C.c_void_p, _F32P, C.c_uint32, _U32P, C.c_uint32, C.c_uint32,
+                                                 C.c_void_p]),
     "cuda_trace_suggest_grid_res": (C.c_uint32, [C.c_uint32]),
     "cuda_trace_upload_scene_with_grid": (C.c_int, [C.c_void_p, _F32P, C.c_uint32, _U32P, C.c_uint32,
                                                     C.POINTER(GridDesc), _U64P, _U32P]),
@@ -269,6 +271,43 @@ class CudaTrace:
         vtx = np.ascontiguousarray(vtx, np.float32)
         tri = np.ascontiguousarray(tri, np.uint32)
         self._ck(self.lib.cuda_trace_upload_scene(self.h, _p(vtx, _F32P), len(vtx), _p(tri, _U32P), len(tri), grid_res))
+
+    def upload_scene_device(self, vertices, triangles, grid_res=64, stream=None):
+        """cuda_trace_upload_scene_device on torch CUDA tensors of the context's first device: ``vertices`` float32
+        (V, 6), position and normal per vertex; ``triangles`` int32 or uint32 (T, 6) in the Mesh layout, columns 0-2
+        the vertex indices and columns 3-5 the float32 bits of the face normal.  From (T, 3) indices ``idx`` and
+        (T, 3) float32 normals ``n``::
+
+            triangles = torch.cat([idx.int(), n.view(torch.int32)], 1)
+
+        Queries need only the positions and the indices; frames shade with the normals given.  The call orders
+        itself after the work enqueued on ``stream`` (default: torch's current stream) and returns once the scene is
+        built, so the tensors may be overwritten or freed right after.  The result is bit-identical to
+        ``upload_scene`` on the same values."""
+        import torch
+        dev = torch.device("cuda", self.devices[0])
+
+        def check(x, name, dtypes):
+            if not isinstance(x, torch.Tensor):
+                raise TypeError("%s must be a torch tensor" % name)
+            if x.device != dev:
+                raise ValueError("%s must be on %s (got %s)" % (name, dev, x.device))
+            if x.dtype not in dtypes:
+                raise TypeError("%s must be %s (got %s)" % (name, " or ".join(str(t) for t in dtypes), x.dtype))
+            if x.dim() != 2 or x.shape[1] != 6 or not 0 < x.shape[0] < 2 ** 32:
+                raise ValueError("%s must have shape (n, 6) with 0 < n < 2^32 (got %s)" % (name, tuple(x.shape)))
+            return x.contiguous()
+
+        index_dtypes = (torch.int32,) + ((torch.uint32,) if hasattr(torch, "uint32") else ())
+        stream = torch.cuda.current_stream(dev) if stream is None else stream
+        with torch.cuda.stream(stream):
+            v = check(vertices, "vertices", (torch.float32,))
+            t = check(triangles, "triangles", index_dtypes)
+            # torch's default stream is the legacy NULL stream, which the C call would read as "the context's
+            # stream": name it as cudaStreamLegacy (0x1) instead
+            self._ck(self.lib.cuda_trace_upload_scene_device(self.h, C.cast(v.data_ptr(), _F32P), v.shape[0],
+                                                             C.cast(t.data_ptr(), _U32P), t.shape[0], grid_res,
+                                                             C.c_void_p(stream.cuda_stream or 1)))
 
     def upload_scene_with_grid(self, vtx, tri, grid):
         vtx = np.ascontiguousarray(vtx, np.float32)

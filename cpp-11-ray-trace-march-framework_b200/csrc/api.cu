@@ -204,6 +204,12 @@ struct cuda_trace_ctx
     // cuda_trace_query_rays: per stream the context has been given, an event behind its last query (device 0).
     // Replacing the scene or destroying the context waits for them before the scene arrays are freed.
     std::vector<std::pair<cudaStream_t, cudaEvent_t>> query_events;
+
+    // cuda_trace_upload_scene_device (device 0): the allocation-range look-up (driver API), an event the context's
+    // stream waits on for the caller's stream, and the word the index check reports its first bad triangle in
+    int (*mem_range)(unsigned long long *, size_t *, unsigned long long) = nullptr;
+    cudaEvent_t ev_mesh_input = nullptr;
+    uint32_t *d_first_bad = nullptr;
 };
 
 namespace
@@ -367,6 +373,75 @@ int check_mesh_args(cuda_trace_ctx *ctx, const float *vertices, uint32_t num_ver
         for (int c = 0; c < 3; c++)
             if (triangles[(size_t) i * 6 + c] >= num_vertices)
                 return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene: vertex index out of bounds");
+    return 0;
+}
+
+// The per-device part of a scene upload, shared by the host and the device entry points: device by device, free the
+// old scene, let `stage(d, i)` put the mesh into d.d_vtx / d.d_tri, build the grid and derive the rest.  Devices are
+// built in order and finish_scene_on_device ends in a synchronisation of the device's stream, so device 0's arrays
+// are complete before device 1 stages.
+template <class Stage>
+int build_scene(cuda_trace_ctx *ctx, uint32_t num_vertices, uint32_t num_triangles, uint32_t grid_res, Stage stage)
+{
+    int rc = 0;
+    ctx->have_scene = false;
+    ctx->num_vtx = num_vertices;
+    ctx->num_tri = num_triangles;
+    for (size_t i = 0; i < ctx->dev.size(); i++)
+    {
+        DeviceState& d = ctx->dev[i];
+        free_scene(d);
+        if ((rc = stage(d, i)))
+            return rc;
+        // Every device builds its own copy of the grid (the build is deterministic and cheaper
+        // than shipping the cell-major records over NVLink would be to code; ~ms)
+        GridBuildResult res;
+        uint64_t launches = 0;
+        std::string err;
+        rc = build_grid_device(d.d_vtx, num_vertices, d.d_tri, num_triangles, grid_res, d.stream, &res, err, &launches);
+        ctx->launches += launches;
+        if (rc)
+            return fail(ctx, rc, err);
+        d.d_cell_start = res.d_cell_start;
+        d.d_tri_index = res.d_tri_index;
+        if (i == 0)
+            ctx->desc = res.desc;
+        else if (std::memcmp(&ctx->desc, &res.desc, sizeof(res.desc)) != 0)
+            return fail(ctx, CUDA_TRACE_ERR_CUDA, "grid build differs between devices");
+        if ((rc = finish_scene_on_device(ctx, d)))
+            return rc;
+    }
+    ctx->have_scene = true;
+    return 0;
+}
+
+// cuda_trace_upload_scene_device's checks of one caller array (`count` 24-byte records), all on the host and before
+// anything is enqueued: 4-byte aligned, device or managed memory of device 0, and inside one allocation
+int check_device_array(cuda_trace_ctx *ctx, const void *p, uint32_t count, const char *name)
+{
+    const int dev0 = ctx->dev[0].ordinal;
+    if ((uintptr_t) p & 3)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, std::string("upload_scene_device: ") + name + " is not 4-byte aligned");
+    cudaPointerAttributes a;
+    const cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess)
+        cudaGetLastError(); // not sticky: clear it so that the next call does not report it
+    if (e != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != dev0)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, std::string("upload_scene_device: ") + name +
+                                                 " is not device memory of the context's device " + std::to_string(dev0));
+    if (!ctx->mem_range)
+        return fail(ctx, CUDA_TRACE_ERR_CUDA, "upload_scene_device: the driver has no cuMemGetAddressRange");
+    unsigned long long base = 0;
+    size_t size = 0;
+    const int r = ctx->mem_range(&base, &size, (unsigned long long) (uintptr_t) p);
+    if (r != 0)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, std::string("upload_scene_device: cuMemGetAddressRange found no "
+                                                         "allocation for ") + name + " (error " + std::to_string(r) + ")");
+    const uint64_t offset = (uint64_t) (uintptr_t) p - base, bytes = (uint64_t) count * 24;
+    if (offset + bytes > size)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, std::string("upload_scene_device: ") + std::to_string(count) + " " + name +
+                                                 " records (" + std::to_string(bytes) + " bytes) run past the end of "
+                                                 "their allocation (" + std::to_string(size - offset) + " bytes left)");
     return 0;
 }
 
@@ -547,6 +622,13 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
             ctx->wait_value32 = reinterpret_cast<int (*)(cudaStream_t, unsigned long long, unsigned int, unsigned int)>(fn);
         else
             cudaGetLastError();
+        // the allocation a device pointer lies in (driver API), for the range check of cuda_trace_upload_scene_device
+        fn = nullptr;
+        if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &fn, cudaEnableDefault, &q) == cudaSuccess &&
+            q == cudaDriverEntryPointSuccess)
+            ctx->mem_range = reinterpret_cast<int (*)(unsigned long long *, size_t *, unsigned long long)>(fn);
+        else
+            cudaGetLastError();
         if (const char *e = std::getenv("RTM_OVERLAP_D2H"))
             ctx->overlap_d2h = std::atoi(e) != 0;
     }
@@ -622,6 +704,8 @@ void cuda_trace_destroy(cuda_trace_ctx *ctx)
             if (ctx->fb_imported) cudaIpcCloseMemHandle(ctx->d_fb); else cudaFree(ctx->d_fb);
         }
         cudaFree(ctx->d_hit_tri); cudaFree(ctx->d_hit_t); cudaFree(ctx->d_hit_u); cudaFree(ctx->d_hit_v);
+        cudaFree(ctx->d_first_bad);
+        if (ctx->ev_mesh_input) cudaEventDestroy(ctx->ev_mesh_input);
     }
     for (DeviceState& d : ctx->dev)
     {
@@ -688,35 +772,69 @@ int cuda_trace_upload_scene(cuda_trace_ctx *ctx, const float *vertices, uint32_t
     if ((rc = cuda_trace_sync(ctx)))
         return rc;
     wait_for_queries(ctx);
-    ctx->have_scene = false;
-    ctx->num_vtx = num_vertices;
-    ctx->num_tri = num_triangles;
-    for (size_t i = 0; i < ctx->dev.size(); i++)
-    {
-        DeviceState& d = ctx->dev[i];
-        free_scene(d);
-        if ((rc = upload_mesh(ctx, d, vertices, num_vertices, triangles, num_triangles)))
-            return rc;
-        // Every device builds its own copy of the grid (the build is deterministic and cheaper
-        // than shipping the cell-major records over NVLink would be to code; ~ms)
-        GridBuildResult res;
-        uint64_t launches = 0;
-        std::string err;
-        rc = build_grid_device(d.d_vtx, num_vertices, d.d_tri, num_triangles, grid_res, d.stream, &res, err, &launches);
-        ctx->launches += launches;
-        if (rc)
-            return fail(ctx, rc, err);
-        d.d_cell_start = res.d_cell_start;
-        d.d_tri_index = res.d_tri_index;
+    return build_scene(ctx, num_vertices, num_triangles, grid_res, [&](DeviceState& d, size_t) {
+        return upload_mesh(ctx, d, vertices, num_vertices, triangles, num_triangles);
+    });
+}
+
+int cuda_trace_upload_scene_device(cuda_trace_ctx *ctx, const float *vertices, uint32_t num_vertices,
+                                   const uint32_t *triangles, uint32_t num_triangles, uint32_t grid_res, void *stream)
+{
+    if (!ctx)
+        return CUDA_TRACE_ERR_ARG;
+    std::lock_guard<std::recursive_mutex> guard(ctx->api_mtx);
+    if (!vertices || !triangles || num_vertices == 0 || num_triangles == 0)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene_device: empty mesh (the reference asserts, grid.cpp:15)");
+    if (grid_res == 0)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene_device: grid_res must be > 0 (grid.cpp:16)");
+    DeviceState& d0 = ctx->dev[0];
+    CK(cudaSetDevice(d0.ordinal));
+    int rc = 0;
+    if ((rc = check_device_array(ctx, vertices, num_vertices, "vertices")) ||
+        (rc = check_device_array(ctx, triangles, num_triangles, "triangles")))
+        return rc;
+    if ((rc = cuda_trace_sync(ctx)))
+        return rc;
+    wait_for_queries(ctx);
+    // The caller's arrays are complete once the work already enqueued on its stream is: the context's stream waits
+    // for that, then checks the vertex indices on the device.  The old scene is freed only after they passed.
+    CK(cudaSetDevice(d0.ordinal));
+    if (!ctx->ev_mesh_input)
+        CK(cudaEventCreateWithFlags(&ctx->ev_mesh_input, cudaEventDisableTiming));
+    if (!ctx->d_first_bad)
+        CK(cudaMalloc(&ctx->d_first_bad, sizeof(uint32_t)));
+    CK(cudaEventRecord(ctx->ev_mesh_input, stream ? (cudaStream_t) stream : d0.stream));
+    CK(cudaStreamWaitEvent(d0.stream, ctx->ev_mesh_input, 0));
+    CK(cudaMemsetAsync(ctx->d_first_bad, 0xFF, sizeof(uint32_t), d0.stream));
+    launch_check_triangle_indices(triangles, num_triangles, num_vertices, ctx->d_first_bad, d0.stream);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    uint32_t first_bad = 0;
+    CK(cudaMemcpyAsync(&first_bad, ctx->d_first_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, d0.stream));
+    CK(cudaStreamSynchronize(d0.stream));
+    if (first_bad != 0xFFFFFFFFu)
+        return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene_device: vertex index out of bounds in triangle " +
+                                                 std::to_string(first_bad) + " (num_vertices " +
+                                                 std::to_string(num_vertices) + ")");
+    const size_t vtx_bytes = (size_t) num_vertices * 24, tri_bytes = (size_t) num_triangles * 24;
+    return build_scene(ctx, num_vertices, num_triangles, grid_res, [&](DeviceState& d, size_t i) {
+        CK(cudaSetDevice(d.ordinal));
+        CK(cudaMalloc(&d.d_vtx, vtx_bytes));
+        CK(cudaMalloc(&d.d_tri, tri_bytes));
         if (i == 0)
-            ctx->desc = res.desc;
-        else if (std::memcmp(&ctx->desc, &res.desc, sizeof(res.desc)) != 0)
-            return fail(ctx, CUDA_TRACE_ERR_CUDA, "grid build differs between devices");
-        if ((rc = finish_scene_on_device(ctx, d)))
-            return rc;
-    }
-    ctx->have_scene = true;
-    return 0;
+        {
+            // ordered after the caller's stream by the event wait above
+            CK(cudaMemcpyAsync(d.d_vtx, vertices, vtx_bytes, cudaMemcpyDeviceToDevice, d.stream));
+            CK(cudaMemcpyAsync(d.d_tri, triangles, tri_bytes, cudaMemcpyDeviceToDevice, d.stream));
+        }
+        else
+        {
+            // device 0's copy is complete: its build synchronised its stream (build_scene)
+            CK(cudaMemcpyPeerAsync(d.d_vtx, d.ordinal, d0.d_vtx, d0.ordinal, vtx_bytes, d.stream));
+            CK(cudaMemcpyPeerAsync(d.d_tri, d.ordinal, d0.d_tri, d0.ordinal, tri_bytes, d.stream));
+        }
+        return 0;
+    });
 }
 
 uint32_t cuda_trace_suggest_grid_res(uint32_t num_triangles)

@@ -375,7 +375,28 @@ __global__ void sum_u32_kernel(const uint32_t *__restrict__ in, uint64_t n, unsi
         atomicAdd(total, s);
 }
 
+// ---- the index check of a mesh given in device memory (the host path checks on the host): the lowest triangle with
+// a vertex index >= num_vtx goes to *first_bad (preset to 0xFFFFFFFF) through atomicMin
+__global__ void check_triangle_indices_kernel(const uint32_t *__restrict__ tri, uint32_t num_tri, uint32_t num_vtx,
+                                              uint32_t *__restrict__ first_bad)
+{
+    for (uint64_t ti = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; ti < num_tri;
+         ti += (uint64_t) gridDim.x * blockDim.x)
+    {
+        const uint32_t *t = tri + ti * 6;
+        if ((t[0] >= num_vtx) | (t[1] >= num_vtx) | (t[2] >= num_vtx))
+            atomicMin(first_bad, (uint32_t) ti);
+    }
+}
+
 } // namespace
+
+void launch_check_triangle_indices(const uint32_t *d_tri, uint32_t num_tri, uint32_t num_vtx, uint32_t *d_first_bad,
+                                   cudaStream_t stream)
+{
+    const unsigned blocks = (unsigned) std::min<uint64_t>(1024, ((uint64_t) num_tri + 255) / 256);
+    check_triangle_indices_kernel<<<std::max(blocks, 1u), 256, 0, stream>>>(d_tri, num_tri, num_vtx, d_first_bad);
+}
 
 int exclusive_scan_u32(const uint32_t *d_in, uint32_t *d_out, uint64_t n, cudaStream_t stream, std::string& err,
                        uint64_t *launches)

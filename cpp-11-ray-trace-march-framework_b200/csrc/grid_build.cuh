@@ -25,6 +25,11 @@ int build_grid_device(const float *d_vtx, uint32_t num_vtx, const uint32_t *d_tr
                       uint32_t grid_res, cudaStream_t stream, GridBuildResult *out, std::string& err,
                       uint64_t *launches);
 
+// Enqueues the vertex-index check of T x 6-word triangle records in device memory: *d_first_bad, which the caller sets
+// to 0xFFFFFFFF first, becomes the lowest triangle with an index >= num_vtx and is left alone when there is none
+void launch_check_triangle_indices(const uint32_t *d_tri, uint32_t num_tri, uint32_t num_vtx, uint32_t *d_first_bad,
+                                   cudaStream_t stream);
+
 // Exclusive prefix sum over n uint32 words (in place allowed); synchronises `stream` when n spans several tiles
 int exclusive_scan_u32(const uint32_t *d_in, uint32_t *d_out, uint64_t n, cudaStream_t stream, std::string& err,
                        uint64_t *launches);

@@ -130,6 +130,27 @@ int cuda_trace_set_shard_signals(cuda_trace_ctx *ctx, int enable);
 int cuda_trace_upload_scene(cuda_trace_ctx *ctx, const float *vertices, uint32_t num_vertices,
                             const uint32_t *triangles, uint32_t num_triangles, uint32_t grid_res);
 
+/* cuda_trace_upload_scene for a mesh that lives on the GPU: the same two 24-byte record arrays (Mesh::m_vertices,
+ * Mesh::m_triangles), in DEVICE (or managed) memory of the context's device 0.  `stream` is the stream the
+ * arrays were produced on (a cudaStream_t of device 0; NULL = cuda_trace_stream(ctx)): the call orders itself
+ * after the work already enqueued there.  Returns once the scene is built, like cuda_trace_upload_scene; the
+ * context keeps its own copies, so the caller may then overwrite or free the arrays.  The result (grid, records,
+ * distance map, every frame and query) is bit-identical to cuda_trace_upload_scene on the same bytes.
+ *
+ * Accepted input is exactly what cuda_trace_upload_scene accepts: a non-empty mesh, grid_res > 0 and every vertex
+ * index < num_vertices.  Nothing else is checked; non-finite coordinates are not rejected.  In this order:
+ *   1. on the host, before anything is enqueued: both pointers 4-byte aligned, device or managed memory of device 0
+ *      (cudaPointerGetAttributes, the rule of cuda_trace_query_rays), and [ptr, ptr + count * 24) inside one
+ *      allocation (cuMemGetAddressRange), so no kernel or copy ever reads past the caller's allocation;
+ *   2. a frame in flight is synced and queries already enqueued are waited for, as on the host path;
+ *   3. on device 0, behind the caller's stream: the vertex indices (one host synchronisation to read the verdict).
+ * A refusal returns CUDA_TRACE_ERR_ARG with a message (for a bad index, naming the lowest offending triangle) and
+ * changes nothing: the previous scene stays in place and usable.  A failing CUDA call returns CUDA_TRACE_ERR_CUDA.
+ * Devices 1..n-1 of the context receive the arrays from device 0's copy (cudaMemcpyPeerAsync). */
+int cuda_trace_upload_scene_device(cuda_trace_ctx *ctx, const float *vertices, uint32_t num_vertices,
+                                   const uint32_t *triangles, uint32_t num_triangles, uint32_t grid_res,
+                                   void *stream);
+
 /* Grid density heuristic for cuda_trace_upload_scene (the reference hard-codes 64 cells on the longest
  * axis, scene.cpp:7): about three cells per triangle, res = cbrt(3 T), while the grid's occupancy map fits in
  * shared memory (res <= 108); about nine, res = cbrt(9 T) <= 896, for the larger grids, which the pooled-ray
