@@ -19,6 +19,7 @@
 #include <tuple>
 #include <vector>
 
+#include "device_array.cuh"
 #include "grid_build.cuh"
 #include "qmc.cuh"
 #include "trace_kernels.cuh"
@@ -29,6 +30,28 @@ namespace
 {
 
 std::string g_init_error;
+
+// A scene's arrays on one device and what describes their contents; replaced whole, by a new scene or by nothing
+struct SceneArrays
+{
+    DeviceArray<float> d_vtx;
+    DeviceArray<uint32_t> d_tri, d_cell_start, d_cell_occ, d_tri_index;
+    DeviceArray<uint32_t> d_pcell_start, d_pcell_occ; // padded grid (rt_device.cuh)
+    DeviceArray<uint8_t> d_pcell_dist;                // its distance map (large grids only)
+    DeviceArray<float4> d_cell_tris, d_cell_tris_b, d_tri_normals;
+    DeviceArray<uint32_t> d_ppair_start; // padded CSR of the pair records (rt_device.cuh)
+    DeviceArray<float4> d_pair_recs;     // two triangles per record, interleaved: the packed-fp32 test of K1
+    DeviceArray<float4> d_pair_recs_rel; // ... relative to rel_origin (primary rays; built on demand, pack.cu)
+    float rel_origin[3] = { 0.0f, 0.0f, 0.0f };
+    bool rel_valid = false;
+    // screen boxes of the pair records (K1's screen cull, pack.cu) for the camera sbox_cam, and the per-scene gate
+    // taken from them: cull only when enough pairs project small (sbox_cull)
+    DeviceArray<float4> d_pair_sbox;
+    DeviceArray<unsigned int> d_sbox_small;
+    CameraDev sbox_cam;
+    uint32_t sbox_small = 0; // boxes of at most kScreenCullSmallPixels pixels for sbox_cam (the gate's count)
+    bool sbox_valid = false, sbox_cull = false;
+};
 
 struct DeviceState
 {
@@ -45,50 +68,29 @@ struct DeviceState
     cudaEvent_t ev_copy = nullptr;
     cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
 
-    // scene
-    float *d_vtx = nullptr;
-    uint32_t *d_tri = nullptr;
-    uint32_t *d_cell_start = nullptr, *d_cell_occ = nullptr, *d_tri_index = nullptr;
-    uint32_t *d_pcell_start = nullptr, *d_pcell_occ = nullptr; // padded grid (rt_device.cuh)
-    uint8_t *d_pcell_dist = nullptr;                           // its distance map (large grids only)
+    SceneArrays scene;
     // K7 trace_pool: per-sample hit records (tri, t, u, v) of this device's strips, read back by K1 <kVariantFromHits>
-    uint32_t *d_pool_tri = nullptr;
-    float *d_pool_t = nullptr, *d_pool_u = nullptr, *d_pool_v = nullptr;
-    uint64_t pool_cap = 0;
+    DeviceArray<uint32_t> d_pool_tri;
+    DeviceArray<float> d_pool_t, d_pool_u, d_pool_v;
     int resolve_blocks_per_sm = 0, resolve_threads = 0;
-    float4 *d_cell_tris = nullptr, *d_cell_tris_b = nullptr, *d_tri_normals = nullptr;
-    uint32_t *d_ppair_start = nullptr;  // padded CSR of the pair records (rt_device.cuh)
-    float4 *d_pair_recs = nullptr;      // two triangles per record, interleaved: the packed-fp32 test of K1
-    float4 *d_pair_recs_rel = nullptr;  // ... relative to rel_origin (primary rays; built on demand, pack.cu)
-    float rel_origin[3] = { 0.0f, 0.0f, 0.0f };
-    bool rel_valid = false;
-    // screen boxes of the pair records (K1's screen cull, pack.cu) for the camera sbox_cam, and the per-scene gate
-    // taken from them: cull only when enough pairs project small (sbox_cull)
-    float4 *d_pair_sbox = nullptr;
-    unsigned int *d_sbox_small = nullptr;
-    CameraDev sbox_cam;
-    uint32_t sbox_small = 0; // boxes of at most kScreenCullSmallPixels pixels for sbox_cam (the gate's count)
-    bool sbox_valid = false, sbox_cull = false;
 
     // frame
-    float2 *d_smp = nullptr;
-    uint32_t smp_cap = 0, smp_valid_spp = 0;
-    uint4 *d_tile_rects = nullptr;
-    uint32_t *d_tile_prefix = nullptr;
-    uint32_t tile_cap = 0;
-    uint32_t *d_strip_counter = nullptr;   // {strip counter, pad to 128 B, this GPU's band piece counts}: one memset per frame
+    DeviceArray<float2> d_smp;
+    uint32_t smp_valid_spp = 0;
+    DeviceArray<uint4> d_tile_rects;
+    DeviceArray<uint32_t> d_tile_prefix;
+    DeviceArray<uint32_t> d_strip_counter; // {strip counter, pad to 128 B, this GPU's band piece counts}: one memset per frame
     uint32_t *d_cancel = nullptr;          // behind them and never cleared: the sequence number of the frame to cancel
-    uint32_t *h_cancel_seen = nullptr;     // page-locked + mapped: the kernel stores its frame number here when it saw the request
+    PinnedArray<uint32_t, cudaHostAllocMapped | cudaHostAllocPortable> h_cancel_seen; // the kernel stores its frame number here when it saw the request
     uint32_t *d_cancel_seen = nullptr;     // device view of h_cancel_seen
     uint32_t launched_seq = 0;             // sequence number of the frame in flight on this device
     uint64_t layout_serial = 0;            // FramePlan the device copies d_tile_rects / d_tile_prefix hold
     std::tuple<TraceTilesKernel, int, size_t> occupancy_key{}; // K1 instance, CTA size, dynamic smem `blocks_per_sm` is for
     int blocks_per_sm = 0;
-    Counters *d_counters = nullptr;
+    DeviceArray<Counters> d_counters;
     // cost-ordered scheduling (schedule.cu): cycles per strip of the last frame -> order of the next
-    uint32_t *d_strip_cycles = nullptr, *d_fetch_order = nullptr, *d_order_scratch = nullptr, *d_visit_total = nullptr, *d_visit_cycles = nullptr;
-    unsigned long long *d_cost_sum = nullptr;
-    uint32_t order_cap = 0;
+    DeviceArray<uint32_t> d_strip_cycles, d_fetch_order, d_order_scratch, d_visit_total, d_visit_cycles;
+    DeviceArray<unsigned long long> d_cost_sum;
     bool order_valid = false;
     std::vector<uint64_t> order_signature; // plan serial + shard the recorded strip costs belong to
     uint32_t order_strips = 0;             // strips of this shard the recorded costs cover
@@ -159,8 +161,9 @@ struct cuda_trace_ctx
     int cost_order_forced = -1; // schedule.cu: -1 automatic, 0 / 1 forced by RTM_COST_ORDER (experiments)
     std::atomic<uint64_t> launches{0};
 
-    // framebuffer (device 0, or an imported IPC mapping of another process' framebuffer)
+    // framebuffer (device 0: fb_own, or an imported IPC mapping of another process' framebuffer)
     uint32_t *d_fb = nullptr;
+    DeviceArray<uint32_t> fb_own;
     bool fb_imported = false;
     uint32_t fb_w = 0, fb_h = 0;
 
@@ -177,17 +180,16 @@ struct cuda_trace_ctx
     // cuda_trace_tiles_into: tiles grouped by the row band that completes them, one event per group
     std::vector<cudaEvent_t> tile_events;
     std::vector<std::vector<uint32_t>> tile_groups;
-    uint32_t *staging = nullptr;  // page-locked W x H image small frames pass through on their way into tile buffers
-    size_t staging_pixels = 0;
+    PinnedArray<uint32_t, cudaHostAllocPortable> staging; // W x H image small frames pass through on their way into tile buffers
     bool overlap_d2h = true;      // RTM_OVERLAP_D2H=0 disables
     bool shard_signals = false;   // cuda_trace_set_shard_signals: other ranks bump the counters too
     int (*wait_value32)(cudaStream_t, unsigned long long, unsigned int, unsigned int) = nullptr;
 
     // per-sample hit records of the last KEEP_HITS frame (device 0)
     unsigned long long mailbox_stats[2] = { 0, 0 }; // last mailbox run of cuda_trace_intersect_rays
-    uint32_t *d_hit_tri = nullptr;
-    float *d_hit_t = nullptr, *d_hit_u = nullptr, *d_hit_v = nullptr;
-    uint64_t hit_cap = 0, hit_count = 0;
+    DeviceArray<uint32_t> d_hit_tri;
+    DeviceArray<float> d_hit_t, d_hit_u, d_hit_v;
+    uint64_t hit_count = 0;
 
     // last frame
     cuda_trace_frame frame;
@@ -199,7 +201,7 @@ struct cuda_trace_ctx
     double t_submitted_ms = 0.0, t_traced_ms = 0.0, t_copied_ms = 0.0, t_return_ms = 0.0;
     double t_prepared_ms = 0.0, t_launching_ms = 0.0, t_launched_ms = 0.0; // submission in detail: host set-up done, first device's kernel about to be / has been launched
     bool marks_armed = false;
-    uint32_t *pinned_cancel_src = nullptr;
+    PinnedArray<uint32_t> pinned_cancel_src;
 
     // cuda_trace_query_rays: per stream the context has been given, an event behind its last query (device 0).
     // Replacing the scene or destroying the context waits for them before the scene arrays are freed.
@@ -209,7 +211,7 @@ struct cuda_trace_ctx
     // stream waits on for the caller's stream, and the word the index check reports its first bad triangle in
     int (*mem_range)(unsigned long long *, size_t *, unsigned long long) = nullptr;
     cudaEvent_t ev_mesh_input = nullptr;
-    uint32_t *d_first_bad = nullptr;
+    DeviceArray<uint32_t> d_first_bad;
 };
 
 namespace
@@ -231,23 +233,6 @@ int fail(cuda_trace_ctx *ctx, int code, const std::string& msg)
             return fail(ctx, CUDA_TRACE_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
     } while (0)
 
-void free_scene(DeviceState& d)
-{
-    cudaSetDevice(d.ordinal);
-    cudaFree(d.d_vtx); cudaFree(d.d_tri); cudaFree(d.d_cell_start); cudaFree(d.d_cell_occ);
-    cudaFree(d.d_tri_index); cudaFree(d.d_cell_tris); cudaFree(d.d_cell_tris_b); cudaFree(d.d_tri_normals);
-    cudaFree(d.d_ppair_start); cudaFree(d.d_pair_recs); cudaFree(d.d_pair_recs_rel);
-    d.d_ppair_start = nullptr; d.d_pair_recs = nullptr; d.d_pair_recs_rel = nullptr;
-    d.rel_valid = false;
-    cudaFree(d.d_pair_sbox); cudaFree(d.d_sbox_small);
-    d.d_pair_sbox = nullptr; d.d_sbox_small = nullptr;
-    d.sbox_valid = false;
-    cudaFree(d.d_pcell_start); cudaFree(d.d_pcell_occ); cudaFree(d.d_pcell_dist);
-    d.d_pcell_start = nullptr; d.d_pcell_occ = nullptr; d.d_pcell_dist = nullptr;
-    d.d_vtx = nullptr; d.d_tri = nullptr; d.d_cell_start = nullptr; d.d_cell_occ = nullptr;
-    d.d_tri_index = nullptr; d.d_cell_tris = nullptr; d.d_cell_tris_b = nullptr; d.d_tri_normals = nullptr;
-}
-
 // Queries still running on their callers' streams read the scene arrays: wait for them before those are freed
 void wait_for_queries(cuda_trace_ctx *ctx)
 {
@@ -260,6 +245,7 @@ void wait_for_queries(cuda_trace_ctx *ctx)
 
 GridDev grid_dev(const cuda_trace_ctx *ctx, const DeviceState& d)
 {
+    const SceneArrays& s = d.scene;
     GridDev g;
     for (int k = 0; k < 3; k++)
     {
@@ -269,18 +255,18 @@ GridDev grid_dev(const cuda_trace_ctx *ctx, const DeviceState& d)
     }
     g.cell_wdh = ctx->desc.cell_wdh;
     g.inv_cell_wdh = ctx->desc.inv_cell_wdh;
-    g.cell_start = d.d_cell_start;
-    g.cell_occ = d.d_cell_occ;
-    g.pcell_start = d.d_pcell_start;
-    g.pcell_occ = d.d_pcell_occ;
-    g.pcell_dist = d.d_pcell_dist;
-    g.cell_tris = d.d_cell_tris;
-    g.cell_tris_b = d.d_cell_tris_b;
-    g.ppair_start = d.d_ppair_start;
-    g.pair_recs = d.d_pair_recs;
-    g.pair_recs_rel = d.d_pair_recs_rel;
-    g.tri_normals = d.d_tri_normals;
-    g.tri = d.d_tri;
+    g.cell_start = s.d_cell_start.get();
+    g.cell_occ = s.d_cell_occ.get();
+    g.pcell_start = s.d_pcell_start.get();
+    g.pcell_occ = s.d_pcell_occ.get();
+    g.pcell_dist = s.d_pcell_dist.get();
+    g.cell_tris = s.d_cell_tris.get();
+    g.cell_tris_b = s.d_cell_tris_b.get();
+    g.ppair_start = s.d_ppair_start.get();
+    g.pair_recs = s.d_pair_recs.get();
+    g.pair_recs_rel = s.d_pair_recs_rel.get();
+    g.tri_normals = s.d_tri_normals.get();
+    g.tri = s.d_tri.get();
     return g;
 }
 
@@ -291,46 +277,47 @@ inline uint64_t occupancy_bits_bytes(uint64_t pcells) { return (pcells + 31) / 3
 // After d_vtx / d_tri / d_cell_start / d_tri_index are in place on device d: derived layout
 int finish_scene_on_device(cuda_trace_ctx *ctx, DeviceState& d)
 {
+    SceneArrays& s = d.scene;
     const uint64_t cells = ctx->desc.num_cells, refs = ctx->desc.num_refs;
     const uint64_t pcells = (uint64_t) (ctx->desc.dim[0] + 2) * (ctx->desc.dim[1] + 2) * (ctx->desc.dim[2] + 2);
     if (pcells >= (1ull << 31))
         return fail(ctx, CUDA_TRACE_ERR_ARG, "grid too large: padded cell count must stay below 2^31");
     if (refs * 3 >= (1ull << 32))
         return fail(ctx, CUDA_TRACE_ERR_ARG, "grid too large: 3 x cell references must stay below 2^32");
-    CK(cudaMalloc(&d.d_cell_occ, ((cells + 31) / 32) * sizeof(uint32_t)));
-    CK(cudaMalloc(&d.d_pcell_start, (pcells + 1) * sizeof(uint32_t)));
-    CK(cudaMalloc(&d.d_pcell_occ, ((pcells + 31) / 32) * sizeof(uint32_t)));
-    CK(cudaMalloc(&d.d_cell_tris, std::max<uint64_t>(refs, 1) * 3 * sizeof(float4)));
-    CK(cudaMalloc(&d.d_cell_tris_b, std::max<uint64_t>(refs, 1) * 2 * sizeof(float4)));
-    CK(cudaMalloc(&d.d_tri_normals, (size_t) ctx->num_tri * 3 * sizeof(float4)));
-    launch_cell_occupancy(d.d_cell_start, cells, d.d_cell_occ, d.stream);
-    launch_pad_grid(d.d_cell_start, ctx->desc.dim, d.d_pcell_start, d.d_pcell_occ, d.stream);
+    CK(s.d_cell_occ.alloc((cells + 31) / 32));
+    CK(s.d_pcell_start.alloc(pcells + 1));
+    CK(s.d_pcell_occ.alloc((pcells + 31) / 32));
+    CK(s.d_cell_tris.alloc(std::max<uint64_t>(refs, 1) * 3));
+    CK(s.d_cell_tris_b.alloc(std::max<uint64_t>(refs, 1) * 2));
+    CK(s.d_tri_normals.alloc((size_t) ctx->num_tri * 3));
+    launch_cell_occupancy(s.d_cell_start.get(), cells, s.d_cell_occ.get(), d.stream);
+    launch_pad_grid(s.d_cell_start.get(), ctx->desc.dim, s.d_pcell_start.get(), s.d_pcell_occ.get(), d.stream);
     ctx->launches += 2;
     // grids whose occupancy bits do not fit in shared memory (choose_cta) get the distance map as a second level
     if (occupancy_bits_bytes(pcells) > kOccSmemBudget || ctx->tune.occ_mode == kOccGlobalDist || ctx->tune.pool == 1)
     {
-        CK(cudaMalloc(&d.d_pcell_dist, pcells));
-        launch_distance_map(d.d_pcell_occ, ctx->desc.dim, d.d_pcell_dist, d.stream);
+        CK(s.d_pcell_dist.alloc(pcells));
+        launch_distance_map(s.d_pcell_occ.get(), ctx->desc.dim, s.d_pcell_dist.get(), d.stream);
         ctx->launches += 3;
     }
-    launch_pack_cell_tris(d.d_vtx, d.d_tri, d.d_tri_index, refs, d.d_cell_tris, d.d_cell_tris_b, d.stream);
-    launch_pack_normals(d.d_vtx, d.d_tri, ctx->num_tri, d.d_tri_normals, d.stream);
+    launch_pack_cell_tris(s.d_vtx.get(), s.d_tri.get(), s.d_tri_index.get(), refs, s.d_cell_tris.get(), s.d_cell_tris_b.get(), d.stream);
+    launch_pack_normals(s.d_vtx.get(), s.d_tri.get(), ctx->num_tri, s.d_tri_normals.get(), d.stream);
     ctx->launches += 2 + (refs ? 1 : 0);
     CK(cudaGetLastError());
     // pair records: count per padded cell -> exclusive scan -> pack
-    CK(cudaMalloc(&d.d_ppair_start, (pcells + 1) * sizeof(uint32_t)));
-    launch_pair_counts(d.d_pcell_start, pcells, d.d_ppair_start, d.stream);
+    CK(s.d_ppair_start.alloc(pcells + 1));
+    launch_pair_counts(s.d_pcell_start.get(), pcells, s.d_ppair_start.get(), d.stream);
     ctx->launches++;
     {
         std::string err;
         uint64_t launches = 0;
-        const int rc = exclusive_scan_u32(d.d_ppair_start, d.d_ppair_start, pcells + 1, d.stream, err, &launches);
+        const int rc = exclusive_scan_u32(s.d_ppair_start.get(), s.d_ppair_start.get(), pcells + 1, d.stream, err, &launches);
         ctx->launches += launches;
         if (rc)
             return fail(ctx, rc, err);
     }
     uint32_t pairs = 0;
-    CK(cudaMemcpyAsync(&pairs, d.d_ppair_start + pcells, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
+    CK(cudaMemcpyAsync(&pairs, s.d_ppair_start.get() + pcells, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
     CK(cudaStreamSynchronize(d.stream));
     if ((uint64_t) pairs * 7 >= (1ull << 32))
         return fail(ctx, CUDA_TRACE_ERR_ARG, "grid too large: 7 x pair records must stay below 2^32");
@@ -338,14 +325,14 @@ int finish_scene_on_device(cuda_trace_ctx *ctx, DeviceState& d)
         ctx->num_pairs = pairs;
     else if (ctx->num_pairs != pairs)
         return fail(ctx, CUDA_TRACE_ERR_CUDA, "pair records differ between devices");
-    CK(cudaMalloc(&d.d_pair_recs, std::max<uint64_t>(pairs, 1) * 5 * sizeof(float4)));
+    CK(s.d_pair_recs.alloc(std::max<uint64_t>(pairs, 1) * 5));
     if (pairs)
     {
-        launch_pack_pairs(d.d_pcell_start, d.d_ppair_start, pcells, d.d_cell_tris, d.d_pair_recs, d.stream);
+        launch_pack_pairs(s.d_pcell_start.get(), s.d_ppair_start.get(), pcells, s.d_cell_tris.get(), s.d_pair_recs.get(), d.stream);
         ctx->launches++;
     }
     else
-        CK(cudaMemsetAsync(d.d_pair_recs, 0, 5 * sizeof(float4), d.stream));
+        CK(cudaMemsetAsync(s.d_pair_recs.get(), 0, 5 * sizeof(float4), d.stream));
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(d.stream));
     return 0;
@@ -355,10 +342,10 @@ int upload_mesh(cuda_trace_ctx *ctx, DeviceState& d, const float *vertices, uint
                 const uint32_t *triangles, uint32_t num_triangles)
 {
     CK(cudaSetDevice(d.ordinal));
-    CK(cudaMalloc(&d.d_vtx, (size_t) num_vertices * 24));
-    CK(cudaMalloc(&d.d_tri, (size_t) num_triangles * 24));
-    CK(cudaMemcpyAsync(d.d_vtx, vertices, (size_t) num_vertices * 24, cudaMemcpyHostToDevice, d.stream));
-    CK(cudaMemcpyAsync(d.d_tri, triangles, (size_t) num_triangles * 24, cudaMemcpyHostToDevice, d.stream));
+    CK(d.scene.d_vtx.alloc((size_t) num_vertices * 6));
+    CK(d.scene.d_tri.alloc((size_t) num_triangles * 6));
+    CK(cudaMemcpyAsync(d.scene.d_vtx.get(), vertices, (size_t) num_vertices * 24, cudaMemcpyHostToDevice, d.stream));
+    CK(cudaMemcpyAsync(d.scene.d_tri.get(), triangles, (size_t) num_triangles * 24, cudaMemcpyHostToDevice, d.stream));
     return 0;
 }
 
@@ -376,12 +363,32 @@ int check_mesh_args(cuda_trace_ctx *ctx, const float *vertices, uint32_t num_ver
     return 0;
 }
 
-// The per-device part of a scene upload, shared by the host and the device entry points: device by device, free the
-// old scene, let `stage(d, i)` put the mesh into d.d_vtx / d.d_tri, build the grid and derive the rest.  Devices are
-// built in order and finish_scene_on_device ends in a synchronisation of the device's stream, so device 0's arrays
-// are complete before device 1 stages.
+// The grid of the mesh staged on device d, the context's i-th.  Every device builds its own copy of the grid (the build
+// is deterministic and cheaper than shipping the cell-major records over NVLink would be to code; ~ms)
+int build_grid(cuda_trace_ctx *ctx, DeviceState& d, size_t i, uint32_t grid_res)
+{
+    GridBuildResult res;
+    uint64_t launches = 0;
+    std::string err;
+    const int rc = build_grid_device(d.scene.d_vtx.get(), ctx->num_vtx, d.scene.d_tri.get(), ctx->num_tri, grid_res, d.stream, &res, err, &launches);
+    ctx->launches += launches;
+    if (rc)
+        return fail(ctx, rc, err);
+    d.scene.d_cell_start = std::move(res.d_cell_start);
+    d.scene.d_tri_index = std::move(res.d_tri_index);
+    if (i == 0)
+        ctx->desc = res.desc;
+    else if (std::memcmp(&ctx->desc, &res.desc, sizeof(res.desc)) != 0)
+        return fail(ctx, CUDA_TRACE_ERR_CUDA, "grid build differs between devices");
+    return 0;
+}
+
+// The per-device part of a scene upload, shared by the entry points: device by device, free the old scene, let
+// `stage(d, i)` put the mesh into d.scene.d_vtx / d_tri and the grid into d_cell_start / d_tri_index (and ctx->desc),
+// and derive the rest.  Devices are built in order and finish_scene_on_device ends in a synchronisation of the device's
+// stream, so device 0's arrays are complete before device 1 stages.  An upload that fails leaves no scene.
 template <class Stage>
-int build_scene(cuda_trace_ctx *ctx, uint32_t num_vertices, uint32_t num_triangles, uint32_t grid_res, Stage stage)
+int build_scene(cuda_trace_ctx *ctx, uint32_t num_vertices, uint32_t num_triangles, Stage stage)
 {
     int rc = 0;
     ctx->have_scene = false;
@@ -390,26 +397,16 @@ int build_scene(cuda_trace_ctx *ctx, uint32_t num_vertices, uint32_t num_triangl
     for (size_t i = 0; i < ctx->dev.size(); i++)
     {
         DeviceState& d = ctx->dev[i];
-        free_scene(d);
-        if ((rc = stage(d, i)))
+        d.scene = SceneArrays();
+        if ((rc = stage(d, i)) || (rc = finish_scene_on_device(ctx, d)))
+        {
+            for (DeviceState& e : ctx->dev) // released once the work enqueued on them is done
+            {
+                cudaStreamSynchronize(e.stream);
+                e.scene = SceneArrays();
+            }
             return rc;
-        // Every device builds its own copy of the grid (the build is deterministic and cheaper
-        // than shipping the cell-major records over NVLink would be to code; ~ms)
-        GridBuildResult res;
-        uint64_t launches = 0;
-        std::string err;
-        rc = build_grid_device(d.d_vtx, num_vertices, d.d_tri, num_triangles, grid_res, d.stream, &res, err, &launches);
-        ctx->launches += launches;
-        if (rc)
-            return fail(ctx, rc, err);
-        d.d_cell_start = res.d_cell_start;
-        d.d_tri_index = res.d_tri_index;
-        if (i == 0)
-            ctx->desc = res.desc;
-        else if (std::memcmp(&ctx->desc, &res.desc, sizeof(res.desc)) != 0)
-            return fail(ctx, CUDA_TRACE_ERR_CUDA, "grid build differs between devices");
-        if ((rc = finish_scene_on_device(ctx, d)))
-            return rc;
+        }
     }
     ctx->have_scene = true;
     return 0;
@@ -455,10 +452,9 @@ int ensure_framebuffer(cuda_trace_ctx *ctx, uint32_t w, uint32_t h)
     if (ctx->fb_imported)
         return fail(ctx, CUDA_TRACE_ERR_ARG, "frame size differs from the imported framebuffer");
     CK(cudaSetDevice(ctx->dev[0].ordinal));
-    if (ctx->d_fb)
-        CK(cudaFree(ctx->d_fb));
     ctx->d_fb = nullptr;
-    CK(cudaMalloc(&ctx->d_fb, fb_alloc_bytes(w, h)));
+    CK(ctx->fb_own.alloc(fb_alloc_bytes(w, h) / sizeof(uint32_t)));
+    ctx->d_fb = ctx->fb_own.get();
     CK(cudaMemsetAsync(ctx->d_fb, 0, fb_alloc_bytes(w, h), ctx->dev[0].stream));
     CK(cudaStreamSynchronize(ctx->dev[0].stream)); // the zeroed band counters are in place before any stream waits on them
     ctx->fb_w = w;
@@ -586,15 +582,15 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
             (e = cudaEventCreateWithFlags(&d.ev_order, cudaEventDisableTiming)) != cudaSuccess ||
             (e = cudaEventCreateWithFlags(&d.ev_copy, cudaEventDisableTiming)) != cudaSuccess ||
             (e = cudaEventCreate(&d.ev_begin)) != cudaSuccess || (e = cudaEventCreate(&d.ev_end)) != cudaSuccess ||
-            (e = cudaMalloc(&d.d_strip_counter, (32 + kMaxBands + 32) * sizeof(uint32_t))) != cudaSuccess || // {strip counter, pad to 128 B | band piece counts | cancel word}
-            (e = cudaHostAlloc(&d.h_cancel_seen, sizeof(uint32_t), cudaHostAllocMapped | cudaHostAllocPortable)) != cudaSuccess ||
-            (e = cudaHostGetDevicePointer((void **) &d.d_cancel_seen, d.h_cancel_seen, 0)) != cudaSuccess ||
-            (e = cudaMalloc(&d.d_counters, sizeof(Counters))) != cudaSuccess ||
-            (e = cudaMemset(d.d_strip_counter, 0, (32 + kMaxBands + 32) * sizeof(uint32_t))) != cudaSuccess ||
-            (e = cudaMemset(d.d_counters, 0, sizeof(Counters))) != cudaSuccess)
+            (e = d.d_strip_counter.alloc(32 + kMaxBands + 32)) != cudaSuccess || // {strip counter, pad to 128 B | band piece counts | cancel word}
+            (e = d.h_cancel_seen.alloc(1)) != cudaSuccess ||
+            (e = cudaHostGetDevicePointer((void **) &d.d_cancel_seen, d.h_cancel_seen.get(), 0)) != cudaSuccess ||
+            (e = d.d_counters.alloc(1)) != cudaSuccess ||
+            (e = cudaMemset(d.d_strip_counter.get(), 0, (32 + kMaxBands + 32) * sizeof(uint32_t))) != cudaSuccess ||
+            (e = cudaMemset(d.d_counters.get(), 0, sizeof(Counters))) != cudaSuccess)
             return bail(std::string("device set-up: ") + cudaGetErrorString(e), CUDA_TRACE_ERR_CUDA);
-        d.d_cancel = d.d_strip_counter + 32 + kMaxBands; // outside the per-frame memset
-        *d.h_cancel_seen = 0;
+        d.d_cancel = d.d_strip_counter.get() + 32 + kMaxBands; // outside the per-frame memset
+        *d.h_cancel_seen.get() = 0;
         if (i > 0)
         {
             // strips rendered on device i are stored straight into device 0's framebuffer
@@ -610,9 +606,9 @@ int cuda_trace_init_devices(const int *device_ordinals, int n, cuda_trace_ctx **
                 return bail(std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(e), CUDA_TRACE_ERR_CUDA);
         }
     }
-    if ((e = cudaHostAlloc(&ctx->pinned_cancel_src, sizeof(uint32_t), cudaHostAllocDefault)) != cudaSuccess)
+    if ((e = ctx->pinned_cancel_src.alloc(1)) != cudaSuccess)
         return bail(std::string("cudaHostAlloc: ") + cudaGetErrorString(e), CUDA_TRACE_ERR_CUDA);
-    *ctx->pinned_cancel_src = 0;
+    *ctx->pinned_cancel_src.get() = 0;
     {
         // stream-ordered "wait until *addr >= value" (driver API), used by the overlapped read-back
         void *fn = nullptr;
@@ -699,22 +695,13 @@ void cuda_trace_destroy(cuda_trace_ctx *ctx)
     if (!ctx->dev.empty())
     {
         cudaSetDevice(ctx->dev[0].ordinal);
-        if (ctx->d_fb)
-        {
-            if (ctx->fb_imported) cudaIpcCloseMemHandle(ctx->d_fb); else cudaFree(ctx->d_fb);
-        }
-        cudaFree(ctx->d_hit_tri); cudaFree(ctx->d_hit_t); cudaFree(ctx->d_hit_u); cudaFree(ctx->d_hit_v);
-        cudaFree(ctx->d_first_bad);
+        if (ctx->fb_imported && ctx->d_fb)
+            cudaIpcCloseMemHandle(ctx->d_fb);
         if (ctx->ev_mesh_input) cudaEventDestroy(ctx->ev_mesh_input);
     }
     for (DeviceState& d : ctx->dev)
     {
-        free_scene(d);
-        cudaFree(d.d_smp); cudaFree(d.d_tile_rects); cudaFree(d.d_tile_prefix); cudaFree(d.d_strip_counter);
-        cudaFree(d.d_pool_tri); cudaFree(d.d_pool_t); cudaFree(d.d_pool_u); cudaFree(d.d_pool_v);
-        cudaFreeHost(d.h_cancel_seen); cudaFree(d.d_counters);
-        cudaFree(d.d_strip_cycles); cudaFree(d.d_fetch_order); cudaFree(d.d_cost_sum); cudaFree(d.d_order_scratch);
-        cudaFree(d.d_visit_total); cudaFree(d.d_visit_cycles);
+        cudaSetDevice(d.ordinal);
         if (d.ev_begin) cudaEventDestroy(d.ev_begin);
         if (d.ev_end) cudaEventDestroy(d.ev_end);
         if (d.stream) cudaStreamDestroy(d.stream);
@@ -727,11 +714,7 @@ void cuda_trace_destroy(cuda_trace_ctx *ctx)
     }
     for (cudaEvent_t ev : ctx->tile_events)
         cudaEventDestroy(ev);
-    if (ctx->staging)
-        cudaFreeHost(ctx->staging);
-    if (ctx->pinned_cancel_src)
-        cudaFreeHost(ctx->pinned_cancel_src);
-    delete ctx;
+    delete ctx; // and with it every array it owns
 }
 
 const char *cuda_trace_last_error(const cuda_trace_ctx *ctx) { return ctx ? ctx->err.c_str() : g_init_error.c_str(); }
@@ -772,8 +755,9 @@ int cuda_trace_upload_scene(cuda_trace_ctx *ctx, const float *vertices, uint32_t
     if ((rc = cuda_trace_sync(ctx)))
         return rc;
     wait_for_queries(ctx);
-    return build_scene(ctx, num_vertices, num_triangles, grid_res, [&](DeviceState& d, size_t) {
-        return upload_mesh(ctx, d, vertices, num_vertices, triangles, num_triangles);
+    return build_scene(ctx, num_vertices, num_triangles, [&](DeviceState& d, size_t i) {
+        const int rc = upload_mesh(ctx, d, vertices, num_vertices, triangles, num_triangles);
+        return rc ? rc : build_grid(ctx, d, i, grid_res);
     });
 }
 
@@ -801,39 +785,39 @@ int cuda_trace_upload_scene_device(cuda_trace_ctx *ctx, const float *vertices, u
     CK(cudaSetDevice(d0.ordinal));
     if (!ctx->ev_mesh_input)
         CK(cudaEventCreateWithFlags(&ctx->ev_mesh_input, cudaEventDisableTiming));
-    if (!ctx->d_first_bad)
-        CK(cudaMalloc(&ctx->d_first_bad, sizeof(uint32_t)));
+    CK(ctx->d_first_bad.grow(1));
     CK(cudaEventRecord(ctx->ev_mesh_input, stream ? (cudaStream_t) stream : d0.stream));
     CK(cudaStreamWaitEvent(d0.stream, ctx->ev_mesh_input, 0));
-    CK(cudaMemsetAsync(ctx->d_first_bad, 0xFF, sizeof(uint32_t), d0.stream));
-    launch_check_triangle_indices(triangles, num_triangles, num_vertices, ctx->d_first_bad, d0.stream);
+    CK(cudaMemsetAsync(ctx->d_first_bad.get(), 0xFF, sizeof(uint32_t), d0.stream));
+    launch_check_triangle_indices(triangles, num_triangles, num_vertices, ctx->d_first_bad.get(), d0.stream);
     ctx->launches++;
     CK(cudaGetLastError());
     uint32_t first_bad = 0;
-    CK(cudaMemcpyAsync(&first_bad, ctx->d_first_bad, sizeof(uint32_t), cudaMemcpyDeviceToHost, d0.stream));
+    CK(cudaMemcpyAsync(&first_bad, ctx->d_first_bad.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, d0.stream));
     CK(cudaStreamSynchronize(d0.stream));
     if (first_bad != 0xFFFFFFFFu)
         return fail(ctx, CUDA_TRACE_ERR_ARG, "upload_scene_device: vertex index out of bounds in triangle " +
                                                  std::to_string(first_bad) + " (num_vertices " +
                                                  std::to_string(num_vertices) + ")");
     const size_t vtx_bytes = (size_t) num_vertices * 24, tri_bytes = (size_t) num_triangles * 24;
-    return build_scene(ctx, num_vertices, num_triangles, grid_res, [&](DeviceState& d, size_t i) {
+    return build_scene(ctx, num_vertices, num_triangles, [&](DeviceState& d, size_t i) {
+        SceneArrays& s = d.scene;
         CK(cudaSetDevice(d.ordinal));
-        CK(cudaMalloc(&d.d_vtx, vtx_bytes));
-        CK(cudaMalloc(&d.d_tri, tri_bytes));
+        CK(s.d_vtx.alloc((size_t) num_vertices * 6));
+        CK(s.d_tri.alloc((size_t) num_triangles * 6));
         if (i == 0)
         {
             // ordered after the caller's stream by the event wait above
-            CK(cudaMemcpyAsync(d.d_vtx, vertices, vtx_bytes, cudaMemcpyDeviceToDevice, d.stream));
-            CK(cudaMemcpyAsync(d.d_tri, triangles, tri_bytes, cudaMemcpyDeviceToDevice, d.stream));
+            CK(cudaMemcpyAsync(s.d_vtx.get(), vertices, vtx_bytes, cudaMemcpyDeviceToDevice, d.stream));
+            CK(cudaMemcpyAsync(s.d_tri.get(), triangles, tri_bytes, cudaMemcpyDeviceToDevice, d.stream));
         }
         else
         {
             // device 0's copy is complete: its build synchronised its stream (build_scene)
-            CK(cudaMemcpyPeerAsync(d.d_vtx, d.ordinal, d0.d_vtx, d0.ordinal, vtx_bytes, d.stream));
-            CK(cudaMemcpyPeerAsync(d.d_tri, d.ordinal, d0.d_tri, d0.ordinal, tri_bytes, d.stream));
+            CK(cudaMemcpyPeerAsync(s.d_vtx.get(), d.ordinal, d0.scene.d_vtx.get(), d0.ordinal, vtx_bytes, d.stream));
+            CK(cudaMemcpyPeerAsync(s.d_tri.get(), d.ordinal, d0.scene.d_tri.get(), d0.ordinal, tri_bytes, d.stream));
         }
-        return 0;
+        return build_grid(ctx, d, i, grid_res);
     });
 }
 
@@ -872,32 +856,25 @@ int cuda_trace_upload_scene_with_grid(cuda_trace_ctx *ctx, const float *vertices
     if ((rc = cuda_trace_sync(ctx)))
         return rc;
     wait_for_queries(ctx);
-    ctx->have_scene = false;
-    ctx->num_vtx = num_vertices;
-    ctx->num_tri = num_triangles;
     ctx->desc = *desc;
-    for (DeviceState& d : ctx->dev)
-    {
-        free_scene(d);
-        if ((rc = upload_mesh(ctx, d, vertices, num_vertices, triangles, num_triangles)))
+    return build_scene(ctx, num_vertices, num_triangles, [&](DeviceState& d, size_t) {
+        const int rc = upload_mesh(ctx, d, vertices, num_vertices, triangles, num_triangles);
+        if (rc)
             return rc;
-        uint64_t *d_off64 = nullptr;
-        CK(cudaMalloc(&d_off64, (cells + 1) * sizeof(uint64_t)));
-        CK(cudaMalloc(&d.d_cell_start, (cells + 1) * sizeof(uint32_t)));
-        CK(cudaMalloc(&d.d_tri_index, std::max<uint64_t>(desc->num_refs, 1) * sizeof(uint32_t)));
-        CK(cudaMemcpyAsync(d_off64, cell_offset, (cells + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.stream));
+        DeviceArray<uint64_t> d_off64;
+        StreamDrain drain(d.stream);
+        CK(d_off64.alloc(cells + 1));
+        CK(d.scene.d_cell_start.alloc(cells + 1));
+        CK(d.scene.d_tri_index.alloc(std::max<uint64_t>(desc->num_refs, 1)));
+        CK(cudaMemcpyAsync(d_off64.get(), cell_offset, (cells + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.stream));
         if (desc->num_refs)
-            CK(cudaMemcpyAsync(d.d_tri_index, tri_index, desc->num_refs * sizeof(uint32_t), cudaMemcpyHostToDevice,
+            CK(cudaMemcpyAsync(d.scene.d_tri_index.get(), tri_index, desc->num_refs * sizeof(uint32_t), cudaMemcpyHostToDevice,
                                d.stream));
-        launch_narrow_offsets(d_off64, cells + 1, d.d_cell_start, d.stream);
+        launch_narrow_offsets(d_off64.get(), cells + 1, d.scene.d_cell_start.get(), d.stream);
         ctx->launches++;
-        CK(cudaStreamSynchronize(d.stream));
-        CK(cudaFree(d_off64));
-        if ((rc = finish_scene_on_device(ctx, d)))
-            return rc;
-    }
-    ctx->have_scene = true;
-    return 0;
+        CK(drain.sync());
+        return 0;
+    });
 }
 
 int cuda_trace_download_grid(cuda_trace_ctx *ctx, cuda_trace_grid_desc *desc, uint64_t *cell_offset,
@@ -913,18 +890,18 @@ int cuda_trace_download_grid(cuda_trace_ctx *ctx, cuda_trace_grid_desc *desc, ui
     CK(cudaSetDevice(d.ordinal));
     if (cell_offset)
     {
-        uint64_t *d_off64 = nullptr;
-        CK(cudaMalloc(&d_off64, (ctx->desc.num_cells + 1) * sizeof(uint64_t)));
-        launch_widen_offsets(d.d_cell_start, ctx->desc.num_cells + 1, d_off64, d.stream);
+        DeviceArray<uint64_t> d_off64;
+        StreamDrain drain(d.stream);
+        CK(d_off64.alloc(ctx->desc.num_cells + 1));
+        launch_widen_offsets(d.scene.d_cell_start.get(), ctx->desc.num_cells + 1, d_off64.get(), d.stream);
         ctx->launches++;
-        CK(cudaMemcpyAsync(cell_offset, d_off64, (ctx->desc.num_cells + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost,
+        CK(cudaMemcpyAsync(cell_offset, d_off64.get(), (ctx->desc.num_cells + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost,
                            d.stream));
-        CK(cudaStreamSynchronize(d.stream));
-        CK(cudaFree(d_off64));
+        CK(drain.sync());
     }
     if (tri_index && ctx->desc.num_refs)
     {
-        CK(cudaMemcpyAsync(tri_index, d.d_tri_index, ctx->desc.num_refs * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+        CK(cudaMemcpyAsync(tri_index, d.scene.d_tri_index.get(), ctx->desc.num_refs * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                            d.stream));
         CK(cudaStreamSynchronize(d.stream));
     }
@@ -940,11 +917,11 @@ int cuda_trace_download_distance_map(cuda_trace_ctx *ctx, uint8_t *out, uint64_t
         return fail(ctx, CUDA_TRACE_ERR_NO_SCENE, "download_distance_map: no scene uploaded");
     DeviceState& d = ctx->dev[0];
     const uint64_t pcells = (uint64_t) (ctx->desc.dim[0] + 2) * (ctx->desc.dim[1] + 2) * (ctx->desc.dim[2] + 2);
-    *num_bytes = d.d_pcell_dist ? pcells : 0;
-    if (out && d.d_pcell_dist)
+    *num_bytes = d.scene.d_pcell_dist.get() ? pcells : 0;
+    if (out && d.scene.d_pcell_dist.get())
     {
         CK(cudaSetDevice(d.ordinal));
-        CK(cudaMemcpyAsync(out, d.d_pcell_dist, pcells, cudaMemcpyDeviceToHost, d.stream));
+        CK(cudaMemcpyAsync(out, d.scene.d_pcell_dist.get(), pcells, cudaMemcpyDeviceToHost, d.stream));
         CK(cudaStreamSynchronize(d.stream));
     }
     return 0;
@@ -959,18 +936,18 @@ int cuda_trace_download_screen_boxes(cuda_trace_ctx *ctx, float *boxes, uint64_t
     *num_pairs = 0;
     *small = 0;
     *cull_on = 0;
-    if (!ctx->have_scene || ctx->dev.empty() || !ctx->dev[0].sbox_valid)
+    if (!ctx->have_scene || ctx->dev.empty() || !ctx->dev[0].scene.sbox_valid)
         return 0;
     // read only: the boxes, their camera and the gate stay as the last frame left them
     DeviceState& d = ctx->dev[0];
     *num_pairs = ctx->num_pairs;
-    *small = d.sbox_small;
-    *cull_on = d.sbox_cull ? 1 : 0;
+    *small = d.scene.sbox_small;
+    *cull_on = d.scene.sbox_cull ? 1 : 0;
     const uint64_t n = std::min<uint64_t>(*num_pairs, capacity / 4);
     if (n)
     {
         CK(cudaSetDevice(d.ordinal));
-        CK(cudaMemcpyAsync(boxes, d.d_pair_sbox, n * sizeof(float4), cudaMemcpyDeviceToHost, d.stream));
+        CK(cudaMemcpyAsync(boxes, d.scene.d_pair_sbox.get(), n * sizeof(float4), cudaMemcpyDeviceToHost, d.stream));
         CK(cudaStreamSynchronize(d.stream));
     }
     return 0;
@@ -1013,11 +990,10 @@ int cuda_trace_import_framebuffer(cuda_trace_ctx *ctx, const void *handle64, uin
     if (rc)
         return rc;
     CK(cudaSetDevice(ctx->dev[0].ordinal));
-    if (ctx->d_fb)
-    {
-        if (ctx->fb_imported) CK(cudaIpcCloseMemHandle(ctx->d_fb)); else CK(cudaFree(ctx->d_fb));
-        ctx->d_fb = nullptr;
-    }
+    if (ctx->fb_imported && ctx->d_fb)
+        CK(cudaIpcCloseMemHandle(ctx->d_fb));
+    ctx->d_fb = nullptr;
+    ctx->fb_own.release();
     cudaIpcMemHandle_t h;
     std::memcpy(&h, handle64, 64);
     void *p = nullptr;
@@ -1195,23 +1171,16 @@ int ensure_hit_buffers(cuda_trace_ctx *ctx, const cuda_trace_frame *f)
 {
     const uint64_t need = (uint64_t) f->width * f->height * f->spp;
     CK(cudaSetDevice(ctx->dev[0].ordinal));
-    if (need > ctx->hit_cap)
-    {
-        cudaFree(ctx->d_hit_tri); cudaFree(ctx->d_hit_t); cudaFree(ctx->d_hit_u); cudaFree(ctx->d_hit_v);
-        ctx->d_hit_tri = nullptr; ctx->d_hit_t = ctx->d_hit_u = ctx->d_hit_v = nullptr;
-        ctx->hit_cap = 0;
-        CK(cudaMalloc(&ctx->d_hit_tri, need * 4));
-        CK(cudaMalloc(&ctx->d_hit_t, need * 4));
-        CK(cudaMalloc(&ctx->d_hit_u, need * 4));
-        CK(cudaMalloc(&ctx->d_hit_v, need * 4));
-        ctx->hit_cap = need;
-    }
+    CK(ctx->d_hit_tri.grow(need));
+    CK(ctx->d_hit_t.grow(need));
+    CK(ctx->d_hit_u.grow(need));
+    CK(ctx->d_hit_v.grow(need));
     ctx->hit_count = need;
     // samples outside the requested tiles read as "miss"
-    CK(cudaMemsetAsync(ctx->d_hit_tri, 0xFF, need * 4, ctx->dev[0].stream));
-    CK(cudaMemsetAsync(ctx->d_hit_t, 0, need * 4, ctx->dev[0].stream));
-    CK(cudaMemsetAsync(ctx->d_hit_u, 0, need * 4, ctx->dev[0].stream));
-    CK(cudaMemsetAsync(ctx->d_hit_v, 0, need * 4, ctx->dev[0].stream));
+    CK(cudaMemsetAsync(ctx->d_hit_tri.get(), 0xFF, need * 4, ctx->dev[0].stream));
+    CK(cudaMemsetAsync(ctx->d_hit_t.get(), 0, need * 4, ctx->dev[0].stream));
+    CK(cudaMemsetAsync(ctx->d_hit_u.get(), 0, need * 4, ctx->dev[0].stream));
+    CK(cudaMemsetAsync(ctx->d_hit_v.get(), 0, need * 4, ctx->dev[0].stream));
     CK(cudaStreamSynchronize(ctx->dev[0].stream));
     return 0;
 }
@@ -1280,11 +1249,11 @@ void choose_occupancy_home(const cuda_trace_ctx *ctx, const DeviceState& d, bool
             occ_smem_words = (uint32_t) bit_words;
         }
     }
-    if (occ_mode == kOccGlobalBits && d.d_pcell_dist && ctx->tune.occ_mode < 0)
+    if (occ_mode == kOccGlobalBits && d.scene.d_pcell_dist.get() && ctx->tune.occ_mode < 0)
         occ_mode = kOccGlobalDist; // too large for shared memory: distance map through L1
     const int m = ctx->tune.occ_mode;
     if (m == kOccGlobalBits) { occ_mode = kOccGlobalBits; occ_smem_words = 0; }
-    if (m == kOccGlobalDist && d.d_pcell_dist) { occ_mode = kOccGlobalDist; occ_smem_words = 0; }
+    if (m == kOccGlobalDist && d.scene.d_pcell_dist.get()) { occ_mode = kOccGlobalDist; occ_smem_words = 0; }
     if (m == kOccSmemBits && bit_words * 4 + other_smem <= 200 * 1024) { occ_mode = kOccSmemBits; occ_smem_words = (uint32_t) bit_words; }
     if (m == kOccSmemBytes && byte_words * 4 + other_smem <= 200 * 1024) { occ_mode = kOccSmemBytes; occ_smem_words = (uint32_t) byte_words; }
 }
@@ -1335,31 +1304,27 @@ int prepare_cost_order(cuda_trace_ctx *ctx, DeviceState& d, const cuda_trace_fra
         CK(cudaStreamWaitEvent(d.stream, d.ev_order, 0)); // the order this frame follows / the buffers it reuses
         d.order_pending = false;
     }
-    if (d.order_cap < shard_strips)
+    if (d.d_strip_cycles.size() < shard_strips)
     {
+        // the order build behind the last frame may still use the buffers.  d_strip_cycles grows last, so that after
+        // a failure half way it is still short and the next frame grows what is missing
         CK(cudaStreamSynchronize(d.order_stream));
-        cudaFree(d.d_strip_cycles); cudaFree(d.d_fetch_order); cudaFree(d.d_order_scratch); cudaFree(d.d_visit_cycles);
-        d.d_strip_cycles = d.d_fetch_order = d.d_order_scratch = d.d_visit_cycles = nullptr;
-        d.order_cap = 0;
         d.order_valid = false;
-        CK(cudaMalloc(&d.d_strip_cycles, sizeof(uint32_t) * shard_strips));
-        CK(cudaMalloc(&d.d_fetch_order, sizeof(uint32_t) * strip_order_capacity(shard_strips, 4)));
-        CK(cudaMalloc(&d.d_visit_cycles, sizeof(uint32_t) * strip_order_capacity(shard_strips, 4)));
-        CK(cudaMalloc(&d.d_order_scratch, sizeof(uint32_t) * strip_order_scratch_words(shard_strips)));
-        if (!d.d_cost_sum)
-            CK(cudaMalloc(&d.d_cost_sum, sizeof(unsigned long long)));
-        if (!d.d_visit_total)
-            CK(cudaMalloc(&d.d_visit_total, sizeof(uint32_t)));
-        d.order_cap = shard_strips;
+        CK(d.d_fetch_order.grow(strip_order_capacity(shard_strips, 4)));
+        CK(d.d_visit_cycles.grow(strip_order_capacity(shard_strips, 4)));
+        CK(d.d_order_scratch.grow(strip_order_scratch_words(shard_strips)));
+        CK(d.d_cost_sum.grow(1));
+        CK(d.d_visit_total.grow(1));
+        CK(d.d_strip_cycles.grow(shard_strips));
     }
     const std::vector<uint64_t> sig = { pl.serial, p.shard_rank, p.shard_world, p.shard_chunk, shard_strips };
     if (d.order_valid && sig == d.order_signature)
-        p.fetch_order = d.d_fetch_order;
-    p.visit_total = d.d_visit_total;
+        p.fetch_order = d.d_fetch_order.get();
+    p.visit_total = d.d_visit_total.get();
     d.order_signature = sig;
     d.order_strips = shard_strips;
-    p.visit_cycles = d.d_visit_cycles;
-    CK(cudaMemsetAsync(d.d_visit_cycles, 0, sizeof(uint32_t) * strip_order_capacity(shard_strips, pl.split_parts), d.stream));
+    p.visit_cycles = d.d_visit_cycles.get();
+    CK(cudaMemsetAsync(d.d_visit_cycles.get(), 0, sizeof(uint32_t) * strip_order_capacity(shard_strips, pl.split_parts), d.stream));
     return 0;
 }
 
@@ -1370,52 +1335,39 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     const FramePlan& pl = ctx->plan;
     const uint32_t n_dev = (uint32_t) ctx->dev.size(), n_tiles = (uint32_t) pl.rects.size();
     CK(cudaSetDevice(d.ordinal));
-    if (d.smp_cap < f->spp)
+    bool new_smp = false, new_tiles = false;
+    CK(d.d_smp.grow(f->spp, &new_smp));
+    if (new_smp || d.smp_valid_spp != f->spp)
     {
-        cudaFree(d.d_smp);
-        d.d_smp = nullptr;
-        CK(cudaMalloc(&d.d_smp, sizeof(float2) * f->spp));
-        d.smp_cap = f->spp;
-        d.smp_valid_spp = 0;
-    }
-    if (d.smp_valid_spp != f->spp)
-    {
-        launch_sample_table(d.d_smp, f->spp, d.stream); // K2
+        launch_sample_table(d.d_smp.get(), f->spp, d.stream); // K2
         ctx->launches++;
         d.smp_valid_spp = f->spp;
     }
-    if (d.tile_cap < n_tiles + 1)
-    {
-        cudaFree(d.d_tile_rects); cudaFree(d.d_tile_prefix);
-        d.d_tile_rects = nullptr; d.d_tile_prefix = nullptr;
-        d.tile_cap = std::max<uint32_t>(n_tiles + 1, 128);
-        d.layout_serial = 0;
-        CK(cudaMalloc(&d.d_tile_rects, sizeof(uint4) * d.tile_cap));
-        CK(cudaMalloc(&d.d_tile_prefix, sizeof(uint32_t) * d.tile_cap));
-    }
+    CK(d.d_tile_rects.grow(std::max<uint32_t>(n_tiles + 1, 128), &new_tiles));
+    CK(d.d_tile_prefix.grow(std::max<uint32_t>(n_tiles + 1, 128), &new_tiles));
     // the tile list usually repeats from frame to frame: upload it only when it changed (the plan owns the host
     // arrays, so the asynchronous copies need no synchronisation before returning)
-    if (d.layout_serial != pl.serial)
+    if (new_tiles || d.layout_serial != pl.serial)
     {
         d.layout_serial = 0;
         if (n_tiles)
-            CK(cudaMemcpyAsync(d.d_tile_rects, pl.rects.data(), sizeof(uint4) * n_tiles, cudaMemcpyHostToDevice, d.stream));
-        CK(cudaMemcpyAsync(d.d_tile_prefix, pl.prefix.data(), sizeof(uint32_t) * (n_tiles + 1), cudaMemcpyHostToDevice, d.stream));
+            CK(cudaMemcpyAsync(d.d_tile_rects.get(), pl.rects.data(), sizeof(uint4) * n_tiles, cudaMemcpyHostToDevice, d.stream));
+        CK(cudaMemcpyAsync(d.d_tile_prefix.get(), pl.prefix.data(), sizeof(uint32_t) * (n_tiles + 1), cudaMemcpyHostToDevice, d.stream));
         CK(cudaStreamSynchronize(d.stream)); // pageable source: consumed before the plan can be replaced
         d.layout_serial = pl.serial;
     }
     // strip counter + this GPU's per-band piece counts (the cancel word behind them is never cleared)
-    CK(cudaMemsetAsync(d.d_strip_counter, 0, (32 + kMaxBands) * sizeof(uint32_t), d.stream));
+    CK(cudaMemsetAsync(d.d_strip_counter.get(), 0, (32 + kMaxBands) * sizeof(uint32_t), d.stream));
     if (ctx->counting)
-        CK(cudaMemsetAsync(d.d_counters, 0, sizeof(Counters), d.stream));
+        CK(cudaMemsetAsync(d.d_counters.get(), 0, sizeof(Counters), d.stream));
 
     TraceParams p;
     p.grid = grid_dev(ctx, d);
     p.pair_sbox = nullptr;
     fill_camera(ctx, f, kind, p);
-    p.smp = d.d_smp;
-    p.tile_rects = d.d_tile_rects;
-    p.tile_strip_prefix = d.d_tile_prefix;
+    p.smp = d.d_smp.get();
+    p.tile_rects = d.d_tile_rects.get();
+    p.tile_strip_prefix = d.d_tile_prefix.get();
     p.n_tiles = n_tiles;
     p.strip_w = pl.strip_w;
     p.strip_h = pl.strip_h;
@@ -1425,23 +1377,23 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     p.shard_world = ctx->shard_world * n_dev;
     p.shard_rank = ctx->shard_rank * n_dev + i;
     p.shard_chunk = ctx->shard_chunk;
-    p.strip_counter = d.d_strip_counter;
+    p.strip_counter = d.d_strip_counter.get();
     p.cancel = d.d_cancel;
     p.cancel_seen = d.d_cancel_seen;
     p.frame_seq = seq;
     p.framebuffer = ctx->d_fb;
     p.band_done = use_bands ? band_counters(ctx) : nullptr;
     p.band_rows = ctx->band_rows;
-    p.band_local = use_bands ? d.d_strip_counter + 32 : nullptr; // own cache line
+    p.band_local = use_bands ? d.d_strip_counter.get() + 32 : nullptr; // own cache line
     std::memset(p.band_share, 0, sizeof(p.band_share));
     if (use_bands)
         std::memcpy(p.band_share, ctx->band_share[p.shard_rank].data(), sizeof(p.band_share));
     p.pool_walk_steps = 0;
-    p.hit_tri = kind.keep_hits ? ctx->d_hit_tri : nullptr;
-    p.hit_t = kind.keep_hits ? ctx->d_hit_t : nullptr;
-    p.hit_u = kind.keep_hits ? ctx->d_hit_u : nullptr;
-    p.hit_v = kind.keep_hits ? ctx->d_hit_v : nullptr;
-    p.counters = d.d_counters;
+    p.hit_tri = kind.keep_hits ? ctx->d_hit_tri.get() : nullptr;
+    p.hit_t = kind.keep_hits ? ctx->d_hit_t.get() : nullptr;
+    p.hit_u = kind.keep_hits ? ctx->d_hit_u.get() : nullptr;
+    p.hit_v = kind.keep_hits ? ctx->d_hit_v.get() : nullptr;
+    p.counters = d.d_counters.get();
 
     const uint64_t strips_here = (pl.total + p.shard_world - 1) / p.shard_world;
     const int threads = choose_cta(ctx, d, f, strips_here, p);
@@ -1458,7 +1410,7 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     // most of the time goes into long triangle lists, which coherent lanes (K1) test with broadcast loads
     const uint64_t pcells_here = (uint64_t) (ctx->desc.dim[0] + 2) * (ctx->desc.dim[1] + 2) * (ctx->desc.dim[2] + 2);
     const bool pool_pays = ctx->tune.pool == 1 || (uint64_t) ctx->num_pairs * 3 < pcells_here;
-    const bool use_pool = d.d_pcell_dist && ctx->tune.pool != 0 && pool_pays && !kind.alternates && !kind.count_inst &&
+    const bool use_pool = d.scene.d_pcell_dist.get() && ctx->tune.pool != 0 && pool_pays && !kind.alternates && !kind.count_inst &&
                           f->variant == kVariantMT && f->spp <= 32 && ctx->num_pairs > 0 &&
                           (uint64_t) f->width * f->height * f->spp < (1ull << 32);
     int rc = prepare_cost_order(ctx, d, f, p, use_pool);
@@ -1479,17 +1431,17 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
     CK(cudaEventRecord(d.ev_begin, d.stream));
     if (kvariant == kVariantMTRel && pl.total)
     {
+        SceneArrays& s = d.scene;
         // records relative to this frame's camera position: rebuilt (inside the timed region) when it moved
-        if (!d.d_pair_recs_rel)
-            CK(cudaMalloc(&d.d_pair_recs_rel, std::max<uint64_t>(ctx->num_pairs, 1) * 7 * sizeof(float4)));
-        if (!d.rel_valid || std::memcmp(d.rel_origin, p.cam.origin, sizeof(d.rel_origin)) != 0)
+        CK(s.d_pair_recs_rel.grow(std::max<uint64_t>(ctx->num_pairs, 1) * 7));
+        if (!s.rel_valid || std::memcmp(s.rel_origin, p.cam.origin, sizeof(s.rel_origin)) != 0)
         {
-            launch_origin_relative_pairs(d.d_pair_recs, std::max<uint64_t>(ctx->num_pairs, 1), p.cam.origin, d.d_pair_recs_rel, d.stream);
+            launch_origin_relative_pairs(s.d_pair_recs.get(), std::max<uint64_t>(ctx->num_pairs, 1), p.cam.origin, s.d_pair_recs_rel.get(), d.stream);
             ctx->launches++;
-            std::memcpy(d.rel_origin, p.cam.origin, sizeof(d.rel_origin));
-            d.rel_valid = true;
+            std::memcpy(s.rel_origin, p.cam.origin, sizeof(s.rel_origin));
+            s.rel_valid = true;
         }
-        p.grid.pair_recs_rel = d.d_pair_recs_rel;
+        p.grid.pair_recs_rel = s.d_pair_recs_rel.get();
         if (ctx->screen_cull != 0)
         {
             // screen boxes for this frame's camera, rebuilt (inside the timed region) when any camera constant the
@@ -1497,31 +1449,28 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
             // of its boxes are <= 32 pixels, 69 % of its pair iterations are skipped; the room of C4: none are, 6 % would
             // be skipped, and every kept iteration costs a box load and a vote -- so the boxes are counted once per
             // camera (a read-back, only then) and the cull is on when at least a fifth are small
-            if (!d.d_pair_sbox)
-            {
-                CK(cudaMalloc(&d.d_pair_sbox, std::max<uint64_t>(ctx->num_pairs, 1) * sizeof(float4)));
-                CK(cudaMalloc(&d.d_sbox_small, sizeof(unsigned int)));
-            }
+            CK(s.d_pair_sbox.grow(std::max<uint64_t>(ctx->num_pairs, 1)));
+            CK(s.d_sbox_small.grow(1));
             const CameraDev& c = p.cam;
-            const bool same = d.sbox_valid && std::memcmp(d.sbox_cam.m, c.m, sizeof(c.m)) == 0 &&
-                              std::memcmp(d.sbox_cam.origin, c.origin, sizeof(c.origin)) == 0 &&
-                              std::memcmp(&d.sbox_cam.fov_xs, &c.fov_xs, sizeof(float)) == 0 &&
-                              std::memcmp(&d.sbox_cam.aspect, &c.aspect, sizeof(float)) == 0 &&
-                              std::memcmp(&d.sbox_cam.width_f, &c.width_f, sizeof(float)) == 0;
+            const bool same = s.sbox_valid && std::memcmp(s.sbox_cam.m, c.m, sizeof(c.m)) == 0 &&
+                              std::memcmp(s.sbox_cam.origin, c.origin, sizeof(c.origin)) == 0 &&
+                              std::memcmp(&s.sbox_cam.fov_xs, &c.fov_xs, sizeof(float)) == 0 &&
+                              std::memcmp(&s.sbox_cam.aspect, &c.aspect, sizeof(float)) == 0 &&
+                              std::memcmp(&s.sbox_cam.width_f, &c.width_f, sizeof(float)) == 0;
             if (!same)
             {
-                launch_screen_boxes(d.d_pair_recs, ctx->num_pairs, c, d.d_pair_sbox, d.d_sbox_small, d.stream);
+                launch_screen_boxes(s.d_pair_recs.get(), ctx->num_pairs, c, s.d_pair_sbox.get(), s.d_sbox_small.get(), d.stream);
                 ctx->launches++;
                 unsigned int small = 0;
-                CK(cudaMemcpyAsync(&small, d.d_sbox_small, sizeof(small), cudaMemcpyDeviceToHost, d.stream));
+                CK(cudaMemcpyAsync(&small, s.d_sbox_small.get(), sizeof(small), cudaMemcpyDeviceToHost, d.stream));
                 CK(cudaStreamSynchronize(d.stream));
-                d.sbox_cam = c;
-                d.sbox_small = small;
-                d.sbox_cull = (uint64_t) small * 5 >= ctx->num_pairs;
-                d.sbox_valid = true;
+                s.sbox_cam = c;
+                s.sbox_small = small;
+                s.sbox_cull = (uint64_t) small * 5 >= ctx->num_pairs;
+                s.sbox_valid = true;
             }
-            if (ctx->screen_cull == 1 || d.sbox_cull)
-                p.pair_sbox = d.d_pair_sbox;
+            if (ctx->screen_cull == 1 || s.sbox_cull)
+                p.pair_sbox = s.d_pair_sbox.get();
         }
     }
     // K1's instance for this frame, now that the records and the cull are decided, and the grid its occupancy allows
@@ -1554,18 +1503,11 @@ int launch_on_device(cuda_trace_ctx *ctx, uint32_t i, const cuda_trace_frame *f,
         if (!kind.keep_hits)
         {
             const uint64_t need = (uint64_t) f->width * f->height * f->spp;
-            if (d.pool_cap < need)
-            {
-                cudaFree(d.d_pool_tri); cudaFree(d.d_pool_t); cudaFree(d.d_pool_u); cudaFree(d.d_pool_v);
-                d.d_pool_tri = nullptr; d.d_pool_t = d.d_pool_u = d.d_pool_v = nullptr;
-                d.pool_cap = 0;
-                CK(cudaMalloc(&d.d_pool_tri, need * 4));
-                CK(cudaMalloc(&d.d_pool_t, need * 4));
-                CK(cudaMalloc(&d.d_pool_u, need * 4));
-                CK(cudaMalloc(&d.d_pool_v, need * 4));
-                d.pool_cap = need;
-            }
-            pp.hit_tri = d.d_pool_tri; pp.hit_t = d.d_pool_t; pp.hit_u = d.d_pool_u; pp.hit_v = d.d_pool_v;
+            CK(d.d_pool_tri.grow(need));
+            CK(d.d_pool_t.grow(need));
+            CK(d.d_pool_u.grow(need));
+            CK(d.d_pool_v.grow(need));
+            pp.hit_tri = d.d_pool_tri.get(); pp.hit_t = d.d_pool_t.get(); pp.hit_u = d.d_pool_u.get(); pp.hit_v = d.d_pool_v.get();
         }
         // K7: one CTA per SM at 1024 threads (64 registers), more of the smaller CTAs of small frames
         const int pool_blocks = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) d.sm_count * std::max(1, 1024 / threads), want));
@@ -1610,8 +1552,8 @@ int enqueue_order_followup(cuda_trace_ctx *ctx, DeviceState& d)
     CK(cudaSetDevice(d.ordinal));
     CK(cudaEventRecord(d.ev_traced, d.stream));
     CK(cudaStreamWaitEvent(d.order_stream, d.ev_traced, 0));
-    launch_build_strip_order(d.d_visit_cycles, d.order_followup_used, d.d_strip_cycles, d.order_strips, ctx->plan.split_parts,
-                             d.d_cost_sum, d.d_order_scratch, d.d_visit_total, d.d_fetch_order, d.order_stream);
+    launch_build_strip_order(d.d_visit_cycles.get(), d.order_followup_used, d.d_strip_cycles.get(), d.order_strips, ctx->plan.split_parts,
+                             d.d_cost_sum.get(), d.d_order_scratch.get(), d.d_visit_total.get(), d.d_fetch_order.get(), d.order_stream);
     CK(cudaEventRecord(d.ev_order, d.order_stream));
     d.order_pending = true;
     ctx->launches += 5;
@@ -1791,14 +1733,14 @@ static int tiles_async_impl(cuda_trace_ctx *ctx, const cuda_trace_frame *f, cons
         if (start_cancelled)
         {
             ctx->cancel_seq.store(seq);
-            *(volatile uint32_t *) ctx->pinned_cancel_src = seq;
+            *(volatile uint32_t *) ctx->pinned_cancel_src.get() = seq;
         }
     }
     if (start_cancelled) // requested while this call was being set up: the kernels find the word already there
         for (DeviceState& d : ctx->dev)
         {
             CK(cudaSetDevice(d.ordinal));
-            CK(cudaMemcpyAsync(d.d_cancel, ctx->pinned_cancel_src, sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
+            CK(cudaMemcpyAsync(d.d_cancel, ctx->pinned_cancel_src.get(), sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
         }
     ctx->band_dirty = use_bands;
     ctx->t_prepared_ms = ms_since(ctx->t_enter);
@@ -1853,7 +1795,7 @@ int cuda_trace_sync(cuda_trace_ctx *ctx)
             float ms = 0.0f;
             CK(cudaEventElapsedTime(&ms, d.ev_begin, d.ev_end));
             ms_max = std::max(ms_max, ms);
-            cancelled = cancelled || *(volatile uint32_t *) d.h_cancel_seen == d.launched_seq; // stored by the kernel itself
+            cancelled = cancelled || *(volatile uint32_t *) d.h_cancel_seen.get() == d.launched_seq; // stored by the kernel itself
             d.frame_pending = false;
             any = true;
         }
@@ -1893,13 +1835,13 @@ int cuda_trace_cancel(cuda_trace_ctx *ctx)
         if (seq == 0)
             return 0; // nothing was ever launched
         ctx->cancel_seq.store(seq);
-        *(volatile uint32_t *) ctx->pinned_cancel_src = seq;
+        *(volatile uint32_t *) ctx->pinned_cancel_src.get() = seq;
     }
     for (DeviceState& d : ctx->dev)
     {
         if (cudaSetDevice(d.ordinal) != cudaSuccess)
             return CUDA_TRACE_ERR_CUDA;
-        if (cudaMemcpyAsync(d.d_cancel, ctx->pinned_cancel_src, sizeof(uint32_t), cudaMemcpyHostToDevice,
+        if (cudaMemcpyAsync(d.d_cancel, ctx->pinned_cancel_src.get(), sizeof(uint32_t), cudaMemcpyHostToDevice,
                             d.side_stream) != cudaSuccess)
             return CUDA_TRACE_ERR_CUDA;
     }
@@ -1976,17 +1918,8 @@ int cuda_trace_tiles_into(cuda_trace_ctx *ctx, const cuda_trace_frame *frame, co
     // class route: 512 x 512 0.52 ms tile by tile -> 0.18 ms through the image; 1080p 1.15 ms either way)
     if (frame && frame->width && frame->height && (uint64_t) frame->width * frame->height <= (1u << 20))
     {
-        const size_t pixels = (size_t) frame->width * frame->height;
-        if (ctx->staging_pixels < pixels)
-        {
-            if (ctx->staging)
-                cudaFreeHost(ctx->staging);
-            ctx->staging = nullptr;
-            ctx->staging_pixels = 0;
-            CK(cudaHostAlloc((void **) &ctx->staging, pixels * sizeof(uint32_t), cudaHostAllocPortable));
-            ctx->staging_pixels = pixels;
-        }
-        dst.staging = ctx->staging;
+        CK(ctx->staging.grow((size_t) frame->width * frame->height));
+        dst.staging = ctx->staging.get();
     }
     int rc = tiles_async_impl(ctx, frame, tiles, n_tiles, dst);
     if (rc)
@@ -2079,10 +2012,10 @@ int cuda_trace_download_hits(cuda_trace_ctx *ctx, uint32_t *tri_idx, float *t, f
         return fail(ctx, CUDA_TRACE_ERR_ARG, "download_hits: last frame was not rendered with CUDA_TRACE_FLAG_KEEP_HITS");
     CK(cudaSetDevice(ctx->dev[0].ordinal));
     const size_t bytes = ctx->hit_count * 4;
-    if (tri_idx) CK(cudaMemcpy(tri_idx, ctx->d_hit_tri, bytes, cudaMemcpyDeviceToHost));
-    if (t) CK(cudaMemcpy(t, ctx->d_hit_t, bytes, cudaMemcpyDeviceToHost));
-    if (u) CK(cudaMemcpy(u, ctx->d_hit_u, bytes, cudaMemcpyDeviceToHost));
-    if (v) CK(cudaMemcpy(v, ctx->d_hit_v, bytes, cudaMemcpyDeviceToHost));
+    if (tri_idx) CK(cudaMemcpy(tri_idx, ctx->d_hit_tri.get(), bytes, cudaMemcpyDeviceToHost));
+    if (t) CK(cudaMemcpy(t, ctx->d_hit_t.get(), bytes, cudaMemcpyDeviceToHost));
+    if (u) CK(cudaMemcpy(u, ctx->d_hit_u.get(), bytes, cudaMemcpyDeviceToHost));
+    if (v) CK(cudaMemcpy(v, ctx->d_hit_v.get(), bytes, cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -2133,43 +2066,30 @@ static int intersect_rays_impl(cuda_trace_ctx *ctx, uint32_t n, const float *ori
         return 0;
     DeviceState& d = ctx->dev[0];
     CK(cudaSetDevice(d.ordinal));
-    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr, *d_u = nullptr, *d_v = nullptr;
-    uint32_t *d_i = nullptr;
-    unsigned long long *d_stats = nullptr;
-    // every return below, failures included, frees the temporaries -- after the stream has drained, because a
-    // failed call may leave copies or the kernel enqueued
-    struct Temporaries
-    {
-        DeviceState& d;
-        std::array<void *, 7> p;
-        ~Temporaries()
-        {
-            cudaStreamSynchronize(d.stream);
-            for (void *q : p)
-                cudaFree(q);
-        }
-    } temps{ d, {} };
-    CK(cudaMalloc(&d_o, (size_t) n * 12)); temps.p[0] = d_o;
-    CK(cudaMalloc(&d_d, (size_t) n * 12)); temps.p[1] = d_d;
-    CK(cudaMalloc(&d_t, (size_t) n * 4)); temps.p[2] = d_t;
-    CK(cudaMalloc(&d_u, (size_t) n * 4)); temps.p[3] = d_u;
-    CK(cudaMalloc(&d_v, (size_t) n * 4)); temps.p[4] = d_v;
-    CK(cudaMalloc(&d_i, (size_t) n * 4)); temps.p[5] = d_i;
-    CK(cudaMemcpyAsync(d_o, origins, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
-    CK(cudaMemcpyAsync(d_d, dirs, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
+    DeviceArray<float> d_o, d_d, d_t, d_u, d_v;
+    DeviceArray<uint32_t> d_i;
+    DeviceArray<unsigned long long> d_stats;
+    StreamDrain drain(d.stream);
+    CK(d_o.alloc((size_t) n * 3));
+    CK(d_d.alloc((size_t) n * 3));
+    CK(d_t.alloc(n));
+    CK(d_u.alloc(n));
+    CK(d_v.alloc(n));
+    CK(d_i.alloc(n));
+    CK(cudaMemcpyAsync(d_o.get(), origins, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
+    CK(cudaMemcpyAsync(d_d.get(), dirs, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
     RayBatchParams p;
     p.grid = grid_dev(ctx, d);
-    p.n = n; p.origins = d_o; p.dirs = d_d; p.tri = d_i; p.t = d_t; p.u = d_u; p.v = d_v;
+    p.n = n; p.origins = d_o.get(); p.dirs = d_d.get(); p.tri = d_i.get(); p.t = d_t.get(); p.u = d_u.get(); p.v = d_v.get();
     p.mailbox_stats = nullptr;
     if (mailbox)
     {
-        CK(cudaMalloc(&d_stats, 2 * sizeof(unsigned long long)));
-        temps.p[6] = d_stats;
-        CK(cudaMemsetAsync(d_stats, 0, 2 * sizeof(unsigned long long), d.stream));
-        p.mailbox_stats = d_stats;
+        CK(d_stats.alloc(2));
+        CK(cudaMemsetAsync(d_stats.get(), 0, 2 * sizeof(unsigned long long), d.stream));
+        p.mailbox_stats = d_stats.get();
     }
     if (brute_force)
-        launch_brute_force(d.d_vtx, d.d_tri, ctx->num_tri, p, d.stream);
+        launch_brute_force(d.scene.d_vtx.get(), d.scene.d_tri.get(), ctx->num_tri, p, d.stream);
     else if (mailbox)
         launch_intersect_rays(p, variant, d.stream);
     else
@@ -2177,21 +2097,21 @@ static int intersect_rays_impl(cuda_trace_ctx *ctx, uint32_t n, const float *ori
         // the warp-cooperative query kernel: the same bits, faster on every workload (profiles/r03_ray_query.txt)
         cuda_trace_ray_batch q = {};
         q.n = n; q.kind = CUDA_TRACE_QUERY_CLOSEST; q.variant = variant; q.t_max_all = INFINITY;
-        q.origins = d_o; q.dirs = d_d; q.tri_idx = d_i; q.t = d_t; q.u = d_u; q.v = d_v;
+        q.origins = p.origins; q.dirs = p.dirs; q.tri_idx = p.tri; q.t = p.t; q.u = p.u; q.v = p.v;
         launch_query(ctx, d, q, d.stream);
     }
     ctx->launches++;
     CK(cudaGetLastError());
     if (mailbox)
     {
-        CK(cudaMemcpyAsync(ctx->mailbox_stats, d_stats, sizeof(ctx->mailbox_stats), cudaMemcpyDeviceToHost, d.stream));
+        CK(cudaMemcpyAsync(ctx->mailbox_stats, d_stats.get(), sizeof(ctx->mailbox_stats), cudaMemcpyDeviceToHost, d.stream));
         CK(cudaStreamSynchronize(d.stream));
     }
-    CK(cudaMemcpyAsync(tri_idx, d_i, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaMemcpyAsync(t, d_t, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaMemcpyAsync(u, d_u, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaMemcpyAsync(v, d_v, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaStreamSynchronize(d.stream));
+    CK(cudaMemcpyAsync(tri_idx, p.tri, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CK(cudaMemcpyAsync(t, p.t, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CK(cudaMemcpyAsync(u, p.u, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CK(cudaMemcpyAsync(v, p.v, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CK(drain.sync());
     return 0;
 }
 
@@ -2300,19 +2220,19 @@ int cuda_trace_ray_march(cuda_trace_ctx *ctx, uint32_t n, const float *origins, 
         return 0;
     DeviceState& d = ctx->dev[0];
     CK(cudaSetDevice(d.ordinal));
-    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr;
-    uint32_t *d_h = nullptr;
-    CK(cudaMalloc(&d_o, (size_t) n * 12)); CK(cudaMalloc(&d_d, (size_t) n * 12));
-    CK(cudaMalloc(&d_t, (size_t) n * 4)); CK(cudaMalloc(&d_h, (size_t) n * 4));
-    CK(cudaMemcpyAsync(d_o, origins, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
-    CK(cudaMemcpyAsync(d_d, dirs, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
-    launch_ray_march(d.d_vtx, d.d_tri, ctx->num_tri, n, d_o, d_d, d_h, d_t, d.stream);
+    DeviceArray<float> d_o, d_d, d_t;
+    DeviceArray<uint32_t> d_h;
+    StreamDrain drain(d.stream);
+    CK(d_o.alloc((size_t) n * 3)); CK(d_d.alloc((size_t) n * 3));
+    CK(d_t.alloc(n)); CK(d_h.alloc(n));
+    CK(cudaMemcpyAsync(d_o.get(), origins, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
+    CK(cudaMemcpyAsync(d_d.get(), dirs, (size_t) n * 12, cudaMemcpyHostToDevice, d.stream));
+    launch_ray_march(d.scene.d_vtx.get(), d.scene.d_tri.get(), ctx->num_tri, n, d_o.get(), d_d.get(), d_h.get(), d_t.get(), d.stream);
     ctx->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(hit, d_h, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaMemcpyAsync(t, d_t, (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaStreamSynchronize(d.stream));
-    cudaFree(d_o); cudaFree(d_d); cudaFree(d_t); cudaFree(d_h);
+    CK(cudaMemcpyAsync(hit, d_h.get(), (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CK(cudaMemcpyAsync(t, d_t.get(), (size_t) n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CK(drain.sync());
     return 0;
 }
 
@@ -2323,14 +2243,14 @@ int cuda_trace_sample_table(cuda_trace_ctx *ctx, uint32_t spp, float *xy)
     std::lock_guard<std::recursive_mutex> guard(ctx->api_mtx);
     DeviceState& d = ctx->dev[0];
     CK(cudaSetDevice(d.ordinal));
-    float2 *d_smp = nullptr;
-    CK(cudaMalloc(&d_smp, sizeof(float2) * spp));
-    launch_sample_table(d_smp, spp, d.stream);
+    DeviceArray<float2> d_smp;
+    StreamDrain drain(d.stream);
+    CK(d_smp.alloc(spp));
+    launch_sample_table(d_smp.get(), spp, d.stream);
     ctx->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(xy, d_smp, sizeof(float2) * spp, cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaStreamSynchronize(d.stream));
-    CK(cudaFree(d_smp));
+    CK(cudaMemcpyAsync(xy, d_smp.get(), sizeof(float2) * spp, cudaMemcpyDeviceToHost, d.stream));
+    CK(drain.sync());
     return 0;
 }
 
@@ -2403,24 +2323,24 @@ int cuda_trace_qmc_sequence(cuda_trace_ctx *ctx, uint32_t kind, uint32_t scrambl
         else
             table.assign(1, 0u); // reverse is a formula, the table is not read
     }
-    uint32_t *d_table = nullptr, *d_offset = nullptr;
-    double *d_out = nullptr;
+    DeviceArray<uint32_t> d_table, d_offset;
+    DeviceArray<double> d_out;
+    StreamDrain drain(d.stream);
     const size_t total = (size_t) count * dim_count;
     if (!table.empty())
     {
-        CK(cudaMalloc(&d_table, table.size() * sizeof(uint32_t)));
-        CK(cudaMalloc(&d_offset, offset.size() * sizeof(uint32_t)));
-        CK(cudaMemcpyAsync(d_table, table.data(), table.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
-        CK(cudaMemcpyAsync(d_offset, offset.data(), offset.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
+        CK(d_table.alloc(table.size()));
+        CK(d_offset.alloc(offset.size()));
+        CK(cudaMemcpyAsync(d_table.get(), table.data(), table.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
+        CK(cudaMemcpyAsync(d_offset.get(), offset.data(), offset.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
     }
-    CK(cudaMalloc(&d_out, total * sizeof(double)));
-    launch_qmc_sequence(kind, scramble, n_begin, count, dim_begin, dim_count, num_smp, bits, d_table, d_offset, n_primes,
-                        d_out, d.stream);
+    CK(d_out.alloc(total));
+    launch_qmc_sequence(kind, scramble, n_begin, count, dim_begin, dim_count, num_smp, bits, d_table.get(), d_offset.get(),
+                        n_primes, d_out.get(), d.stream);
     ctx->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out, d_out, total * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaStreamSynchronize(d.stream));
-    cudaFree(d_table); cudaFree(d_offset); cudaFree(d_out);
+    CK(cudaMemcpyAsync(out, d_out.get(), total * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    CK(drain.sync());
     return 0;
 }
 
@@ -2433,16 +2353,16 @@ int cuda_trace_qmc_cranley_patterson(cuda_trace_ctx *ctx, const double *x, doubl
         return 0;
     DeviceState& d = ctx->dev[0];
     CK(cudaSetDevice(d.ordinal));
-    double *d_x = nullptr, *d_o = nullptr;
-    CK(cudaMalloc(&d_x, count * sizeof(double)));
-    CK(cudaMalloc(&d_o, count * sizeof(double)));
-    CK(cudaMemcpyAsync(d_x, x, count * sizeof(double), cudaMemcpyHostToDevice, d.stream));
-    launch_cranley_patterson(d_x, e, count, d_o, d.stream);
+    DeviceArray<double> d_x, d_o;
+    StreamDrain drain(d.stream);
+    CK(d_x.alloc(count));
+    CK(d_o.alloc(count));
+    CK(cudaMemcpyAsync(d_x.get(), x, count * sizeof(double), cudaMemcpyHostToDevice, d.stream));
+    launch_cranley_patterson(d_x.get(), e, count, d_o.get(), d.stream);
     ctx->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out, d_o, count * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
-    CK(cudaStreamSynchronize(d.stream));
-    cudaFree(d_x); cudaFree(d_o);
+    CK(cudaMemcpyAsync(out, d_o.get(), count * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    CK(drain.sync());
     return 0;
 }
 
@@ -2459,7 +2379,7 @@ int cuda_trace_get_counters(cuda_trace_ctx *ctx, cuda_trace_counters *out)
     {
         Counters c;
         CK(cudaSetDevice(d.ordinal));
-        CK(cudaMemcpy(&c, d.d_counters, sizeof(c), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(&c, d.d_counters.get(), sizeof(c), cudaMemcpyDeviceToHost));
         out->rays += c.rays; out->cells += c.cells; out->tri_tests += c.tri_tests; out->hits += c.hits;
     }
     return 0;
@@ -2512,7 +2432,7 @@ int cuda_trace_download_strip_cycles(cuda_trace_ctx *ctx, uint32_t *cycles, uint
     if (n)
     {
         CK(cudaSetDevice(d.ordinal));
-        CK(cudaMemcpy(cycles, d.d_strip_cycles, n * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(cycles, d.d_strip_cycles.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     }
     return 0;
 }

@@ -10,6 +10,7 @@
 #include "grid_build.cuh"
 
 #include <cfloat>
+#include <utility>
 #include <vector>
 
 namespace rtm
@@ -404,23 +405,20 @@ int exclusive_scan_u32(const uint32_t *d_in, uint32_t *d_out, uint64_t n, cudaSt
     if (n == 0)
         return 0;
     const uint64_t tiles = (n + kScanTile - 1) / kScanTile;
-    uint32_t *d_sums = nullptr;
+    DeviceArray<uint32_t> d_sums;
     if (tiles > 1)
-        GB_CK(cudaMalloc(&d_sums, tiles * sizeof(uint32_t)));
-    scan_tile_kernel<<<(unsigned) tiles, kScanThreads, 0, stream>>>(d_in, d_out, n, d_sums);
+        GB_CK(d_sums.alloc(tiles));
+    scan_tile_kernel<<<(unsigned) tiles, kScanThreads, 0, stream>>>(d_in, d_out, n, d_sums.get());
     (*launches)++;
     if (tiles > 1)
     {
-        const int rc = exclusive_scan_u32(d_sums, d_sums, tiles, stream, err, launches);
+        StreamDrain drain(stream);
+        const int rc = exclusive_scan_u32(d_sums.get(), d_sums.get(), tiles, stream, err, launches);
         if (rc)
-        {
-            cudaFree(d_sums);
             return rc;
-        }
-        scan_add_kernel<<<(unsigned) tiles, kScanThreads, 0, stream>>>(d_out, n, d_sums);
+        scan_add_kernel<<<(unsigned) tiles, kScanThreads, 0, stream>>>(d_out, n, d_sums.get());
         (*launches)++;
-        GB_CK(cudaStreamSynchronize(stream));
-        cudaFree(d_sums);
+        GB_CK(drain.sync());
     }
     GB_CK(cudaGetLastError());
     return 0;
@@ -528,92 +526,89 @@ int build_grid_device(const float *d_vtx, uint32_t num_vtx, const uint32_t *d_tr
         err = "build_grid: empty mesh or grid_res == 0";
         return CUDA_TRACE_ERR_ARG;
     }
-    out->d_cell_start = nullptr;
-    out->d_tri_index = nullptr;
+    DeviceArray<float> d_partial;
+    DeviceArray<GridParamsDev> d_gp;
+    DeviceArray<unsigned long long> d_total;
+    DeviceArray<uint32_t> d_counts, d_big_list, d_big_count, d_cursor, d_tri_index, d_scratch;
+    StreamDrain drain(stream);
 
     // mesh box -> grid parameters
     const uint32_t aabb_blocks = (uint32_t) std::min<uint64_t>(1024, (num_tri + 255) / 256);
-    float *d_partial = nullptr;
-    GridParamsDev *d_gp = nullptr;
-    GB_CK(cudaMalloc(&d_partial, sizeof(float) * 6 * aabb_blocks));
-    GB_CK(cudaMalloc(&d_gp, sizeof(GridParamsDev)));
-    mesh_aabb_partial_kernel<<<aabb_blocks, 256, 0, stream>>>(d_vtx, d_tri, num_tri, d_partial);
-    grid_params_kernel<<<1, 1, 0, stream>>>(d_partial, aabb_blocks, grid_res, d_gp);
+    GB_CK(d_partial.alloc(6 * aabb_blocks));
+    GB_CK(d_gp.alloc(1));
+    mesh_aabb_partial_kernel<<<aabb_blocks, 256, 0, stream>>>(d_vtx, d_tri, num_tri, d_partial.get());
+    grid_params_kernel<<<1, 1, 0, stream>>>(d_partial.get(), aabb_blocks, grid_res, d_gp.get());
     *launches += 2;
     GridParamsDev gp;
-    GB_CK(cudaMemcpyAsync(&gp, d_gp, sizeof(gp), cudaMemcpyDeviceToHost, stream));
+    GB_CK(cudaMemcpyAsync(&gp, d_gp.get(), sizeof(gp), cudaMemcpyDeviceToHost, stream));
     GB_CK(cudaStreamSynchronize(stream));
-    cudaFree(d_partial);
 
     const uint64_t num_cells = (uint64_t) gp.dim[0] * gp.dim[1] * gp.dim[2];
     if (num_cells == 0 || num_cells >= (1ull << 31))
     {
-        cudaFree(d_gp);
         err = "build_grid: grid has " + std::to_string(num_cells) + " cells (supported: 1 .. 2^31-1)";
         return CUDA_TRACE_ERR_ARG;
     }
 
     // K3 count
-    uint32_t *d_counts = nullptr, *d_big_list = nullptr, *d_big_count = nullptr;
-    GB_CK(cudaMalloc(&d_counts, (num_cells + 1) * sizeof(uint32_t)));
-    GB_CK(cudaMalloc(&d_big_list, (size_t) num_tri * sizeof(uint32_t)));
-    GB_CK(cudaMalloc(&d_big_count, sizeof(uint32_t)));
-    GB_CK(cudaMemsetAsync(d_counts, 0, (num_cells + 1) * sizeof(uint32_t), stream));
-    GB_CK(cudaMemsetAsync(d_big_count, 0, sizeof(uint32_t), stream));
+    GB_CK(d_counts.alloc(num_cells + 1));
+    GB_CK(d_big_list.alloc(num_tri));
+    GB_CK(d_big_count.alloc(1));
+    GB_CK(cudaMemsetAsync(d_counts.get(), 0, (num_cells + 1) * sizeof(uint32_t), stream));
+    GB_CK(cudaMemsetAsync(d_big_count.get(), 0, sizeof(uint32_t), stream));
     const unsigned tri_blocks = (num_tri + 127) / 128;
-    grid_bin_small_kernel<<<tri_blocks, 128, 0, stream>>>(d_vtx, d_tri, num_tri, d_gp, false, d_counts, nullptr,
-                                                          d_big_list, d_big_count);
+    grid_bin_small_kernel<<<tri_blocks, 128, 0, stream>>>(d_vtx, d_tri, num_tri, d_gp.get(), false, d_counts.get(), nullptr,
+                                                          d_big_list.get(), d_big_count.get());
     (*launches)++;
     uint32_t big_count = 0;
-    GB_CK(cudaMemcpyAsync(&big_count, d_big_count, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    GB_CK(cudaMemcpyAsync(&big_count, d_big_count.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
     GB_CK(cudaStreamSynchronize(stream));
     if (big_count)
     {
-        grid_bin_big_kernel<<<big_count, 256, 0, stream>>>(d_vtx, d_tri, d_gp, false, d_counts, nullptr, d_big_list);
+        grid_bin_big_kernel<<<big_count, 256, 0, stream>>>(d_vtx, d_tri, d_gp.get(), false, d_counts.get(), nullptr,
+                                                           d_big_list.get());
         (*launches)++;
     }
 
     // total references (64-bit, to refuse grids whose CSR offsets would not fit uint32)
-    unsigned long long *d_total = nullptr, total = 0;
-    GB_CK(cudaMalloc(&d_total, sizeof(unsigned long long)));
-    GB_CK(cudaMemsetAsync(d_total, 0, sizeof(unsigned long long), stream));
-    sum_u32_kernel<<<1024, 256, 0, stream>>>(d_counts, num_cells, d_total);
+    unsigned long long total = 0;
+    GB_CK(d_total.alloc(1));
+    GB_CK(cudaMemsetAsync(d_total.get(), 0, sizeof(unsigned long long), stream));
+    sum_u32_kernel<<<1024, 256, 0, stream>>>(d_counts.get(), num_cells, d_total.get());
     (*launches)++;
-    GB_CK(cudaMemcpyAsync(&total, d_total, sizeof(total), cudaMemcpyDeviceToHost, stream));
+    GB_CK(cudaMemcpyAsync(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost, stream));
     GB_CK(cudaStreamSynchronize(stream));
-    cudaFree(d_total);
     if (total >= (1ull << 32))
     {
-        cudaFree(d_counts); cudaFree(d_big_list); cudaFree(d_big_count); cudaFree(d_gp);
         err = "build_grid: " + std::to_string(total) + " cell references do not fit 32-bit offsets";
         return CUDA_TRACE_ERR_ARG;
     }
 
     // K4 scan (in place: counts -> exclusive offsets; entry num_cells becomes the total)
-    int rc = exclusive_scan_u32(d_counts, d_counts, num_cells + 1, stream, err, launches);
+    int rc = exclusive_scan_u32(d_counts.get(), d_counts.get(), num_cells + 1, stream, err, launches);
     if (rc)
         return rc;
-    uint32_t *d_cell_start = d_counts;
+    uint32_t *d_cell_start = d_counts.get();
 
     // K5 fill through a cursor copy
-    uint32_t *d_cursor = nullptr, *d_tri_index = nullptr;
-    GB_CK(cudaMalloc(&d_cursor, num_cells * sizeof(uint32_t)));
-    GB_CK(cudaMalloc(&d_tri_index, std::max<uint64_t>(total, 1) * sizeof(uint32_t)));
-    GB_CK(cudaMemcpyAsync(d_cursor, d_cell_start, num_cells * sizeof(uint32_t), cudaMemcpyDeviceToDevice, stream));
-    grid_bin_small_kernel<<<tri_blocks, 128, 0, stream>>>(d_vtx, d_tri, num_tri, d_gp, true, d_cursor, d_tri_index,
-                                                          d_big_list, d_big_count);
+    GB_CK(d_cursor.alloc(num_cells));
+    GB_CK(d_tri_index.alloc(std::max<uint64_t>(total, 1)));
+    GB_CK(cudaMemcpyAsync(d_cursor.get(), d_cell_start, num_cells * sizeof(uint32_t), cudaMemcpyDeviceToDevice, stream));
+    grid_bin_small_kernel<<<tri_blocks, 128, 0, stream>>>(d_vtx, d_tri, num_tri, d_gp.get(), true, d_cursor.get(),
+                                                          d_tri_index.get(), d_big_list.get(), d_big_count.get());
     (*launches)++;
     if (big_count)
     {
-        grid_bin_big_kernel<<<big_count, 256, 0, stream>>>(d_vtx, d_tri, d_gp, true, d_cursor, d_tri_index, d_big_list);
+        grid_bin_big_kernel<<<big_count, 256, 0, stream>>>(d_vtx, d_tri, d_gp.get(), true, d_cursor.get(), d_tri_index.get(),
+                                                           d_big_list.get());
         (*launches)++;
     }
 
     // K5b per-cell sort (d_cursor is dead now: reuse it as the long-cell list)
-    uint32_t *d_long_cells = d_cursor, *d_long_count = d_big_count;
+    uint32_t *d_long_cells = d_cursor.get(), *d_long_count = d_big_count.get();
     GB_CK(cudaMemsetAsync(d_long_count, 0, sizeof(uint32_t), stream));
     sort_small_cells_kernel<<<(unsigned) ((num_cells + 255) / 256), 256, 0, stream>>>(d_cell_start, num_cells,
-                                                                                      d_tri_index, d_long_cells,
+                                                                                      d_tri_index.get(), d_long_cells,
                                                                                       d_long_count);
     (*launches)++;
     uint32_t long_count = 0;
@@ -622,23 +617,16 @@ int build_grid_device(const float *d_vtx, uint32_t num_vtx, const uint32_t *d_tr
     if (long_count)
     {
         const uint32_t smem_cap = 32768; // keys; 128 KB of shared memory
-        uint32_t *d_scratch = nullptr;
-        GB_CK(cudaMalloc(&d_scratch, std::max<uint64_t>(total, 1) * sizeof(uint32_t)));
+        GB_CK(d_scratch.alloc(std::max<uint64_t>(total, 1)));
         GB_CK(cudaFuncSetAttribute(sort_long_cells_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int) (smem_cap * sizeof(uint32_t))));
         sort_long_cells_kernel<<<long_count, 512, smem_cap * sizeof(uint32_t), stream>>>(d_cell_start, d_long_cells,
-                                                                                        d_tri_index, d_scratch,
-                                                                                        smem_cap);
+                                                                                        d_tri_index.get(),
+                                                                                        d_scratch.get(), smem_cap);
         (*launches)++;
-        GB_CK(cudaStreamSynchronize(stream));
-        cudaFree(d_scratch);
     }
-    GB_CK(cudaStreamSynchronize(stream));
+    GB_CK(drain.sync());
     GB_CK(cudaGetLastError());
-    cudaFree(d_cursor);
-    cudaFree(d_big_list);
-    cudaFree(d_big_count);
-    cudaFree(d_gp);
 
     for (int k = 0; k < 3; k++)
     {
@@ -650,8 +638,8 @@ int build_grid_device(const float *d_vtx, uint32_t num_vtx, const uint32_t *d_tr
     out->desc.inv_cell_wdh = gp.inv_cell_wdh;
     out->desc.num_cells = num_cells;
     out->desc.num_refs = total;
-    out->d_cell_start = d_cell_start;
-    out->d_tri_index = d_tri_index;
+    out->d_cell_start = std::move(d_counts);
+    out->d_tri_index = std::move(d_tri_index);
     return 0;
 }
 

@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/cuda_trace.h"
+#include "device_array.cuh"
 
 namespace rtm
 {
@@ -13,8 +14,8 @@ namespace rtm
 struct GridBuildResult
 {
     cuda_trace_grid_desc desc;
-    uint32_t *d_cell_start; // num_cells + 1
-    uint32_t *d_tri_index;  // num_refs (at least 1 allocated)
+    DeviceArray<uint32_t> d_cell_start; // num_cells + 1
+    DeviceArray<uint32_t> d_tri_index;  // num_refs (at least 1 allocated)
 };
 
 // Builds the reference's grid (grid.cpp:12-154) for the mesh in device memory (d_vtx: V x 6 floats,
