@@ -297,7 +297,7 @@ __global__ void origin_relative_pairs_kernel(const float4 *__restrict__ pair_rec
 // operation as tools/screen_cull.py restates it; the final narrowing rounds outwards.
 constexpr double kCullEps = 5.9604644775390625e-8; // 2^-24
 constexpr double kCullTau = 0.015625;              // a vertex counts as in front if its depth > 2^-6 |camera-space vector|
-constexpr double kCullRound = 16.0, kCullDir = 16.0, kCullSafety = 16.0, kCullKappaMax = 1.0e4;
+constexpr double kCullRound = 16.0, kCullDir = 16.0, kCullSafety = 4.0, kCullKappaMax = 1.0e4;
 
 struct CullCamera
 {

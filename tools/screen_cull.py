@@ -15,7 +15,7 @@ import numpy as np
 EPS = 2.0 ** -24
 TAU = 2.0 ** -6          # a vertex must lie clearly in front of the camera: depth w > TAU * |camera-space vector|
 C_ROUND, C_DIR = 16.0, 16.0  # rounding-error constants of the test and of generate_ray's direction (DESIGN.md)
-SAFETY = 16.0  # the slack used is SAFETY x the derived bound
+SAFETY = 4.0   # the slack used is SAFETY x the bound (DESIGN.md section 3 counts the rounding terms at <= 10 and 4)
 KAPPA_MAX = 1.0e4        # cameras whose 3x3 has a larger condition number cull nothing
 DUMMY = 0xFFFFFFFF       # tri index of the unhittable b half of an odd list's last pair (pack.cu)
 INF = float("inf")
@@ -187,6 +187,32 @@ def footprint_skips(boxes, x, y):
         return np.zeros(len(b), bool)
     x_lo, x_hi, y_lo, y_hi = x.min(), x.max(), y.min(), y.max()
     return (x_hi < b[:, 0]) | (x_lo > b[:, 1]) | (y_hi < b[:, 2]) | (y_lo > b[:, 3])
+
+
+def cell_scan(beg, length, boxes, x, y):
+    """The warp scan of the screen cull extended to every phase-B round, an alternative to the pair-by-pair walk that
+    test_pair_list keeps for lanes on different cells (profiles/r08_cull_tight.txt): the lanes with a list
+    (length > 0) are served one cell at a time, lowest list start first, each cell with footprint_skips over the points
+    of its own lanes.
+    beg, length: (32,) per lane, the lane's list [beg, beg + length) in the pairs' boxes (n, 4) float32; x, y: the
+    lanes' float32 image points.  -> (per lane, the pair indices it tests with `mine` set, in order; cells served;
+    chunks of 32 boxes loaded)"""
+    beg, length = np.asarray(beg, np.int64), np.asarray(length, np.int64)
+    x, y = np.asarray(x, np.float32), np.asarray(y, np.float32)
+    tested = [[] for _ in range(len(beg))]
+    todo = length > 0
+    cells = chunks = 0
+    while todo.any():
+        cell_beg = beg[todo].min()
+        mine = todo & (beg == cell_beg)
+        todo &= ~mine
+        n = int(length[mine].max())
+        kept = cell_beg + np.nonzero(~footprint_skips(boxes[cell_beg:cell_beg + n], x[mine], y[mine]))[0]
+        for lane in np.nonzero(mine)[0]:
+            tested[lane].extend(kept.tolist())
+        cells += 1
+        chunks += (n + 31) // 32
+    return tested, cells, chunks
 
 
 def image_point(px, py, w, h, off_x, off_y, fov_xs, aspect):

@@ -15,7 +15,9 @@ With --warp-scan it also replays the warp scan of the cull (csrc/warp_trace.cuh 
 whose lanes with a list all stand on one cell, 32 boxes are checked at once against the footprint of the lanes' image
 points (screen_cull.footprint_skips) and only the pairs left are walked; other rounds keep the serial walk.  It reports
 how often the fast path applies, the 32-pair chunks, the pairs the footprint keeps against those the per-lane check
-keeps, and the pair iterations before and after; and, as the alternative for phase A, the share of a lane's occupied-
+keeps, and the pair iterations before and after; the cells, chunks and kept pairs a scan per cell of the multi-cell
+rounds would have (screen_cull.cell_scan; measured on the B200 without a gain, profiles/r08_cull_tight.txt); and, as
+the alternative for phase A, the share of a lane's occupied-
 cell visits whose point lies outside the cell's box (the union of its pair boxes).
 
 python tools/warp_walk_model.py [workload] [n_strips] [--screen-cull | --warp-scan]   (test infrastructure: imports oracle/)"""
@@ -149,7 +151,7 @@ def cull_model():
     cnt = dict(iters=0, skip_pair=0, skip_tri=0, lane_tests=0, lane_out=0)
     # --warp-scan: rounds, one-cell rounds, their chunks, pair iterations, and the pairs kept by footprint / per lane
     scan = dict(rounds=0, one_cell=0, chunks=0, iters_one=0, kept_fp=0, kept_lane=0, iters_after=0, checks_after=0,
-                visits=0, visits_out=0)
+                visits=0, visits_out=0, multi=0, multi_serial=0, multi_cells=0, multi_chunks=0, multi_kept=0)
     if SCAN:
         ncell = len(pstart) - 1
         cell_of = np.repeat(np.arange(ncell), np.diff(pstart))
@@ -206,6 +208,14 @@ def cull_model():
                     else:
                         scan["iters_after"] += int(ln.max())
                         scan["checks_after"] += int(ln.max())
+                        # the alternative: one scan per distinct cell (sc.cell_scan), whose kept pairs would be the
+                        # warp's iterations (the cells' pair ranges are disjoint)
+                        tested, n_cells, n_chunks = sc.cell_scan(beg, ln, pb.astype(np.float32), xs, ys)
+                        scan["multi"] += 1
+                        scan["multi_serial"] += int(ln.max())
+                        scan["multi_cells"] += n_cells
+                        scan["multi_chunks"] += n_chunks
+                        scan["multi_kept"] += len(set(p for t in tested for p in t))
                 for i in range(int(ln.max())):
                     mine = i < ln
                     j = beg + np.minimum(i, np.maximum(ln - 1, 0))
@@ -234,6 +244,8 @@ def cull_model():
                  c["checks_after"]))
         print("  %d skipped iterations of %d remain (the serial walk of multi-cell rounds, and pairs the footprint keeps)"
               % (c["iters_after"] - (cnt["iters"] - cnt["skip_pair"]), c["iters_after"]))
+        print("  multi-cell rounds %d: serial walk %d pair iterations; a per-cell scan would take %d cells in %d chunks "
+              "and keep %d pairs" % (c["multi"], c["multi_serial"], c["multi_cells"], c["multi_chunks"], c["multi_kept"]))
         print("cell boxes (a phase-A alternative): lane occupied-cell visits outside the cell's box %d of %d (%.1f %%)"
               % (c["visits_out"], c["visits"], 100 * c["visits_out"] / c["visits"]))
 
